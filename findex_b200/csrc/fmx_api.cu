@@ -281,7 +281,7 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
     DevIndex &d = ix->d;
     d.blocks = (const uint4 *)blocks; d.stride = (uint64_t)nblk; d.bwt = d_bwt; d.C = d_C; d.base = d_base; d.code = d_code;
     d.bm = nullptr;
-    d.kmer = nullptr; d.kmer_k = 0; d.kmer_sigma = 0; d.sa = nullptr; d.isat = nullptr; d.isat_bits = 8; d.isat_syms = 12; d.ctx = nullptr; d.ctx_J = 0; d.ctx_raw = 0; d.ctx_plan = nullptr; d.ctx8 = nullptr; d.ctx8_J = 0;
+    d.kmer = nullptr; d.kmer_k = 0; d.kmer_sigma = 0; d.kmer_rows = 0; d.sa = nullptr; d.isat = nullptr; d.isat_bits = 8; d.isat_syms = 12; d.ctx = nullptr; d.ctx_J = 0; d.ctx_raw = 0; d.ctx_plan = nullptr; d.ctx8 = nullptr; d.ctx8_J = 0;
     d.dict = nullptr; d.dict_buckets = 0; d.dict_D = 0; d.dict_bits = 0; d.dict_Dx = 0; d.dict_Jc = 1;
     for (int t = 0; t < 8; ++t) d.ctx_S[t] = 0;
     d.mark = nullptr; d.samples = nullptr; d.n = (uint32_t)n; d.eof = (uint32_t)eof; d.layout = layout; d.levels = levels;
@@ -429,7 +429,7 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
         if (K >= 2) {
             const int64_t entries = entries_of(K);
             void *tab = nullptr;
-            e = cudaMalloc(&tab, (size_t)entries * 8); CU(e); ix->owned.push_back(tab);
+            e = cudaMalloc(&tab, (size_t)((entries + kKmerGroup - 1) / kKmerGroup) * kKmerGroup * 8); CU(e); ix->owned.push_back(tab);   // whole groups
             CU(build_kmer_table(d, ix->cfg, d_sym, (uint32_t)sigma, K, (uint2 *)tab, ix->stream));
             CU(cudaStreamSynchronize(ix->stream));
             d.kmer = (const uint2 *)tab; d.kmer_k = K; d.kmer_sigma = (uint32_t)sigma;
@@ -463,6 +463,21 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
             }
         }
         trim_pool(ix->device);
+    }
+    // k-mer group blocks: with a saturating table (intervals of about one row) most queries that go on with a full-depth hop through the row
+    // contexts find the rows' contexts in the table's own 64-byte block — one request instead of two (DESIGN.md §3/§5).  The group form needs
+    // the lexicographic order, so the table is built again in that order (same bytes, no more memory); the dictionary is grown from the
+    // plain order and is not combined with it.  FMX_KMER_ROWS=0 keeps the plain table (the A/B switch of the measurement).
+    const char *kr_env = std::getenv("FMX_KMER_ROWS");
+    const bool want_groups = !(kr_env && std::atoi(kr_env) == 0);
+    if (want_groups && is_auto && d.kmer != nullptr && d.ctx != nullptr && d.dict == nullptr && std::pow((double)sigma, d.kmer_k) >= n / 2.0) {
+        uint64_t entries = 1;
+        for (int j = 0; j < d.kmer_k; ++j) entries *= (uint64_t)sigma;
+        uint2 *tab = const_cast<uint2 *>(d.kmer);
+        CU(build_kmer_table(d, ix->cfg, d_sym, (uint32_t)sigma, d.kmer_k, tab, ix->stream, true));
+        CU(pack_kmer_groups(tab, entries, d.ctx, ix->stream));
+        CU(cudaStreamSynchronize(ix->stream));
+        d.kmer_rows = (int32_t)kKmerInlineRows;
     }
     // two lanes per query: with the 256-bit load a 64-B rank block is one request from two lanes (as from four lanes with 128-bit
     // loads), and twice as many queries are in flight per SM
@@ -624,6 +639,7 @@ int fmx_dict_info(const fmx_index *ix, int32_t *depth, int32_t *chain_depth, int
     if (bytes) *bytes = ix->d.dict ? (int64_t)ix->d.dict_buckets * 32 : 0;
     return FMX_OK;
 }
+int fmx_kmer_rows(const fmx_index *ix) { return ix && ix->d.kmer ? ix->d.kmer_rows : 0; }
 int fmx_ctx_depth(const fmx_index *ix) { return !ix ? 0 : ix->d.ctx ? ix->d.ctx_J : ix->d.ctx8 ? ix->d.ctx8_J : 0; }
 int fmx_ctx_entry_bytes(const fmx_index *ix) { return !ix ? 0 : ix->d.ctx ? 32 : ix->d.ctx8 ? 8 : 0; }
 int fmx_info(const fmx_index *ix, int32_t *layout, int32_t *levels, int32_t *sigma, int64_t *index_bytes, int32_t *rate) {

@@ -519,7 +519,9 @@ cudaError_t build_lcp(const uint32_t *d_sa, const uint32_t *d_isa, const uint8_t
 // k-mer table: entry idx <-> the K-byte pattern P with P[K-1-j] = sym[digit_j(idx)] (digit 0 most significant = the byte search()
 // consumes first, i.e. the LAST pattern byte); entry = (sp,ep) after those K backward steps, (0,0) when the interval is empty.
 // Built level by level: level 1 is (C[c], C[c+1]); an entry of level j+1 is one backward step from its parent idx/sigma of level j
-// with symbol idx%sigma — sigma^K * sigma/(sigma-1) steps in all instead of sigma^K * (K-1).
+// with symbol idx%sigma — sigma^K * sigma/(sigma-1) steps in all instead of sigma^K * (K-1).  In lexicographic order (lex) the new symbol is
+// the most significant digit instead: parent idx % sigma^(j), symbol idx / sigma^(j).  Dense codes ascend with the byte value, so there
+// consecutive entries are consecutive intervals of rows.
 __global__ void kmer_level1_kernel(const DevIndex ix, const uint8_t *__restrict__ sym, uint32_t sigma, uint2 *__restrict__ out) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= sigma) return;
@@ -529,19 +531,21 @@ __global__ void kmer_level1_kernel(const DevIndex ix, const uint8_t *__restrict_
 template <int G, int LAYOUT>
 __global__ void __launch_bounds__(kThreads)
 kmer_extend_kernel(const __grid_constant__ DevIndex ix, const uint8_t *__restrict__ sym, uint32_t sigma, const uint2 *__restrict__ prev,
-                   unsigned long long count, uint2 *__restrict__ out) {
+                   unsigned long long count, bool lex, uint2 *__restrict__ out) {
     __shared__ SharedTables tb;
     load_tables(tb, ix);
     __syncthreads();
     const unsigned long long t = (unsigned long long)blockIdx.x * (kThreads / G) + threadIdx.x / G;
     if (t >= count) return;                                // group-uniform
-    const uint2 p = prev[t / sigma];
+    const unsigned long long sub = count / sigma;          // entries of the parent level
+    const uint2 p = prev[lex ? t % sub : t / sigma];
     uint32_t sp = p.x, ep = p.y, touched = 0;
-    if (sp < ep) backward_step<G, LAYOUT, false>(ix, tb, (uint32_t)sym[t % sigma], sp, ep, touched);
+    if (sp < ep) backward_step<G, LAYOUT, false>(ix, tb, (uint32_t)sym[lex ? t / sub : t % sigma], sp, ep, touched);
     if ((threadIdx.x % G) == 0) out[t] = sp < ep ? make_uint2(sp, ep) : make_uint2(0u, 0u);
 }
 
-cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, uint32_t sigma, int K, uint2 *d_table, cudaStream_t st) {
+cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, uint32_t sigma, int K, uint2 *d_table, cudaStream_t st,
+                             bool lex) {
     if (K < 1 || sigma < 1) return cudaErrorInvalidValue;
     std::vector<unsigned long long> size((size_t)K + 1, 1);
     for (int j = 1; j <= K; ++j) size[(size_t)j] = size[(size_t)j - 1] * sigma;
@@ -554,7 +558,7 @@ cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d
         const unsigned long long cnt = size[(size_t)j];
         const unsigned long long per = kThreads / G;
         const unsigned grid = (unsigned)((cnt + per - 1) / per);
-#define CALL(GG, LAY) kmer_extend_kernel<GG, LAY><<<grid, kThreads, 0, st>>>(ix, d_sym, sigma, buf(j - 1), cnt, buf(j))
+#define CALL(GG, LAY) kmer_extend_kernel<GG, LAY><<<grid, kThreads, 0, st>>>(ix, d_sym, sigma, buf(j - 1), cnt, lex, buf(j))
         if (ix.layout == FMX_LAYOUT_PLANES) { if (G == 1) CALL(1, FMX_LAYOUT_PLANES); else if (G == 2) CALL(2, FMX_LAYOUT_PLANES); else CALL(4, FMX_LAYOUT_PLANES); }
         else if (ix.layout == FMX_LAYOUT_WMX) { if (G == 1) CALL(1, FMX_LAYOUT_WMX); else if (G == 2) CALL(2, FMX_LAYOUT_WMX); else CALL(4, FMX_LAYOUT_WMX); }
         else { if (G == 1) CALL(1, FMX_LAYOUT_WM); else if (G == 2) CALL(2, FMX_LAYOUT_WM); else CALL(4, FMX_LAYOUT_WM); }
@@ -562,6 +566,67 @@ cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d
         CK(cudaGetLastError());
     }
     if (d_tmp) cudaFreeAsync(d_tmp, st);
+    return cudaGetLastError();
+}
+
+// k-mer group blocks (layout: fmx_device.cuh, kmer_group): one thread per group of 8 lexicographically consecutive entries reads them and
+// writes the block over the same 64 bytes.  A group is narrow when its non-empty intervals follow each other without a gap and span at most
+// 255 rows; the J-hop halves of the row contexts of its first rows (up to kKmerInlineRows) then fill the rest of the block.
+__global__ void pack_kmer_groups_kernel(uint2 *__restrict__ table, unsigned long long entries, const uint4 *__restrict__ ctx) {
+    const unsigned long long g = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g * kKmerGroup >= entries) return;
+    uint2 v[kKmerGroup];
+#pragma unroll
+    for (uint32_t e = 0; e < kKmerGroup; ++e) {
+        const unsigned long long idx = g * kKmerGroup + e;
+        v[e] = idx < entries ? table[idx] : make_uint2(0u, 0u);
+        if (v[e].x >= v[e].y) v[e] = make_uint2(0u, 0u);
+    }
+    uint32_t base = 0, last = 0;
+    bool any = false, gap = false;
+#pragma unroll
+    for (uint32_t e = 0; e < kKmerGroup; ++e) {
+        if (v[e].x >= v[e].y) continue;
+        if (!any) { base = v[e].x; any = true; }
+        else if (v[e].x != last) gap = true;
+        last = v[e].y;
+    }
+    uint32_t w[16];
+#pragma unroll
+    for (int k = 0; k < 16; ++k) w[k] = 0;
+    w[0] = base;
+    if (gap || last - base > 255u) {
+        uint32_t prev = base;
+#pragma unroll
+        for (uint32_t e = 0; e < kKmerGroup; ++e) {
+            const bool ne = v[e].x < v[e].y;
+            const uint32_t end = ne ? v[e].y : prev, lead = ne ? v[e].x - prev : 0u;      // lead <= k: rows of no k-mer
+            w[4 + e] = end;
+            w[12 + e / 4] |= (lead & 0xFFu) << (8 * (e % 4));
+            prev = end;
+        }
+        w[3] = kKmerWide << 24;
+    } else {
+        uint32_t end = 0;
+#pragma unroll
+        for (uint32_t e = 0; e < kKmerGroup; ++e) {
+            if (v[e].x < v[e].y) end = v[e].y - base;
+            w[1 + e / 4] |= end << (8 * (e % 4));
+        }
+        const uint32_t kind = any ? min(last - base, kKmerInlineRows) : 0u;
+        w[3] = kind << 24;
+        for (uint32_t k = 0; k < kind; ++k) {
+            const uint4 c = ctx[2ull * (base + k) + 1];
+            w[4 + 4 * k] = c.x; w[5 + 4 * k] = c.y; w[6 + 4 * k] = c.z; w[7 + 4 * k] = c.w;
+        }
+    }
+    uint4 *dst = reinterpret_cast<uint4 *>(table + g * kKmerGroup);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) dst[k] = make_uint4(w[4 * k], w[4 * k + 1], w[4 * k + 2], w[4 * k + 3]);
+}
+cudaError_t pack_kmer_groups(uint2 *d_table, uint64_t entries, const uint4 *d_ctx, cudaStream_t st) {
+    const unsigned long long groups = (entries + kKmerGroup - 1) / kKmerGroup;
+    pack_kmer_groups_kernel<<<(unsigned)((groups + 255) / 256), 256, 0, st>>>(d_table, entries, d_ctx);
     return cudaGetLastError();
 }
 

@@ -34,8 +34,13 @@ cudaError_t build_ctx8(const uint32_t *d_sa, const uint32_t *d_isa, const uint8_
                        uint2 *d_ctx8, cudaStream_t st);
 // d_lcp[r] = lcp(suffix of row r, suffix of row r+1), d_lcp[n-1] = 0   (bwtFm2LCP, util.scala:153-212)
 cudaError_t build_lcp(const uint32_t *d_sa, const uint32_t *d_isa, const uint8_t *d_text, int64_t n, int32_t *d_lcp, cudaStream_t st);
-// (sp,ep) after the first K backward steps for every K-mer over the sigma occurring symbols
-cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, uint32_t sigma, int K, uint2 *d_table, cudaStream_t st);
+// (sp,ep) after the first K backward steps for every K-mer over the sigma occurring symbols; lex = false: the first consumed (last) pattern
+// byte is the most significant digit of the entry index, lex = true: lexicographic order of the K-mer (its first byte most significant)
+cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, uint32_t sigma, int K, uint2 *d_table, cudaStream_t st,
+                             bool lex = false);
+// converts a lexicographic table of `entries` (sp,ep) in place into k-mer group blocks (fmx_device.cuh kmer_group) that carry ctx[2r+1] of
+// up to kKmerInlineRows of their first rows; the buffer must hold ceil(entries / 8) * 64 bytes
+cudaError_t pack_kmer_groups(uint2 *d_table, uint64_t entries, const uint4 *d_ctx, cudaStream_t st);
 // dictionary of wide intervals (DevIndex::dict) grown from the dense k-mer table of `ix`: depths kmer_k+1 .. <= Dmax, intervals of more than
 // min_rows rows, at most max_entries entries; *d_table_out = nullptr when there is nothing to store (cudaMalloc'ed otherwise, 32 * buckets bytes)
 // (the deepest level, d = Dmax, keeps intervals of more than min_rows_top rows when those fit)

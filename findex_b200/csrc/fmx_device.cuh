@@ -43,9 +43,12 @@ struct DevIndex {
     uint64_t wmx_stride;        // blocks per level
     uint32_t zx[2][16];
     // ---- optional accelerators (bit-exact shortcuts that spend HBM capacity; DESIGN.md §3) ----
-    const uint2   *kmer;        // sigma^kmer_k entries: (sp,ep) after the first kmer_k backward steps, (0,0) if empty
+    const uint2   *kmer;        // sigma^kmer_k entries: (sp,ep) after the first kmer_k backward steps, (0,0) if empty — or, when kmer_rows > 0,
+                                // the same bytes as 64-byte k-mer group blocks (see kmer_group below)
     int32_t        kmer_k;
     uint32_t       kmer_sigma;
+    int32_t        kmer_rows;   // 0 = plain table (first consumed symbol most significant); > 0 = group blocks in lexicographic k-mer order
+                                // carrying the J-hop half of the row contexts of up to this many of their first rows
     const uint32_t *sa;         // full suffix array  sa[row]   (bwtFm2sa, util.scala:213-224)
     const uint4    *isat;       // per text position p: { isa[p], 96 bits of T'[p..] } — inverse SA and the text behind it in one 16-B fetch
     int32_t         isat_bits;  // bits per text symbol in isat: ceil(log2(sigma+1)); stored value = dense code + 1, 0 = '$' / past the end
@@ -520,6 +523,141 @@ __device__ __forceinline__ bool dict_chain(const DevIndex &ix, const uint8_t *co
     return true;
 }
 
+// ---- row-context hops ------------------------------------------------------------------------------------------------------------
+// The pattern side of a hop of j symbols that consumes pattern bytes o .. o+j-1, in the packing of the entries' 96-bit symbol field.
+// zero: one of those bytes is 0 (the '$' row wraps the text: ordinary steps instead); absent: one does not occur in the text (nothing matches).
+struct CtxQuery {
+    unsigned long long qlo, qhi, mlo, mhi;
+    uint32_t sh;
+    bool zero, absent;
+};
+template <typename PatFn>
+__device__ __forceinline__ CtxQuery ctx_query(const DevIndex &ix, const SharedTables &tb, PatFn pat, int j, int o) {
+    CtxQuery q;
+    const uint32_t bits = (uint32_t)ix.isat_bits;
+    q.qlo = 0; q.qhi = 0;
+    q.sh = (uint32_t)(ix.ctx_J - j) * bits;
+    const uint32_t nb = (uint32_t)j * bits;                                          // nb >= 1
+    q.mlo = nb >= 64 ? ~0ull : ((1ull << nb) - 1ull);
+    q.mhi = nb <= 64 ? 0ull : ((1ull << (nb - 64)) - 1ull);
+    q.zero = false; q.absent = false;
+    if (ix.ctx_raw) {                                     // raw bytes: pattern words compare directly, no translation;
+        uint32_t w0, w1, w2;                              // a byte that is absent from the text just never matches
+        pat.bytes12(o, w0, w1, w2);
+        q.qlo = ((unsigned long long)w1 << 32) | w0;
+        q.qhi = w2;
+        const unsigned long long l = q.qlo | ~q.mlo, h = (q.qhi & q.mhi) | ~q.mhi;   // bytes past the hop must not look like zeros
+        q.zero = (((l - 0x0101010101010101ull) & ~l) | ((h - 0x0101010101010101ull) & ~h)) & 0x8080808080808080ull;
+    } else {
+        for (int k = 0; k < j; ++k) {
+            const uint32_t pc = pat(o + k), cd = tb.code[pc];
+            q.zero = q.zero || (pc == 0);
+            q.absent = q.absent || (cd == (uint32_t)kCodeAbsent);
+            const unsigned long long v = (unsigned long long)((cd + 1u) & ((1u << bits) - 1u));
+            const uint32_t ob = (uint32_t)k * bits;
+            if (ob < 64) { q.qlo |= v << ob; if (ob + bits > 64) q.qhi |= v >> (64 - ob); }
+            else q.qhi |= v << (ob - 64);
+        }
+    }
+    return q;
+}
+// does the row whose context's second half is `b` = ctx[2r+1] go on with the hop's bytes?
+__device__ __forceinline__ bool ctx_match(const CtxQuery &q, const uint4 &b) {
+    const unsigned long long elo = ((unsigned long long)b.z << 32) | b.y, ehi = b.w;
+    unsigned long long lo, hi;
+    if (q.sh == 0) { lo = elo; hi = ehi; }
+    else if (q.sh < 64) { lo = (elo >> q.sh) | (ehi << (64 - q.sh)); hi = ehi >> q.sh; }
+    else { lo = ehi >> (q.sh - 64); hi = 0; }
+    return (((lo ^ q.qlo) & q.mlo) | ((hi ^ q.qhi) & q.mhi)) == 0ull;
+}
+
+// ---- k-mer group blocks (DevIndex::kmer_rows > 0; DESIGN.md §3) ------------------------------------------------------------------------
+// One 64-byte block per kKmerGroup consecutive k-mers in lexicographic order, in the bytes the plain table gives them.  Byte 15 = kind.
+//   narrow (kind 0..3 = inline rows): bytes 0-3 base row, bytes 4-11 eight cumulative u8 ends — entry e = [base + end[e-1], base + end[e]),
+//     end[-1] = 0; bytes 16-63 = ctx[2r+1] (the J-hop half of the row context) of rows base .. base+kind-1.
+//   wide (kind 0xFF: more than 255 rows, or a row of no k-mer — '$' or a suffix shorter than k — between two of the group's intervals):
+//     bytes 0-3 base, bytes 16-47 eight u32 ends, bytes 48-55 eight u8 leading gaps — entry e = [end[e-1] + gap[e], end[e]), end[-1] = base.
+// An empty entry decodes to (0,0), as in the plain table.
+constexpr uint32_t kKmerGroup = 8, kKmerWide = 0xFFu, kKmerInlineRows = 3;
+
+// The table lookup of a group-form index: one request per block at one lane per query (the count kernels' setting on such indexes; at 2
+// and 4 lanes every lane of the group loads the whole block, two requests).  When the next hop the plan takes is the
+// full-depth one (J symbols) and the interval is small enough for row contexts, the hop is resolved at once for the rows the block carries:
+// all of them inline -> the hop is done here (i -= J); otherwise the partial (minimum, count) and the first row still to fetch are handed to
+// the first row-context step of search_pattern, which looks only at the rest.  Group-uniform (every lane holds the whole block).
+// Every thread of the warp calls this together; `fetch` = this lane's query looks its block up.
+template <int G, bool STATS, typename PatFn>
+__device__ __forceinline__ void kmer_group(const DevIndex &ix, const SharedTables &tb, PatFn pat, bool fetch, uint32_t idx, int &i,
+                                           uint32_t &sp, uint32_t &ep, uint32_t &touched, uint32_t &steps, uint32_t &pre_from,
+                                           uint32_t &pre_best, uint32_t &pre_cnt) {
+    const uint4 *blk = reinterpret_cast<const uint4 *>(ix.kmer) + (uint64_t)(idx / kKmerGroup) * 4;
+    uint4 q0, q1, q2, q3;
+    if constexpr (G == 1) {
+        // What a random load costs is one request per load instruction and line: one lane's two 256-bit loads of its block are two.  So
+        // the lanes of a pair fetch each other's block halves — one instruction per block, two lanes x 32 B — and swap what the other needs.
+        const uint32_t odd = threadIdx.x & 1u;
+        const unsigned long long mine = reinterpret_cast<unsigned long long>(blk);
+        const unsigned long long pe = __shfl_sync(0xFFFFFFFFu, mine, (threadIdx.x & 31u) & ~1u);
+        const unsigned long long po = __shfl_sync(0xFFFFFFFFu, mine, (threadIdx.x & 31u) | 1u);
+        const bool fe = __shfl_sync(0xFFFFFFFFu, fetch, (threadIdx.x & 31u) & ~1u), fo = __shfl_sync(0xFFFFFFFFu, fetch, (threadIdx.x & 31u) | 1u);
+        uint4 x0 = make_uint4(0, 0, 0, 0), x1 = x0, y0 = x0, y1 = x0;
+        if (fe) ldg256(reinterpret_cast<const uint4 *>(pe) + 2 * odd, x0, x1);     // half `odd` of the even lane's block
+        if (fo) ldg256(reinterpret_cast<const uint4 *>(po) + 2 * odd, y0, y1);     // half `odd` of the odd lane's block
+        uint4 s0 = odd ? x0 : y0, s1 = odd ? x1 : y1;                            // what the partner lacks of its own block
+        s0.x = __shfl_xor_sync(0xFFFFFFFFu, s0.x, 1); s0.y = __shfl_xor_sync(0xFFFFFFFFu, s0.y, 1);
+        s0.z = __shfl_xor_sync(0xFFFFFFFFu, s0.z, 1); s0.w = __shfl_xor_sync(0xFFFFFFFFu, s0.w, 1);
+        s1.x = __shfl_xor_sync(0xFFFFFFFFu, s1.x, 1); s1.y = __shfl_xor_sync(0xFFFFFFFFu, s1.y, 1);
+        s1.z = __shfl_xor_sync(0xFFFFFFFFu, s1.z, 1); s1.w = __shfl_xor_sync(0xFFFFFFFFu, s1.w, 1);
+        if (odd) { q0 = s0; q1 = s1; q2 = y0; q3 = y1; } else { q0 = x0; q1 = x1; q2 = s0; q3 = s1; }
+    } else {
+        if (!fetch) return;
+        ldg256(blk, q0, q1);
+        ldg256(blk + 2, q2, q3);
+    }
+    if (!fetch) return;
+    const uint32_t e = idx % kKmerGroup, kind = q0.w >> 24, base = q0.x;
+    uint32_t lo, hi;
+    if (kind != kKmerWide) {
+        const unsigned long long ends = ((unsigned long long)q0.z << 32) | q0.y;
+        hi = base + (uint32_t)((ends >> (8 * e)) & 0xFFu);
+        lo = base + (e ? (uint32_t)((ends >> (8 * e - 8)) & 0xFFu) : 0u);
+    } else {
+        auto end_of = [&](uint32_t k) {
+            return k < 4 ? (k < 2 ? (k == 0 ? q1.x : q1.y) : (k == 2 ? q1.z : q1.w)) : (k < 6 ? (k == 4 ? q2.x : q2.y) : (k == 6 ? q2.z : q2.w));
+        };
+        hi = end_of(e);
+        lo = (e ? end_of(e - 1) : base) + (((e < 4 ? q3.x : q3.y) >> (8 * (e & 3))) & 0xFFu);
+    }
+    if (lo < hi) { sp = lo; ep = hi; } else { sp = 0; ep = 0; }
+    if (STATS) { touched += 1; steps += ix.kmer_k; }
+    if (kind == kKmerWide || kind == 0 || ix.ctx == nullptr || sp >= ep || i < 0) return;
+    const int rem = i + 1;
+    const uint32_t rows = ep - sp;
+    const int t = rem <= kCtxPlanMax ? (int)tb.plan[rem] : kCtxHops - 1;
+    const uint32_t need = rem <= kCtxPlanMax ? (uint32_t)tb.plan[128 + rem] : (uint32_t)(rem / ix.ctx_J + 3);
+    // exactly the condition under which search_pattern's first step is this hop through the row contexts
+    if (t != kCtxHops - 1 || rows > kCtxMaxRows || !(rows == 1u || rows * need <= (uint32_t)rem)) return;
+    const int j = ix.ctx_J;
+    const CtxQuery q = ctx_query(ix, tb, pat, j, rem - j);
+    if (q.zero) return;
+    uint32_t best = 0xFFFFFFFFu, cnt = 0;
+#pragma unroll
+    for (uint32_t k = 0; k < kKmerInlineRows; ++k) {
+        const uint4 &pl = k == 0 ? q1 : k == 1 ? q2 : q3;
+        if (k < kind && base + k >= sp && base + k < ep && !q.absent && ctx_match(q, pl)) { best = pl.x < best ? pl.x : best; ++cnt; }
+    }
+    if (ep <= base + kind) {
+        if (cnt) { sp = best; ep = best + cnt; } else { sp = 0; ep = 0; }
+        i -= j;
+        if (STATS) steps += j;
+    } else {
+        const int lane = (G == 1) ? 0 : (threadIdx.x & (G - 1));
+        pre_from = base + kind;
+        pre_best = best;
+        pre_cnt = lane == 0 ? cnt : 0u;                   // the lanes' counts are summed
+    }
+}
+
 // `mode` — how the two-pass count (dictionary first, the rest compacted; fmx_kernels.cu) hands a query over: kSearchFresh = from the
 // start; kSearchTopMissed = the dictionary probe at the deepest possible prefix has been done and missed (bisection goes on below it);
 // kSearchResume = the dictionary has been followed as far as it goes, (rsp, rep) is the interval after `rconsumed` symbols;
@@ -535,6 +673,9 @@ __device__ __forceinline__ void search_pattern(const DevIndex &ix, const SharedT
     ep = active ? ix.n : 0u;
     int i = len - 1;
     bool noshort = (ix.isat == nullptr);
+    uint32_t pre_from = 0, pre_best = 0xFFFFFFFFu, pre_cnt = 0;      // rows of the first row-context hop already resolved by kmer_group
+    bool kfetch = false;                                               // group-form table: this query's block is to be fetched (entry kidx)
+    uint32_t kidx = 0;
     if (active && (mode == kSearchResume || mode == kSearchChainMissed)) {
         sp = rsp; ep = rep;
         i -= rconsumed;
@@ -573,19 +714,23 @@ __device__ __forceinline__ void search_pattern(const DevIndex &ix, const SharedT
             }
         }
         if (!done && ix.kmer != nullptr && len >= ix.kmer_k) {
+            const int K = ix.kmer_k;
             uint32_t idx = 0;
             bool ok = true;
-            for (int j = 0; j < ix.kmer_k; ++j) {
-                const uint32_t c = pat(len - 1 - j), code = tb.code[c];
+            for (int j = 0; j < K; ++j) {                 // plain table: the last pattern byte most significant; groups: the k-mer's first
+                const uint32_t c = pat(ix.kmer_rows ? len - K + j : len - 1 - j), code = tb.code[c];
                 ok = ok && (code != (uint32_t)kCodeAbsent) && (c != 0);
                 idx = idx * ix.kmer_sigma + code;
             }
             if (ok) {
-                const uint2 v = ldg64(ix.kmer + idx);
-                sp = v.x; ep = v.y;
-                i -= ix.kmer_k;
+                i -= K;
                 done = true;
-                if (STATS) { touched += 1; steps += ix.kmer_k; }
+                if (ix.kmer_rows) { kfetch = true; kidx = idx; }     // the block is fetched below, where the whole warp is converged
+                else {
+                    const uint2 v = ldg64(ix.kmer + idx);
+                    sp = v.x; ep = v.y;
+                    if (STATS) { touched += 1; steps += K; }
+                }
             }
         }
         if (!done) {
@@ -596,6 +741,7 @@ __device__ __forceinline__ void search_pattern(const DevIndex &ix, const SharedT
             if (STATS) ++steps;
         }
     }
+    if (ix.kmer != nullptr && ix.kmer_rows) kmer_group<G, STATS>(ix, tb, pat, kfetch, kidx, i, sp, ep, touched, steps, pre_from, pre_best, pre_cnt);
     bool noctx = (ix.ctx == nullptr && ix.ctx8 == nullptr);
     for (;;) {
         const bool go = (i >= 0) && (sp < ep);
@@ -639,51 +785,26 @@ __device__ __forceinline__ void search_pattern(const DevIndex &ix, const SharedT
                 const int t = rem <= kCtxPlanMax ? (int)tb.plan[rem] : kCtxHops - 1;
                 const uint32_t need = rem <= kCtxPlanMax ? (uint32_t)tb.plan[128 + rem] : (uint32_t)(rem / ix.ctx_J + 3);
                 if (rows == 1u || rows * need <= (uint32_t)rem) {
-                    const int j = (int)tb.hops[t], o = rem - j;      // this hop consumes pattern bytes o .. rem-1
-                    const uint32_t bits = (uint32_t)ix.isat_bits;
-                    unsigned long long qlo = 0, qhi = 0;                  // those bytes in the entry's packing
-                    const uint32_t sh = (uint32_t)(ix.ctx_J - j) * bits, nb = (uint32_t)j * bits;       // nb >= 1
-                    const unsigned long long mlo = nb >= 64 ? ~0ull : ((1ull << nb) - 1ull);
-                    const unsigned long long mhi = nb <= 64 ? 0ull : ((1ull << (nb - 64)) - 1ull);
-                    bool zero = false, absent = false;
-                    if (ix.ctx_raw) {                                     // raw bytes: pattern words compare directly, no translation;
-                        uint32_t w0, w1, w2;                              // a byte that is absent from the text just never matches
-                        pat.bytes12(o, w0, w1, w2);
-                        qlo = ((unsigned long long)w1 << 32) | w0;
-                        qhi = w2;
-                        const unsigned long long l = qlo | ~mlo, h = (qhi & mhi) | ~mhi;   // bytes past the hop must not look like zeros
-                        zero = (((l - 0x0101010101010101ull) & ~l) | ((h - 0x0101010101010101ull) & ~h)) & 0x8080808080808080ull;
-                    } else {
-                        for (int k = 0; k < j; ++k) {
-                            const uint32_t pc = pat(o + k), cd = tb.code[pc];
-                            zero = zero || (pc == 0);
-                            absent = absent || (cd == (uint32_t)kCodeAbsent);
-                            const unsigned long long v = (unsigned long long)((cd + 1u) & ((1u << bits) - 1u));
-                            const uint32_t ob = (uint32_t)k * bits;
-                            if (ob < 64) { qlo |= v << ob; if (ob + bits > 64) qhi |= v >> (64 - ob); }
-                            else qhi |= v << (ob - 64);
-                        }
-                    }
-                    if (zero) noctx = true;                               // byte 0: the '$' row wraps the text, take the ordinary steps
+                    const int j = (int)tb.hops[t];                       // this hop consumes pattern bytes rem-j .. rem-1
+                    const CtxQuery q = ctx_query(ix, tb, pat, j, rem - j);
+                    if (q.zero) noctx = true;                             // byte 0: the '$' row wraps the text, take the ordinary steps
                     else {
-                        uint32_t best = 0xFFFFFFFFu, cnt = 0;
-                        if (!absent) {
-                            for (uint32_t r = sp + (uint32_t)lane; r < ep; r += G) {
+                        // rows before pre_from were resolved from the k-mer group block (their minimum and count carried in)
+                        const uint32_t from = sp > pre_from ? sp : pre_from;
+                        uint32_t best = pre_best, cnt = pre_cnt;
+                        if (!q.absent) {
+                            for (uint32_t r = from + (uint32_t)lane; r < ep; r += G) {
                                 uint4 a, b;
                                 ldg256(ix.ctx + (uint64_t)r * 2, a, b);
-                                const unsigned long long elo = ((unsigned long long)b.z << 32) | b.y, ehi = b.w;
-                                unsigned long long lo, hi;
-                                if (sh == 0) { lo = elo; hi = ehi; }
-                                else if (sh < 64) { lo = (elo >> sh) | (ehi << (64 - sh)); hi = ehi >> sh; }
-                                else { lo = ehi >> (sh - 64); hi = 0; }
-                                if ((((lo ^ qlo) & mlo) | ((hi ^ qhi) & mhi)) == 0ull) {
+                                if (ctx_match(q, b)) {
                                     const uint32_t row = t == 0 ? a.x : t == 1 ? a.y : t == 2 ? a.z : t == 3 ? a.w : b.x;
                                     best = row < best ? row : best;
                                     ++cnt;
                                 }
                             }
                         }
-                        if (STATS && lane == 0) { touched += absent ? 0u : rows; steps += j; }
+                        pre_from = 0; pre_best = 0xFFFFFFFFu; pre_cnt = 0;
+                        if (STATS && lane == 0) { touched += q.absent ? 0u : ep - from; steps += j; }
                         if (G >= 2) { best = min(best, __shfl_xor_sync(gmask, best, 1)); cnt += __shfl_xor_sync(gmask, cnt, 1); }
                         if (G >= 4) { best = min(best, __shfl_xor_sync(gmask, best, 2)); cnt += __shfl_xor_sync(gmask, cnt, 2); }
                         if (cnt) { sp = best; ep = best + cnt; } else { sp = 0; ep = 0; }

@@ -70,6 +70,7 @@ def lib():
     L.fmx_accel_info.argtypes = [p, C.POINTER(i32), C.POINTER(i32)]
     L.fmx_get_lanes.argtypes = [p]
     L.fmx_ctx_depth.argtypes = [p]
+    L.fmx_kmer_rows.argtypes = [p]
     L.fmx_dict_info.argtypes = [p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.fmx_ctx_entry_bytes.argtypes = [p]
     L.fmx_occ_batch.argtypes = [p, p, p, i64, p]
@@ -305,7 +306,7 @@ class GpuFMSearcher:
         _check(lib().fmx_dict_info(self.h, C.byref(dd), C.byref(dx), C.byref(de), C.byref(db)))
         return {"layout": {1: "wm", 2: "planes", 3: "wmx"}[lay.value], "levels": lev.value, "sigma": sig.value,
                 "dict_depth": dd.value, "dict_chain_depth": dx.value, "dict_entries": de.value, "dict_bytes": db.value,
-                "index_bytes": nb.value, "sa_sample_rate": rate.value, "kmer_k": k.value, "text_shortcut": bool(t.value),
+                "index_bytes": nb.value, "sa_sample_rate": rate.value, "kmer_k": k.value, "kmer_rows": lib().fmx_kmer_rows(self.h), "text_shortcut": bool(t.value),
                 "ctx_depth": lib().fmx_ctx_depth(self.h), "ctx_entry_bytes": lib().fmx_ctx_entry_bytes(self.h),
                 "lanes_per_query": lib().fmx_get_lanes(self.h)}
 

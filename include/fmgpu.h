@@ -111,6 +111,9 @@ int     fmx_accel_info(const fmx_index *ix, int32_t *kmer_k, int32_t *text_short
  * through the chain entries behind it (>= depth)                                                                                     */
 int     fmx_dict_info(const fmx_index *ix, int32_t *depth, int32_t *chain_depth, int64_t *entries, int64_t *bytes);
 int     fmx_ctx_depth(const fmx_index *ix);                  /* J of the row contexts (FMX_ACCEL_CTX / _CTX8), 0 = not built */
+/* rows whose row-context J-hop the k-mer table's 64-byte group blocks carry inline (0 = plain table of (sp,ep) entries).  Built under
+ * FMX_ACCEL_AUTO with 32-byte row contexts, a saturating table and no dictionary; FMX_KMER_ROWS=0 in the environment at open keeps the plain table */
+int     fmx_kmer_rows(const fmx_index *ix);
 int     fmx_ctx_entry_bytes(const fmx_index *ix);            /* 32, 8 or 0 */
 
 /* ---- occ(c,key)  M/bwtmerger.scala:354-375  (number of c in BWT[0..key], key=-1 -> 0) --------------- */
