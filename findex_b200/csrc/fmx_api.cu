@@ -1816,7 +1816,8 @@ int fmx_write_lcp_file(fmx_index *ix, const char *path) {
     return FMX_OK;
 }
 
-// SACreator.create (bwtmerger.scala:535-556): <base>.sa = n x int32 big-endian, no header, sa[r] as bwtFm2sa (util.scala:213-224).
+// SACreator.create (bwtmerger.scala:535-556): <base>.sa = n x 32-bit big-endian, no header, sa[r] as bwtFm2sa (util.scala:213-224).
+// The words are unsigned: positions at or beyond 2^31 (n < 2^32 - 1) are written as they are.
 // The reference walks the .fm array with one seek+write per row; here the suffix array the index already holds (or one built for
 // the occasion by the parallel LF chain walks) is copied out.
 int fmx_write_sa_file(fmx_index *ix, const char *path) {

@@ -539,7 +539,8 @@ class GpuFMSearcher:
         return cnt
 
     def write_sa_file(self, path):
-        """SACreator(path).create(): <base>.sa, n x int32 big-endian"""
+        """SACreator(path).create(): <base>.sa, n x 32-bit big-endian words, unsigned: positions at or beyond 2^31 are stored as they are,
+        so read them back as >u4 (the reference's int32 reading agrees below 2^31)"""
         lib().fmx_write_sa_file.argtypes = [C.c_void_p, C.c_char_p]
         _check(lib().fmx_write_sa_file(self.h, os.fsencode(path)))
 
@@ -587,7 +588,7 @@ class LCPSearcher(GpuFMSearcher):
         if not os.path.exists(base + ".sa"):
             self.write_sa_file(base)
         self._lcp = np.memmap(base + ".lcp", dtype=">i4", mode="r")
-        self._sa = np.memmap(base + ".sa", dtype=">i4", mode="r")
+        self._sa = np.memmap(base + ".sa", dtype=">u4", mode="r")          # unsigned: texts past 2^31 (fmx_write_sa_file)
 
     def getLCP(self, i):
         return int(self._lcp[i])
