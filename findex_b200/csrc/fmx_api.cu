@@ -36,7 +36,7 @@ struct fmx_index {
     int64_t n = 0, eof = 0;
     int64_t C[257] = {0};
     int64_t counts0[256] = {0};        // raw counts (bucketStarts0 / pos2char)
-    int sigma = 0, levels = 0, sample_rate = 0;
+    int sigma = 0, levels = 0, sample_rate = 0, text_rate = 0;
     int64_t nblk = 0, index_bytes = 0, n_samples = 0, rank_units64 = 0, dict_entries = 0;
     int api_layout = FMX_LAYOUT_WM;    // what fmx_info reports
     std::vector<void *> owned;         // device allocations freed at close
@@ -68,6 +68,12 @@ struct DBuf {
     ~DBuf() { if (p) cudaFreeAsync(p, st); }
     cudaError_t alloc(size_t bytes) { return cudaMallocAsync(&p, bytes ? bytes : 1, st); }
     template <typename T> T *as() { return reinterpret_cast<T *>(p); }
+};
+
+struct Events {                                                 // per-chunk events of a pipelined call, destroyed on every exit path
+    std::vector<cudaEvent_t> v;
+    ~Events() { for (cudaEvent_t e : v) if (e) cudaEventDestroy(e); }
+    cudaError_t make(size_t k) { v.assign(k, nullptr); for (auto &e : v) { cudaError_t r = cudaEventCreateWithFlags(&e, cudaEventDisableTiming); if (r != cudaSuccess) return r; } return cudaSuccess; }
 };
 
 struct SaBuf {
@@ -160,6 +166,7 @@ int bitrev(int v, int bits) { int r = 0; for (int i = 0; i < bits; ++i) r |= ((v
 int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, const int64_t counts[256], const fmx_opts &o) {
     if (n < 1 || eof < 0 || eof >= n) return fail(FMX_E_ARG, "bad n/eof");
     if (n >= (1ll << 32) - 1) return fail(FMX_E_UNSUPPORTED, "n = %lld needs 64-bit rows; this build indexes n < 2^32-1", (long long)n);
+    if (o.text_sample_rate < 0 || o.text_sample_rate > 65536) return fail(FMX_E_ARG, "text_sample_rate = %d: 0 (none) or 1 .. 65536", o.text_sample_rate);
     ix->n = n; ix->eof = eof;
     // C table: bucketStarts with counts[0] := 1   (bwtmerger.scala:346-350, util.scala:109-119)
     int64_t tot = 0;
@@ -194,7 +201,8 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
     if (layout == FMX_LAYOUT_AUTO) {
         size_t fr = 0, to = 0;
         cudaMemGetInfo(&fr, &to);
-        const int64_t sampled = o.sa_sample_rate > 0 ? nblk * 64 + (n / o.sa_sample_rate + 1) * 4 + (n / kRowsPerWalkBlock + 1) * 64 : 0;
+        const int64_t sampled = (o.sa_sample_rate > 0 ? nblk * 64 + (n / o.sa_sample_rate + 1) * 4 + (n / kRowsPerWalkBlock + 1) * 64 : 0) +
+                                (o.text_sample_rate > 0 ? ((n - 1) / o.text_sample_rate + 1) * 4 : 0);
         layout = (planes_bytes <= budget && planes_bytes + n + sampled <= total_cap && planes_bytes + (6ll << 30) + 2 * n < (int64_t)fr) ? FMX_LAYOUT_PLANES
                  : (wmx_bytes + n + sampled <= total_cap ? FMX_LAYOUT_WMX : FMX_LAYOUT_WM);
     }
@@ -284,19 +292,37 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
     d.kmer = nullptr; d.kmer_k = 0; d.kmer_sigma = 0; d.kmer_rows = 0; d.sa = nullptr; d.isat = nullptr; d.isat_bits = 8; d.isat_syms = 12; d.ctx = nullptr; d.ctx_J = 0; d.ctx_raw = 0; d.ctx_plan = nullptr; d.ctx8 = nullptr; d.ctx8_J = 0;
     d.dict = nullptr; d.dict_buckets = 0; d.dict_D = 0; d.dict_bits = 0; d.dict_Dx = 0; d.dict_Jc = 1;
     for (int t = 0; t < 8; ++t) d.ctx_S[t] = 0;
+    d.tsamp = nullptr; d.tsamp_rate = 0; d.sym = d_sym;
     d.mark = nullptr; d.samples = nullptr; d.n = (uint32_t)n; d.eof = (uint32_t)eof; d.layout = layout; d.levels = levels;
     for (int l = 0; l < 8; ++l) d.z[l] = z[l];
     d.wmx_b = wmx ? xb : 0; d.wmx_levels = wmx ? xlevels : 0; d.wmx_stride = (uint64_t)nblkx;
     for (int l = 0; l < 2; ++l) for (int v = 0; v < 16; ++v) d.zx[l][v] = zx[l][v];
 
     ix->sample_rate = o.sa_sample_rate;
+    // text samples (extract): the row of every text_rate-th T' position, recorded by the same chain walk as the sampled SA (or by that walk
+    // alone without a sampled SA)
+    uint32_t *tsamp = nullptr;
+    if (o.text_sample_rate > 0) {
+        const int64_t nt = (n - 1) / o.text_sample_rate + 1;
+        if (ix->index_bytes + nt * 4 > total_cap)
+            return fail(FMX_E_ARG, "max_total_bytes = %lld leaves no room for the %lld bytes of text samples", (long long)total_cap, (long long)nt * 4);
+        e = cudaMalloc((void **)&tsamp, (size_t)nt * 4); CU(e); ix->owned.push_back(tsamp);
+        ix->index_bytes += nt * 4;
+        ix->text_rate = o.text_sample_rate;
+        if (o.sa_sample_rate <= 0) {
+            std::string err;
+            e = build_sa_samples(d, layout, 0, nullptr, nblk, nullptr, 0, ix->stream, err, o.text_sample_rate, tsamp);
+            if (e != cudaSuccess) return fail(err.empty() ? FMX_E_CUDA : FMX_E_FORMAT, "text sample construction failed: %s", err.empty() ? cudaGetErrorString(e) : err.c_str());
+        }
+        d.tsamp = tsamp; d.tsamp_rate = (uint32_t)o.text_sample_rate;
+    }
     if (o.sa_sample_rate > 0) {
         const int64_t ns = (n + o.sa_sample_rate - 1) / o.sa_sample_rate;
         void *mark = nullptr, *samples = nullptr;
         e = cudaMalloc(&mark, (size_t)nblk * 64); CU(e); ix->owned.push_back(mark);
         e = cudaMalloc(&samples, (size_t)ns * 4); CU(e); ix->owned.push_back(samples);
         std::string err;
-        e = build_sa_samples(d, layout, o.sa_sample_rate, (uint32_t *)mark, nblk, (uint32_t *)samples, ns, ix->stream, err);
+        e = build_sa_samples(d, layout, o.sa_sample_rate, (uint32_t *)mark, nblk, (uint32_t *)samples, ns, ix->stream, err, o.text_sample_rate, tsamp);
         if (e != cudaSuccess) return fail(err.empty() ? FMX_E_CUDA : FMX_E_FORMAT, "sampled SA construction failed: %s", err.empty() ? cudaGetErrorString(e) : err.c_str());
         d.mark = (const uint4 *)mark; d.samples = (const uint32_t *)samples;
         ix->n_samples = ns;
@@ -896,11 +922,7 @@ static int count_fixed_pipeline(fmx_index *ix, const uint8_t *pat, int32_t len, 
     if (only_counts) CU(dcnt.alloc(m * 4));
     const int64_t chunk = cc.chunk_queries > 0 ? cc.chunk_queries : (1 << 20);
     const int64_t nchunks = (m + chunk - 1) / chunk;
-    struct Events {                                            // destroyed on every exit path
-        std::vector<cudaEvent_t> v;
-        ~Events() { for (cudaEvent_t e : v) if (e) cudaEventDestroy(e); }
-        cudaError_t make(size_t k) { v.assign(k, nullptr); for (auto &e : v) { cudaError_t r = cudaEventCreateWithFlags(&e, cudaEventDisableTiming); if (r != cudaSuccess) return r; } return cudaSuccess; }
-    } evs_in, evs_k;
+    Events evs_in, evs_k;
     CU(evs_in.make((size_t)nchunks)); CU(evs_k.make((size_t)nchunks));
     std::vector<cudaEvent_t> &ev_in = evs_in.v, &ev_k = evs_k.v;
     // the copy streams may touch the stream-ordered allocations only after the allocating stream reached this point
@@ -1130,6 +1152,85 @@ int fmx_next_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t 
 // One name for both walks (the sketch of SURVEY §8b): direction > 0 = nextSubstr, else prevSubstr.
 int fmx_extract_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t len, int32_t direction, uint8_t *out, int32_t *out_len) {
     return direction > 0 ? fmx_next_substr_batch(ix, row, m, len, out, out_len) : fmx_prev_substr_batch(ix, row, m, len, out, out_len);
+}
+
+// ---- extract: file bytes at file offsets (include/fmgpu.h) -----------------------------------------------------
+int fmx_text_sample_rate(const fmx_index *ix) { return ix ? ix->text_rate : 0; }
+
+// Host-buffer form: the requests flow through the call's three streams in chunks, as in the count pipeline (H2D of the offsets of chunk
+// k+1, the walks of chunk k and the D2H of chunk k-1 overlap).
+int fmx_text_batch(fmx_index *ix, const int64_t *off, int64_t m, int32_t len, uint8_t *out, int32_t *out_len) {
+    CHECK_IX(ix);
+    if (m < 0 || len < 0 || (m && (!off || !out_len || (len && !out)))) return fail(FMX_E_ARG, "bad argument");
+    for (int64_t i = 0; i < m; ++i)
+        if (off[i] < 0 || off[i] > ix->n - 1) return fail(FMX_E_ARG, "file offset %lld at %lld is outside [0, %lld]", (long long)off[i], (long long)i, (long long)(ix->n - 1));
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    if (text_path(cc.d) < 0) return fail(FMX_E_UNSUPPORTED, "extract needs text samples (fmx_opts.text_sample_rate) or the singleton shortcut (FMX_ACCEL_TEXT)");
+    if (m == 0) return FMX_OK;
+    DeviceGuard g(ix->device);
+    cudaStream_t st = cc.stream;
+    std::vector<uint32_t> off32((size_t)m);
+    for (int64_t i = 0; i < m; ++i) off32[(size_t)i] = (uint32_t)off[i];
+    DBuf doff(st), dout(st), dlen(st), dreq(st);
+    CU(doff.alloc((size_t)m * 4)); CU(dout.alloc((size_t)m * len)); CU(dlen.alloc((size_t)m * 4));
+    if (cc.stats) { CU(dreq.alloc(8)); CU(cudaMemsetAsync(dreq.p, 0, 8, st)); }
+    // chunks of about 64 MiB of output (at least 2^12 requests), or the caller's fmx_set_chunk
+    const int64_t chunk = cc.chunk_queries > 0 ? cc.chunk_queries : std::max<int64_t>(1 << 12, (64ll << 20) / std::max<int32_t>(len, 1));
+    const int64_t nchunks = (m + chunk - 1) / chunk;
+    Events evs_in, evs_k;
+    CU(evs_in.make((size_t)nchunks)); CU(evs_k.make((size_t)nchunks));
+    CU(cudaEventRecord(cc.ev_alloc, st));
+    CU(cudaStreamWaitEvent(cc.h2d, cc.ev_alloc, 0));
+    CU(cudaStreamWaitEvent(cc.d2h, cc.ev_alloc, 0));
+    Timed t(ix, cc);
+    int rc = FMX_OK;
+    for (int64_t k = 0; k < nchunks && rc == FMX_OK; ++k) {
+        const int64_t q0 = k * chunk, nq = std::min(chunk, m - q0);
+        cudaError_t e = cudaMemcpyAsync(doff.as<uint32_t>() + q0, off32.data() + q0, (size_t)nq * 4, cudaMemcpyHostToDevice, cc.h2d);
+        if (e == cudaSuccess) e = cudaEventRecord(evs_in.v[(size_t)k], cc.h2d);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(st, evs_in.v[(size_t)k], 0);
+        if (e == cudaSuccess) e = launch_text(cc.d, cc.cfg, doff.as<uint32_t>() + q0, nq, len, dout.as<uint8_t>() + q0 * len, dlen.as<int>() + q0,
+                                              cc.stats ? dreq.as<unsigned long long>() : nullptr, st);
+        if (e == cudaSuccess) e = cudaEventRecord(evs_k.v[(size_t)k], st);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(cc.d2h, evs_k.v[(size_t)k], 0);
+        if (e == cudaSuccess && len) e = cudaMemcpyAsync(out + q0 * len, dout.as<uint8_t>() + q0 * len, (size_t)nq * len, cudaMemcpyDeviceToHost, cc.d2h);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(out_len + q0, dlen.as<int>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
+        if (e != cudaSuccess) rc = fail(FMX_E_CUDA, "CUDA error %s in the extract pipeline (%s)", cudaGetErrorName(e), cudaGetErrorString(e));
+    }
+    ix->last_launches = nchunks; ix->total_launches += nchunks;
+    t.stop();
+    cudaError_t e1 = cudaStreamSynchronize(cc.h2d), e2 = cudaStreamSynchronize(st), e3 = cudaStreamSynchronize(cc.d2h);
+    if (rc == FMX_OK && (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess)) rc = fail(FMX_E_CUDA, "CUDA error while draining the extract pipeline");
+    t.collect();
+    if (rc == FMX_OK && cc.stats) {
+        unsigned long long h = 0;
+        CU(cudaMemcpy(&h, dreq.p, 8, cudaMemcpyDeviceToHost));
+        ix->last_steps = (int64_t)h;
+    }
+    return rc;
+}
+
+int fmx_text_dev(fmx_index *ix, const void *d_off, int64_t m, int32_t len, void *d_out, void *d_out_len, void *stream) {
+    CHECK_IX(ix);
+    if (m < 0 || len < 0 || (m && (!d_off || !d_out_len || (len && !d_out)))) return fail(FMX_E_ARG, "bad argument");
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    if (text_path(cc.d) < 0) return fail(FMX_E_UNSUPPORTED, "extract needs text samples (fmx_opts.text_sample_rate) or the singleton shortcut (FMX_ACCEL_TEXT)");
+    if (m == 0) return FMX_OK;
+    DeviceGuard g(ix->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    DBuf dreq(st);
+    if (cc.stats) { CU(dreq.alloc(8)); CU(cudaMemsetAsync(dreq.p, 0, 8, st)); }
+    CU(launch_text(cc.d, cc.cfg, (const uint32_t *)d_off, m, len, (uint8_t *)d_out, (int *)d_out_len, cc.stats ? dreq.as<unsigned long long>() : nullptr, st));
+    ix->last_launches = 1; ix->total_launches += 1;
+    if (cc.stats) {                                            // counting runs are untimed: wait for the count
+        unsigned long long h = 0;
+        CU(cudaMemcpyAsync(&h, dreq.p, 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        ix->last_steps = (int64_t)h;
+    }
+    return FMX_OK;
 }
 
 // ---- locate ---------------------------------------------------------------------------------------------------

@@ -224,7 +224,8 @@ chain_len_kernel(const __grid_constant__ DevIndex ix, uint32_t S, uint32_t nchai
 template <int LAYOUT>
 __global__ void __launch_bounds__(kThreads)
 chain_mark_kernel(const __grid_constant__ DevIndex ix, uint32_t S, uint32_t nchains, uint32_t eof_chain, const uint32_t *__restrict__ start_sa,
-                  uint32_t rate, uint32_t *__restrict__ mark_blocks, uint2 *__restrict__ pairs, unsigned long long *n_pairs) {
+                  uint32_t rate, uint32_t *__restrict__ mark_blocks, uint2 *__restrict__ pairs, unsigned long long *n_pairs, uint32_t text_rate,
+                  uint32_t *__restrict__ tsamp) {
     __shared__ SharedTables tb;
     load_tables(tb, ix);
     __syncthreads();
@@ -232,7 +233,8 @@ chain_mark_kernel(const __grid_constant__ DevIndex ix, uint32_t S, uint32_t ncha
     if (j >= nchains) return;
     uint32_t r = (j == eof_chain) ? ix.eof : j * S, v = start_sa[j];
     for (;;) {
-        if (v % rate == 0) {
+        if (tsamp != nullptr && v % text_rate == 0) tsamp[v / text_rate] = r;
+        if (rate != 0 && v % rate == 0) {
             const uint32_t b = r / kBitsPerBlock, o = r - b * kBitsPerBlock;
             atomicOr(&mark_blocks[(uint64_t)b * 16 + 1 + (o >> 5)], 1u << (o & 31));
             pairs[atomicAdd(n_pairs, 1ull)] = make_uint2(r, v);
@@ -327,18 +329,25 @@ cudaError_t prepare_chains(const DevIndex &ix, int layout, Chains &ch, cudaStrea
 }  // namespace
 
 cudaError_t build_sa_samples(const DevIndex &ix, int layout, int rate, uint32_t *d_mark_blocks, int64_t nblk, uint32_t *d_samples,
-                             int64_t n_samples, cudaStream_t st, std::string &err) {
+                             int64_t n_samples, cudaStream_t st, std::string &err, int text_rate, uint32_t *d_tsamp) {
     Chains ch;
     CK(prepare_chains(ix, layout, ch, st, err));
     const unsigned grid = (ch.nchains + kThreads - 1) / kThreads;
-    uint2 *d_pairs; unsigned long long *d_np;
-    CK(cudaMallocAsync(&d_pairs, (size_t)n_samples * 8, st));
-    CK(cudaMallocAsync(&d_np, 8, st));
-    CK(cudaMemsetAsync(d_np, 0, 8, st));
-    CK(cudaMemsetAsync(d_mark_blocks, 0, (size_t)nblk * 64, st));
-    if (layout == FMX_LAYOUT_PLANES) chain_mark_kernel<FMX_LAYOUT_PLANES><<<grid, kThreads, 0, st>>>(ix, ch.S, ch.nchains, ch.eof_chain, ch.d_start, (uint32_t)rate, d_mark_blocks, d_pairs, d_np);
-    else if (layout == FMX_LAYOUT_WMX) chain_mark_kernel<FMX_LAYOUT_WMX><<<grid, kThreads, 0, st>>>(ix, ch.S, ch.nchains, ch.eof_chain, ch.d_start, (uint32_t)rate, d_mark_blocks, d_pairs, d_np);
-    else chain_mark_kernel<FMX_LAYOUT_WM><<<grid, kThreads, 0, st>>>(ix, ch.S, ch.nchains, ch.eof_chain, ch.d_start, (uint32_t)rate, d_mark_blocks, d_pairs, d_np);
+    uint2 *d_pairs = nullptr; unsigned long long *d_np = nullptr;
+    if (rate > 0) {
+        CK(cudaMallocAsync(&d_pairs, (size_t)n_samples * 8, st));
+        CK(cudaMallocAsync(&d_np, 8, st));
+        CK(cudaMemsetAsync(d_np, 0, 8, st));
+        CK(cudaMemsetAsync(d_mark_blocks, 0, (size_t)nblk * 64, st));
+    }
+    const uint32_t r32 = rate > 0 ? (uint32_t)rate : 0u, t32 = d_tsamp ? (uint32_t)text_rate : 0u;
+    if (layout == FMX_LAYOUT_PLANES) chain_mark_kernel<FMX_LAYOUT_PLANES><<<grid, kThreads, 0, st>>>(ix, ch.S, ch.nchains, ch.eof_chain, ch.d_start, r32, d_mark_blocks, d_pairs, d_np, t32, d_tsamp);
+    else if (layout == FMX_LAYOUT_WMX) chain_mark_kernel<FMX_LAYOUT_WMX><<<grid, kThreads, 0, st>>>(ix, ch.S, ch.nchains, ch.eof_chain, ch.d_start, r32, d_mark_blocks, d_pairs, d_np, t32, d_tsamp);
+    else chain_mark_kernel<FMX_LAYOUT_WM><<<grid, kThreads, 0, st>>>(ix, ch.S, ch.nchains, ch.eof_chain, ch.d_start, r32, d_mark_blocks, d_pairs, d_np, t32, d_tsamp);
+    if (rate <= 0) {                                         // text samples only
+        cudaFreeAsync(ch.d_start, st);
+        return cudaGetLastError();
+    }
     CK(finish_headers(d_mark_blocks, nblk, 1, st));
     unsigned long long np = 0;
     CK(cudaMemcpyAsync(&np, d_np, 8, cudaMemcpyDeviceToHost, st));

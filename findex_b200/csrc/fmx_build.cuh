@@ -17,9 +17,11 @@ cudaError_t build_wmx(const uint8_t *d_bwt, int64_t n, uint32_t eof, const uint8
 // per-symbol planes: d_blocks holds sigma*nblk rank blocks; d_sym[code] = byte value
 cudaError_t build_planes(const uint8_t *d_bwt, int64_t n, uint32_t eof, const uint8_t *d_sym, int sigma, uint32_t *d_blocks,
                          int64_t nblk, cudaStream_t st);
-// sampled SA: marks rows with sa % rate == 0 (rank blocks, nblk) and stores their sa values in mark-rank order
+// sampled SA: marks rows with sa % rate == 0 (rank blocks, nblk) and stores their sa values in mark-rank order.  In the same chain walk,
+// d_tsamp != nullptr receives the text samples d_tsamp[v / text_rate] = row of T' position v for every v % text_rate == 0; rate = 0 walks
+// for the text samples alone (no marks, no samples)
 cudaError_t build_sa_samples(const DevIndex &ix, int layout, int rate, uint32_t *d_mark_blocks, int64_t nblk, uint32_t *d_samples,
-                             int64_t n_samples, cudaStream_t st, std::string &err);
+                             int64_t n_samples, cudaStream_t st, std::string &err, int text_rate = 0, uint32_t *d_tsamp = nullptr);
 // locate walk blocks (56 BWT bytes + 56 mark bits per 64 B); nwb = n/56 + 1
 cudaError_t build_walk_blocks(const uint8_t *d_bwt, const uint32_t *d_mark_blocks, int64_t n, uint8_t *d_bm, int64_t nwb, cudaStream_t st);
 // full suffix array, its inverse and T' (text[n-1] = 0) by the same chain walks

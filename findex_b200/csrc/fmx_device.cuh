@@ -80,6 +80,11 @@ struct DevIndex {
     uint64_t        dict_buckets;   // multiple of 4
     int32_t         dict_D, dict_bits;
     int32_t         dict_Dx, dict_Jc;   // deepest depth stored at all (= dict_D without chain entries); symbols per chain tier
+    // text samples (fmx_opts.text_sample_rate): tsamp[k] = row of the suffix at T' position k * tsamp_rate, k = 0 .. (n-1) / tsamp_rate —
+    // where an extract walk starts; sym[code] = the byte of a dense code (decodes the packed symbols of isat / ctx / ctx8)
+    const uint32_t *tsamp;
+    uint32_t        tsamp_rate;     // 0 = no samples
+    const uint8_t  *sym;
 };
 
 // Pattern accessors handed to search_pattern: operator()(i) = byte i; word(w) = bytes 4w..4w+3 packed little-endian (bytes at or

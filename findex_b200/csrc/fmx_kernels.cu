@@ -338,6 +338,107 @@ prev_substr_kernel(const __grid_constant__ DevIndex ix, const long long *__restr
     }
 }
 
+// ---- extract: the file bytes F[f .. f+len) = T'[q-1], T'[q-2], ... with q = n-1-f (fmx_text_batch / fmx_text_dev) --------------------
+// One work item per segment of at most kTextSegment output bytes: output bytes [a, b) of request j are T' positions [q-b, q-a), reached
+// from the sample at the first multiple of the sample rate at or above q-a (position n-1 = row 0 when that is past the text).  A step
+// from position x (row r) emits T'[x-1], T'[x-2], ... and keeps those inside the segment's positions:
+//   TEXT_ISAT: no walk — isat[p] holds T'[p .. p+isat_syms), independent loads from p = q-b on;
+//   TEXT_CTX : ctx[2r+1] = { isa[x-J], T'[x-J .. x-1] } — J symbols and the row J positions back in one 16-byte request;
+//   TEXT_CTX8: ctx8[r] = { isa[x-16], T'[x-16 .. x-1] as 2-bit codes }, LF steps for the last x < 16 positions (no hop there);
+//   TEXT_LF  : one LF step per symbol (BWT byte + rank), as prevSubstr.
+// STATS: *requests += the index requests the walks make (the sample, each entry / BWT byte / rank block).
+enum { kTextIsat = 0, kTextCtx = 1, kTextCtx8 = 2, kTextLf = 3 };
+constexpr int kTextSegment = 512;
+
+// the byte of packed symbol k of a 96-bit isat / ctx field (e.y, e.z, e.w): dense code + 1 -> byte, or the byte itself (raw contexts)
+__device__ __forceinline__ uint32_t text_sym(const uint4 &e, uint32_t k, uint32_t bits, bool raw, const uint8_t *sym) {
+    const uint32_t o = k * bits, w = o >> 5;
+    const uint32_t lo = w == 0 ? e.y : w == 1 ? e.z : e.w, hi = w == 0 ? e.z : w == 1 ? e.w : 0u;
+    const uint32_t v = __funnelshift_r(lo, hi, o & 31u) & ((1u << bits) - 1u);
+    return raw ? v : (uint32_t)sym[(v - 1u) & 0xFFu];
+}
+
+template <int G, int LAYOUT, int PATH, bool STATS>
+__global__ void __launch_bounds__(kThreads)
+text_kernel(const __grid_constant__ DevIndex ix, const uint32_t *__restrict__ off, long long m, int len, int nseg, uint8_t *__restrict__ out,
+            int *__restrict__ out_len, unsigned long long *__restrict__ requests) {
+    __shared__ SharedTables tb;
+    __shared__ uint8_t sym[256];
+    load_tables(tb, ix);
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) sym[i] = ix.sym[i];
+    __syncthreads();
+    const uint32_t t = blockIdx.x * (kThreads / G) + threadIdx.x / G;     // < 2^31: the launcher slices larger batches
+    if ((long long)t >= m * nseg) return;
+    const bool lead = (threadIdx.x % G) == 0;
+    const uint32_t j = t / (uint32_t)nseg;
+    const int s = (int)(t - j * (uint32_t)nseg);
+    const uint32_t f = off[j], last = ix.n - 1u;                  // |F| = n - 1
+    if (f > last) {                                              // only the device form gets here unchecked
+        if (s == 0 && lead) out_len[j] = -1;
+        return;
+    }
+    const uint32_t q = last - f;
+    const int olen = (int)min((uint32_t)len, q);
+    if (s == 0 && lead) out_len[j] = olen;
+    const int a = s * kTextSegment, b = min(a + kTextSegment, olen);
+    if (a >= b) return;
+    const uint32_t lo = q - (uint32_t)b, hi = q - (uint32_t)a;   // T' positions of this segment: [lo, hi)
+    uint8_t *row = out + (long long)j * len;
+#define FMX_PUT(P, V) (row[q - 1u - (P)] = (uint8_t)(V))            // T' position P is output byte q-1-P
+    uint64_t req = 0;
+    if constexpr (PATH == kTextIsat) {
+        const uint32_t bits = (uint32_t)ix.isat_bits, syms = (uint32_t)ix.isat_syms;
+        for (uint32_t p = lo; p < hi; p += syms) {
+            const uint4 e = ldg128(ix.isat + p);
+            const uint32_t cnt = min(syms, hi - p);
+            for (uint32_t k = 0; k < cnt; ++k) FMX_PUT(p + k, text_sym(e, k, bits, false, sym));
+            if (STATS) ++req;
+        }
+    } else {
+        const uint32_t rate = ix.tsamp_rate;
+        const uint64_t k0 = ((uint64_t)hi + rate - 1) / rate;
+        uint64_t x64 = k0 * rate;                                // 64-bit: near n = 2^32 - 2 the multiple overflows uint32
+        uint32_t r = 0;
+        if (x64 > last) x64 = last;                              // position n-1 (the '$' suffix) is row 0
+        else { r = ldg32(ix.tsamp + k0); if (STATS) ++req; }
+        uint32_t x = (uint32_t)x64;
+        if constexpr (PATH == kTextCtx) {
+            const uint32_t J = (uint32_t)ix.ctx_J, bits = (uint32_t)ix.isat_bits;
+            const bool raw = ix.ctx_raw != 0;
+            while (x > lo) {
+                const uint4 e = ldg128(ix.ctx + (uint64_t)r * 2 + 1);
+                if (STATS) ++req;
+                // symbol k of the entry is T'[x-J+k]; keep positions inside [lo, hi)
+                const uint32_t kmin = x >= J ? (lo > x - J ? lo - (x - J) : 0u) : J - x + lo;
+                const uint32_t kend = x <= hi ? J : x - hi >= J ? 0u : J - (x - hi);
+                for (uint32_t k = kmin; k < kend; ++k) FMX_PUT(x - J + k, text_sym(e, k, bits, raw, sym));
+                r = e.x;
+                x = x > J ? x - J : 0u;
+            }
+        } else if constexpr (PATH == kTextCtx8) {
+            constexpr uint32_t J = 16;
+            while (x > lo && x >= J) {
+                const uint2 e = ldg64(ix.ctx8 + r);
+                if (STATS) ++req;
+                const uint32_t kmin = lo > x - J ? lo - (x - J) : 0u, kend = x <= hi ? J : x - hi >= J ? 0u : J - (x - hi);
+                for (uint32_t k = kmin; k < kend; ++k) FMX_PUT(x - J + k, sym[(e.y >> (2 * k)) & 3u]);
+                r = e.x;
+                x -= J;
+            }
+        }
+        // LF steps: the whole walk (TEXT_LF), or the last x < 16 positions of a compact-context walk
+        const uint32_t per_step = 1u + (LAYOUT == FMX_LAYOUT_WM ? (uint32_t)ix.levels : LAYOUT == FMX_LAYOUT_WMX ? (uint32_t)ix.wmx_levels : 1u);
+        while (x > lo) {
+            const uint32_t c = ix.bwt[r];
+            if (x - 1u < hi && lead) FMX_PUT(x - 1u, c);
+            if (--x > lo) { r = lf_value<G, LAYOUT>(ix, tb, c, r); if (STATS) req += per_step; }
+            else if (STATS) ++req;
+        }
+    }
+#undef FMX_PUT
+    if (STATS && lead) atomicAdd(requests, (unsigned long long)req);
+}
+
 // FL step (getNextI, bwtmerger.scala:390-392: fm[i]) without the 4n-byte .fm array: the F-column symbol of row i
 // is the c with C[c] <= i < C[c+1]; the answer is the row of its (i-C[c])-th occurrence in the BWT, found by
 // binary search on rank_c.
@@ -697,6 +798,41 @@ cudaError_t launch_prev_substr(const DevIndex &ix, LaunchCfg cfg, const int64_t 
 #define CALL(G, LAY) prev_substr_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (const long long *)d_row, m, len, d_out)
     FMX_DISPATCH(cfg, CALL);
 #undef CALL
+    return cudaGetLastError();
+}
+
+int text_path(const DevIndex &ix) {
+    return ix.isat != nullptr ? kTextIsat : ix.tsamp == nullptr ? -1 : ix.ctx != nullptr ? kTextCtx : ix.ctx8 != nullptr ? kTextCtx8 : kTextLf;
+}
+
+cudaError_t launch_text(const DevIndex &ix, LaunchCfg cfg, const uint32_t *d_off, int64_t m, int len, uint8_t *d_out, int *d_out_len,
+                        unsigned long long *d_requests, cudaStream_t st) {
+    if (m <= 0) return cudaSuccess;
+    const int path = text_path(ix);
+    if (path < 0) return cudaErrorInvalidValue;
+    const int nseg = len > 0 ? (len + kTextSegment - 1) / kTextSegment : 1;
+    // the hop paths are one lane per segment (one request per entry); the LF walk shares each rank block among cfg.lanes lanes
+#define TEXT1(LAY, P) TEXTG(1, LAY, P)
+#define TEXTG(G, LAY, P)                                                                                                                  \
+    do {                                                                                                                                  \
+        if (d_requests) text_kernel<G, LAY, P, true><<<grid_for(mj * nseg, G), kThreads, 0, st>>>(ix, d_off + j0, mj, len, nseg, d_out + j0 * len, d_out_len + j0, d_requests); \
+        else text_kernel<G, LAY, P, false><<<grid_for(mj * nseg, G), kThreads, 0, st>>>(ix, d_off + j0, mj, len, nseg, d_out + j0 * len, d_out_len + j0, nullptr);          \
+    } while (0)
+#define CALL(G, LAY) TEXTG(G, LAY, kTextLf)
+    const int64_t slice = (1ll << 30) / nseg;                     // requests per launch: the kernel's work-item indices stay 32-bit
+    for (int64_t j0 = 0; j0 < m; j0 += slice) {
+        const int64_t mj = std::min(slice, m - j0);
+        if (path == kTextIsat) TEXT1(FMX_LAYOUT_PLANES, kTextIsat);
+        else if (path == kTextCtx) TEXT1(FMX_LAYOUT_PLANES, kTextCtx);
+        else if (path == kTextCtx8) {
+            if (cfg.layout == FMX_LAYOUT_PLANES) TEXT1(FMX_LAYOUT_PLANES, kTextCtx8);
+            else if (cfg.layout == FMX_LAYOUT_WMX) TEXT1(FMX_LAYOUT_WMX, kTextCtx8);
+            else TEXT1(FMX_LAYOUT_WM, kTextCtx8);
+        } else FMX_DISPATCH(cfg, CALL);
+    }
+#undef CALL
+#undef TEXTG
+#undef TEXT1
     return cudaGetLastError();
 }
 

@@ -44,6 +44,12 @@ cudaError_t launch_next_substr(const DevIndex &ix, LaunchCfg cfg, const int64_t 
 // prevSubstr: len LF steps per row, emitting the BWT byte at each visited row
 cudaError_t launch_prev_substr(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_row, int64_t m, int len,
                                uint8_t *d_out, cudaStream_t st);
+// extract: d_out row j (len bytes) = file bytes F[off[j] .. off[j] + out_len[j]), out_len[j] = min(len, n-1-off[j]) (-1 for off[j] > n-1).
+// The path follows what `ix` shows: isat, else (with text samples) ctx, ctx8 or LF steps; text_path = that choice (-1: neither isat nor
+// samples, the launch fails).  d_requests != nullptr: += the index requests of the walks (the counting instance of the kernel).
+int text_path(const DevIndex &ix);
+cudaError_t launch_text(const DevIndex &ix, LaunchCfg cfg, const uint32_t *d_off, int64_t m, int len, uint8_t *d_out, int *d_out_len,
+                        unsigned long long *d_requests, cudaStream_t st);
 // locate: one work item per occurrence of the queries [q0, q1) — occurrences [t0, t0 + count) of the batch, d_off[m+1] = exclusive
 // offsets over the whole batch; writes the unsorted sa values of the slab to d_pos[0 .. count), or — d_key != nullptr — the sort keys
 // ((query - q0) << 32 | sa value) of the per-query ordering to d_key[0 .. count)

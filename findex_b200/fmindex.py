@@ -39,7 +39,8 @@ class ReUnsupported(FmxError):
 class fmx_opts(C.Structure):
     _fields_ = [("device", C.c_int32), ("layout", C.c_int32), ("sa_sample_rate", C.c_int32), ("require_fm", C.c_int32),
                 ("max_index_bytes", C.c_int64), ("lanes_per_query", C.c_int32), ("accel", C.c_int32), ("kmer_table_bytes", C.c_int64),
-                ("max_total_bytes", C.c_int64), ("dict_bytes", C.c_int64), ("dict_min_rows", C.c_int32), ("dict_top_min_rows", C.c_int32)]
+                ("max_total_bytes", C.c_int64), ("dict_bytes", C.c_int64), ("dict_min_rows", C.c_int32), ("dict_top_min_rows", C.c_int32),
+                ("text_sample_rate", C.c_int32)]
 
 
 _lib = None
@@ -104,6 +105,9 @@ def lib():
     L.fmx_get_next_i_batch.argtypes = [p, p, i64, p]
     L.fmx_pos2char.argtypes = [p, i64, C.POINTER(i32)]
     L.fmx_prev_substr_batch.argtypes = [p, p, i64, i32, p, p]
+    L.fmx_text_sample_rate.argtypes = [p]
+    L.fmx_text_batch.argtypes = [p, p, i64, i32, p, p]
+    L.fmx_text_dev.argtypes = [p, p, i64, i32, p, p, p]
     L.fmx_next_substr_batch.argtypes = [p, p, i64, i32, p, p]
     L.fmx_regex_compile.argtypes = [p, i64, C.c_int, pp]
     L.fmx_regex_compile_engine.argtypes = [p, i64, C.c_int, C.c_int, pp]
@@ -161,7 +165,7 @@ def _u8(a):
 
 
 def make_opts(device=-1, layout=LAYOUT_AUTO, sa_sample_rate=0, require_fm=False, max_index_bytes=0, lanes_per_query=0, accel=ACCEL_AUTO,
-              kmer_table_bytes=0, max_total_bytes=0, dict_bytes=0, dict_min_rows=0, dict_top_min_rows=0):
+              kmer_table_bytes=0, max_total_bytes=0, dict_bytes=0, dict_min_rows=0, dict_top_min_rows=0, text_sample_rate=0):
     o = fmx_opts()
     lib().fmx_opts_default(C.byref(o))
     o.device, o.layout, o.sa_sample_rate = device, layout, sa_sample_rate
@@ -169,6 +173,7 @@ def make_opts(device=-1, layout=LAYOUT_AUTO, sa_sample_rate=0, require_fm=False,
     o.kmer_table_bytes = kmer_table_bytes
     o.max_total_bytes = max_total_bytes
     o.dict_bytes, o.dict_min_rows, o.dict_top_min_rows = dict_bytes, dict_min_rows, dict_top_min_rows
+    o.text_sample_rate = text_sample_rate
     return o
 
 
@@ -308,7 +313,7 @@ class GpuFMSearcher:
                 "dict_depth": dd.value, "dict_chain_depth": dx.value, "dict_entries": de.value, "dict_bytes": db.value,
                 "index_bytes": nb.value, "sa_sample_rate": rate.value, "kmer_k": k.value, "kmer_rows": lib().fmx_kmer_rows(self.h), "text_shortcut": bool(t.value),
                 "ctx_depth": lib().fmx_ctx_depth(self.h), "ctx_entry_bytes": lib().fmx_ctx_entry_bytes(self.h),
-                "lanes_per_query": lib().fmx_get_lanes(self.h)}
+                "lanes_per_query": lib().fmx_get_lanes(self.h), "text_sample_rate": lib().fmx_text_sample_rate(self.h)}
 
     # ---- scalar trait members (each is a batch of one) -------------------------------------------------
     def cf(self, c):
@@ -466,6 +471,23 @@ class GpuFMSearcher:
         lib().fmx_extract_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
         _check(lib().fmx_extract_batch(self.h, _ptr(rows), len(rows), ln, direction, _ptr(out), _ptr(olen)))
         return [out[i, :olen[i]].tobytes() for i in range(len(rows))]
+
+    def text(self, off, length):
+        """the indexed file bytes F[off .. off+length) (0x00 dropped; shorter at the end of the text)"""
+        return self.text_batch([off], length)[0]
+
+    def text_batch(self, offs, length):
+        """fmx_text_batch: F[off .. off+length) for every file offset in `offs` (0 <= off <= n-1); list of bytes"""
+        offs = _i64(offs)
+        out = np.zeros((len(offs), max(length, 1)), np.uint8)
+        olen = np.zeros(len(offs), np.int32)
+        _check(lib().fmx_text_batch(self.h, _ptr(offs), len(offs), length, _ptr(out), _ptr(olen)))
+        return [out[i, :olen[i]].tobytes() for i in range(len(offs))]
+
+    def text_dev(self, d_off, m, length, d_out, d_out_len, stream=0):
+        """fmx_text_dev (raw device pointers as ints): uint32 file offsets [m] in, uint8 [m, length] rows and int32 lengths out;
+        asynchronous on `stream`"""
+        _check(lib().fmx_text_dev(self.h, C.c_void_p(d_off), m, length, C.c_void_p(d_out), C.c_void_p(d_out_len), C.c_void_p(stream)))
 
     def regex_search_batch(self, trees, cap_total=1 << 20):
         """trees: list of ReTree.  Returns per regex the sorted list of (len, sp, ep)."""

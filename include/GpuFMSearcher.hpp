@@ -91,6 +91,16 @@ public:
         out.resize((size_t)ol);
         return out;
     }
+    // file bytes F[off .. off+len) (0x00 dropped; shorter at the text's end): needs fmx_opts.text_sample_rate or FMX_ACCEL_TEXT
+    std::string text(int64_t off, int len) const { return textBatch({off}, len)[0]; }
+    std::vector<std::string> textBatch(const std::vector<int64_t> &off, int len) const {
+        std::vector<uint8_t> out(off.size() * (size_t)(len > 0 ? len : 0) + 1);
+        std::vector<int32_t> ol(off.size() + 1);
+        check(fmx_text_batch(h_, off.data(), (int64_t)off.size(), len, out.data(), ol.data()));
+        std::vector<std::string> r;
+        for (size_t i = 0; i < off.size(); ++i) r.emplace_back(reinterpret_cast<const char *>(out.data()) + i * (size_t)len, (size_t)ol[i]);
+        return r;
+    }
     std::string nextSubstr(int64_t sp, int len) const {
         std::string out((size_t)(len > 0 ? len : 1), '\0'); int32_t ol = 0;
         check(fmx_next_substr_batch(h_, &sp, 1, len, reinterpret_cast<uint8_t *>(&out[0]), &ol));

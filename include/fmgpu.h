@@ -84,6 +84,8 @@ typedef struct fmx_opts {
                                    max(this, 8) rows: narrower ones are what the row contexts take in one fetch per row)                      */
     int32_t  dict_top_min_rows; /* threshold of the deepest keyed level D (where every pattern at least that long probes first); 0 = 1:
                                    everything that occurs twice, when it fits the budget, else dict_min_rows                                   */
+    int32_t  text_sample_rate;  /* 0 = none; s in 1..65536: the row of every s-th text position is kept (4 * ((n-1)/s + 1) bytes), which
+                                   fmx_text_batch / fmx_text_dev start their walks from                                                   */
 } fmx_opts;
 
 void        fmx_opts_default(fmx_opts *o);
@@ -184,8 +186,9 @@ int fmx_locate_dev(fmx_index *ix, const void *d_sp_u32, const void *d_ep_u32, in
 /* Occurrences per internal slab of the locate calls (default 2^30; 0 restores it).  A batch may hold any number of occurrences; it is
  * processed slab by slab.  Exposed so that tests can exercise the slab seams on small inputs.                                       */
 int fmx_set_locate_slab(int64_t occurrences);
-/* Roofline accounting: fmx_set_stats(ix, 1) makes locate calls count the LF steps of their walks (untimed runs only); regex searches
- * always count the items they process (one backward step each).  fmx_last_steps = that count for the last locate / regex call.      */
+/* Roofline accounting: fmx_set_stats(ix, 1) makes locate calls count the LF steps of their walks and text calls the index requests of
+ * theirs (untimed runs only); regex searches always count the items they process (one backward step each).  fmx_last_steps = that
+ * count for the last locate / text / regex call.                                                                                      */
 int     fmx_set_stats(fmx_index *ix, int32_t on);
 int64_t fmx_last_steps(const fmx_index *ix);
 /* Split of the last locate call's device time: LF walks vs the per-query sort.                              */
@@ -207,6 +210,21 @@ int fmx_prev_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t 
 int fmx_next_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t len, uint8_t *out, int32_t *out_len);
 /* Both walks under one name: direction > 0 = nextSubstr, else prevSubstr.                              */
 int fmx_extract_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t len, int32_t direction, uint8_t *out, int32_t *out_len);
+
+/* ---- extract: the indexed text at any file offset ------------------------------------------------------
+ * F = the indexed file bytes (0x00 dropped, as FileBWTReader reads them) = reverse(T'[0 .. n-2]), |F| = n-1.  Out row q (len bytes,
+ * row-major) = F[off[q] .. off[q] + out_len[q]), out_len[q] = min(len, n-1-off[q]).  From a located position: patterns are matched
+ * in T', so a length-k match at T' position p (fmx_locate_*) is reverse(pattern) at file offset (n-1) - p - k.
+ * A walk starts at the text sample at or after the request's end (fmx_opts.text_sample_rate) and goes backwards through T' by the row
+ * contexts' J-hops (FMX_ACCEL_CTX: J symbols per 16-byte request; FMX_ACCEL_CTX8: 16), else by LF steps; with the singleton shortcut
+ * (FMX_ACCEL_TEXT) the text is read directly, without samples.  What fmx_set_accel_mask hides is not used.
+ * FMX_E_UNSUPPORTED when the index has neither text samples nor a visible singleton shortcut; FMX_E_ARG for an offset outside
+ * [0, n-1], len < 0 or null pointers.  With fmx_set_stats(ix, 1), fmx_last_steps = the index requests of the last call's walks.      */
+int fmx_text_sample_rate(const fmx_index *ix);              /* 0 = no samples */
+int fmx_text_batch(fmx_index *ix, const int64_t *off, int64_t m, int32_t len, uint8_t *out, int32_t *out_len);
+/* device-resident, asynchronous on `stream`: d_off uint32[m] file offsets, d_out uint8[m*len], d_out_len int32[m]; an offset above
+ * n-1 is not checked on the host and yields out_len = -1                                                                               */
+int fmx_text_dev(fmx_index *ix, const void *d_off_u32, int64_t m, int32_t len, void *d_out, void *d_out_len, void *stream);
 
 /* ---- regex: REParser.re2post M/re2/re2.scala:50-185 + ReTree.apply M/re2/retree.scala:156-370 -------
  * Compiles on the host to the reference's Glushkov position automaton, quirks included (SURVEY Q1-Q5);
