@@ -65,9 +65,10 @@ struct DBuf {
     void *p = nullptr;
     cudaStream_t st;
     explicit DBuf(cudaStream_t s) : st(s) {}
+    DBuf(DBuf &&o) noexcept : p(o.p), st(o.st) { o.p = nullptr; }
     ~DBuf() { if (p) cudaFreeAsync(p, st); }
     cudaError_t alloc(size_t bytes) { return cudaMallocAsync(&p, bytes ? bytes : 1, st); }
-    template <typename T> T *as() { return reinterpret_cast<T *>(p); }
+    template <typename T> T *as() const { return reinterpret_cast<T *>(p); }
 };
 
 struct Events {                                                 // per-chunk events of a pipelined call, destroyed on every exit path
@@ -130,6 +131,81 @@ struct Timed {
     void stop() { cudaEventRecord(cc.ev1, cc.stream); }
     void collect() { float ms = 0; if (cudaEventElapsedTime(&ms, cc.ev0, cc.ev1) == cudaSuccess) ix->last_ms = ms; }
 };
+
+struct DeviceGuard {
+    int prev = -1;
+    explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
+    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+// A host-buffer call that is one kernel launch.  The inputs are copied in on the call's stream; then launch(d, cc) runs between the
+// call's timing events and counts as one launch, where d holds the device buffers of the inputs and then of the outputs, in the order
+// listed; then the outputs are copied back and the stream is synchronised.  An output marked `zero` starts zero-filled on the device.
+struct HostIn { const void *p; int64_t bytes; };
+struct HostOut { void *p; int64_t bytes; bool zero = false; };
+template <typename Launch>
+int one_launch_call(fmx_index *ix, std::initializer_list<HostIn> in, std::initializer_list<HostOut> out, Launch &&launch) {
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = cc.stream;
+    std::vector<DBuf> d;
+    d.reserve(in.size() + out.size());
+    for (const HostIn &b : in) {
+        d.emplace_back(st);
+        CU(d.back().alloc((size_t)b.bytes));
+        if (b.bytes) CU(cudaMemcpyAsync(d.back().p, b.p, (size_t)b.bytes, cudaMemcpyHostToDevice, st));
+    }
+    for (const HostOut &b : out) {
+        d.emplace_back(st);
+        CU(d.back().alloc((size_t)b.bytes));
+        if (b.zero) CU(cudaMemsetAsync(d.back().p, 0, (size_t)b.bytes, st));
+    }
+    Timed t(ix, cc);
+    CU(launch(d, cc));
+    ix->last_launches = 1; ix->total_launches += 1;
+    t.stop();
+    size_t i = in.size();
+    for (const HostOut &b : out) CU(cudaMemcpyAsync(b.p, d[i++].p, (size_t)b.bytes, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    t.collect();
+    return FMX_OK;
+}
+
+// The chunked pipeline of a host-buffer call: chunk k's inputs go in on cc.h2d, its kernels run on cc.stream and its results come
+// back on cc.d2h, each stage behind the previous one's event, so that the copies of chunks k+1 and k-1 overlap the kernels of chunk k
+// (PCIe is full duplex).  h2d / kernel / d2h(q0, nq) enqueue that stage for the items [q0, q0 + nq) and return its first error; the
+// first error ends the loop and is reported as FMX_E_CUDA naming `what`.  All three streams are drained, after an error too.
+template <typename H2D, typename Kernel, typename D2H>
+int chunk_pipeline(fmx_index *ix, CallCtx &cc, const char *what, int64_t m, int64_t chunk, int64_t launches_per_chunk, H2D &&h2d,
+                   Kernel &&kernel, D2H &&d2h) {
+    const int64_t nchunks = (m + chunk - 1) / chunk;
+    Events evs_in, evs_k;
+    CU(evs_in.make((size_t)nchunks)); CU(evs_k.make((size_t)nchunks));
+    // the copy streams may touch the stream-ordered allocations only after the allocating stream reached this point
+    CU(cudaEventRecord(cc.ev_alloc, cc.stream));
+    CU(cudaStreamWaitEvent(cc.h2d, cc.ev_alloc, 0));
+    CU(cudaStreamWaitEvent(cc.d2h, cc.ev_alloc, 0));
+    Timed t(ix, cc);
+    int rc = FMX_OK;
+    for (int64_t k = 0; k < nchunks && rc == FMX_OK; ++k) {
+        const int64_t q0 = k * chunk, nq = std::min(chunk, m - q0);
+        cudaError_t e = h2d(q0, nq);
+        if (e == cudaSuccess) e = cudaEventRecord(evs_in.v[(size_t)k], cc.h2d);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(cc.stream, evs_in.v[(size_t)k], 0);
+        if (e == cudaSuccess) e = kernel(q0, nq);
+        if (e == cudaSuccess) e = cudaEventRecord(evs_k.v[(size_t)k], cc.stream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(cc.d2h, evs_k.v[(size_t)k], 0);
+        if (e == cudaSuccess) e = d2h(q0, nq);
+        if (e != cudaSuccess) rc = fail(FMX_E_CUDA, "CUDA error %s in the %s pipeline (%s)", cudaGetErrorName(e), what, cudaGetErrorString(e));
+    }
+    ix->last_launches = nchunks * launches_per_chunk; ix->total_launches += nchunks * launches_per_chunk;
+    t.stop();
+    cudaError_t e1 = cudaStreamSynchronize(cc.h2d), e2 = cudaStreamSynchronize(cc.stream), e3 = cudaStreamSynchronize(cc.d2h);
+    if (rc == FMX_OK && (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess)) rc = fail(FMX_E_CUDA, "CUDA error while draining the %s pipeline", what);
+    t.collect();
+    return rc;
+}
 
 int ensure_device(int device, int *chosen) {
     int count = 0;
@@ -212,7 +288,6 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
     int lanes = o.lanes_per_query ? o.lanes_per_query : (wmx ? 4 : 2);      // re-tuned below once the accelerators are known
     if (lanes != 1 && lanes != 2 && lanes != 4) return fail(FMX_E_ARG, "lanes_per_query must be 1, 2 or 4");
     ix->cfg = LaunchCfg{layout, lanes};
-    if (const char *mb = std::getenv("FMX_MINB")) ix->cfg.min_blocks = std::atoi(mb);      // occupancy experiment (profiles/r01_count_design_sweep.jsonl)
     ix->index_bytes = (layout == FMX_LAYOUT_PLANES ? planes_bytes : wmx ? wmx_bytes : wm_bytes) + n;
 
     // base[c]: PLANES: C[c].  WM: C[c] - start_final[code], where after `levels` stable bit partitions the
@@ -565,12 +640,6 @@ struct Phases {
     }
 };
 
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-
 #define CHECK_IX(ix) do { if (!(ix)) return fail(FMX_E_ARG, "null index"); } while (0)
 
 }  // namespace
@@ -756,22 +825,9 @@ int fmx_occ_batch(fmx_index *ix, const uint8_t *c, const int64_t *key, int64_t m
     CHECK_IX(ix);
     if (m < 0 || (m && (!c || !key || !out))) return fail(FMX_E_ARG, "bad argument");
     if (m == 0) return FMX_OK;
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dc(st), dk(st), dout(st);
-    CU(dc.alloc(m)); CU(dk.alloc(m * 8)); CU(dout.alloc(m * 8));
-    CU(cudaMemcpyAsync(dc.p, c, m, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(dk.p, key, m * 8, cudaMemcpyHostToDevice, st));
-    Timed t(ix, cc);
-    CU(launch_occ(cc.d, cc.cfg, dc.as<uint8_t>(), dk.as<int64_t>(), m, dout.as<int64_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(out, dout.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
-    return FMX_OK;
+    return one_launch_call(ix, {{c, m}, {key, m * 8}}, {{out, m * 8}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_occ(cc.d, cc.cfg, d[0].as<uint8_t>(), d[1].as<int64_t>(), m, d[2].as<int64_t>(), cc.stream);
+    });
 }
 
 int fmx_prev_range_batch(fmx_index *ix, const int64_t *sp, const int64_t *ep, const uint8_t *c, int64_t m, int64_t *sp1, int64_t *ep1) {
@@ -780,24 +836,9 @@ int fmx_prev_range_batch(fmx_index *ix, const int64_t *sp, const int64_t *ep, co
     if (m == 0) return FMX_OK;
     for (int64_t i = 0; i < m; ++i)
         if (sp[i] < 0 || ep[i] < 0 || sp[i] > ix->n || ep[i] > ix->n) return fail(FMX_E_ARG, "row out of range at %lld", (long long)i);
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dsp(st), dep(st), dc(st), o1(st), o2(st);
-    CU(dsp.alloc(m * 8)); CU(dep.alloc(m * 8)); CU(dc.alloc(m)); CU(o1.alloc(m * 8)); CU(o2.alloc(m * 8));
-    CU(cudaMemcpyAsync(dsp.p, sp, m * 8, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(dep.p, ep, m * 8, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(dc.p, c, m, cudaMemcpyHostToDevice, st));
-    Timed t(ix, cc);
-    CU(launch_prev_range(cc.d, cc.cfg, dsp.as<int64_t>(), dep.as<int64_t>(), dc.as<uint8_t>(), m, o1.as<int64_t>(), o2.as<int64_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(sp1, o1.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(ep1, o2.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
-    return FMX_OK;
+    return one_launch_call(ix, {{sp, m * 8}, {ep, m * 8}, {c, m}}, {{sp1, m * 8}, {ep1, m * 8}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_prev_range(cc.d, cc.cfg, d[0].as<int64_t>(), d[1].as<int64_t>(), d[2].as<uint8_t>(), m, d[3].as<int64_t>(), d[4].as<int64_t>(), cc.stream);
+    });
 }
 
 int fmx_interval_prev_range(fmx_index *ix, int64_t sp, int64_t ep, int cstart, int cend, int32_t *out_c, int64_t *out_sp,
@@ -809,21 +850,11 @@ int fmx_interval_prev_range(fmx_index *ix, int64_t sp, int64_t ep, int cstart, i
     const int m = cend - cstart + 1;
     if (m <= 0) return FMX_OK;
     if (!out_c || !out_sp || !out_ep) return fail(FMX_E_ARG, "null argument");
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf o1(st), o2(st);
-    CU(o1.alloc(m * 8)); CU(o2.alloc(m * 8));
-    Timed t(ix, cc);
-    CU(launch_interval_prev_range(cc.d, cc.cfg, sp, ep, cstart, cend, o1.as<int64_t>(), o2.as<int64_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
     std::vector<int64_t> a(m), b(m);
-    CU(cudaMemcpyAsync(a.data(), o1.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(b.data(), o2.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
+    const int rc = one_launch_call(ix, {}, {{a.data(), m * 8}, {b.data(), m * 8}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_interval_prev_range(cc.d, cc.cfg, sp, ep, cstart, cend, d[0].as<int64_t>(), d[1].as<int64_t>(), cc.stream);
+    });
+    if (rc) return rc;
     int64_t k = 0;
     for (int c = cend; c >= cstart; --c)                       // the reference prepends while c ascends
         if (a[c - cstart] < b[c - cstart]) { out_c[k] = c; out_sp[k] = a[c - cstart]; out_ep[k] = b[c - cstart]; ++k; }
@@ -921,55 +952,31 @@ static int count_fixed_pipeline(fmx_index *ix, const uint8_t *pat, int32_t len, 
     CU(dsp.alloc(m * ((only_counts || narrow) ? 4 : 8))); CU(dep.alloc(m * ((only_counts || narrow) ? 4 : 8)));
     if (only_counts) CU(dcnt.alloc(m * 4));
     const int64_t chunk = cc.chunk_queries > 0 ? cc.chunk_queries : (1 << 20);
-    const int64_t nchunks = (m + chunk - 1) / chunk;
-    Events evs_in, evs_k;
-    CU(evs_in.make((size_t)nchunks)); CU(evs_k.make((size_t)nchunks));
-    std::vector<cudaEvent_t> &ev_in = evs_in.v, &ev_k = evs_k.v;
-    // the copy streams may touch the stream-ordered allocations only after the allocating stream reached this point
-    CU(cudaEventRecord(cc.ev_alloc, st));
-    CU(cudaStreamWaitEvent(cc.h2d, cc.ev_alloc, 0));
-    CU(cudaStreamWaitEvent(cc.d2h, cc.ev_alloc, 0));
-    Timed t(ix, cc);
-    int rc = FMX_OK;
-    for (int64_t k = 0; k < nchunks && rc == FMX_OK; ++k) {
-        const int64_t q0 = k * chunk, nq = std::min(chunk, m - q0);
-        cudaError_t e = cudaSuccess;
-        uint8_t *wire_dst = packed ? dwire.as<uint8_t>() + q0 * wire_len : dp.as<uint8_t>() + q0 * len;
-        if (len) e = cudaMemcpyAsync(wire_dst, pat + q0 * wire_len, (size_t)nq * wire_len, cudaMemcpyHostToDevice, cc.h2d);
-        if (e == cudaSuccess) e = cudaEventRecord(ev_in[(size_t)k], cc.h2d);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(st, ev_in[(size_t)k], 0);
-        if (e == cudaSuccess && packed && len) e = launch_unpack2(wire_dst, len, nq, alpha4, dp.as<uint8_t>() + q0 * len, st);
-        if (e == cudaSuccess) {
+    auto wire = [&](int64_t q0) { return packed ? dwire.as<uint8_t>() + q0 * wire_len : dp.as<uint8_t>() + q0 * len; };
+    return chunk_pipeline(ix, cc, "count", m, chunk, packed ? 2 : 1,
+        [&](int64_t q0, int64_t nq) {
+            return len ? cudaMemcpyAsync(wire(q0), pat + q0 * wire_len, (size_t)nq * wire_len, cudaMemcpyHostToDevice, cc.h2d) : cudaSuccess;
+        },
+        [&](int64_t q0, int64_t nq) {
+            if (packed && len) {
+                const cudaError_t e = launch_unpack2(wire(q0), len, nq, alpha4, dp.as<uint8_t>() + q0 * len, st);
+                if (e != cudaSuccess) return e;
+            }
             if (only_counts) {                       // ep-sp lands in dcnt through the kernel's fused-exchange sink; only that goes back
                 PeerSinks ps{};
                 ps.n = 1; ps.offset = q0; ps.p[0] = dcnt.as<uint32_t>();
-                e = launch_count_fixed(cc.d, cc.cfg, dp.as<uint8_t>() + q0 * len, len, nq, dsp.as<uint32_t>() + q0, dep.as<uint32_t>() + q0, false, nullptr, st, &ps);
-            } else if (narrow) {
-                e = launch_count_fixed(cc.d, cc.cfg, dp.as<uint8_t>() + q0 * len, len, nq, dsp.as<uint32_t>() + q0, dep.as<uint32_t>() + q0, false, nullptr, st);
-            } else {
-                e = launch_count_fixed(cc.d, cc.cfg, dp.as<uint8_t>() + q0 * len, len, nq, dsp.as<int64_t>() + q0, dep.as<int64_t>() + q0, true, nullptr, st);
+                return launch_count_fixed(cc.d, cc.cfg, dp.as<uint8_t>() + q0 * len, len, nq, dsp.as<uint32_t>() + q0, dep.as<uint32_t>() + q0, false, nullptr, st, &ps);
             }
-        }
-        if (e == cudaSuccess) e = cudaEventRecord(ev_k[(size_t)k], st);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(cc.d2h, ev_k[(size_t)k], 0);
-        if (only_counts) {
-            if (e == cudaSuccess) e = cudaMemcpyAsync(counts + q0, dcnt.as<uint32_t>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
-        } else if (narrow) {
-            if (e == cudaSuccess) e = cudaMemcpyAsync(sp32 + q0, dsp.as<uint32_t>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(ep32 + q0, dep.as<uint32_t>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
-        } else {
-            if (e == cudaSuccess) e = cudaMemcpyAsync(sp + q0, dsp.as<int64_t>() + q0, (size_t)nq * 8, cudaMemcpyDeviceToHost, cc.d2h);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(ep + q0, dep.as<int64_t>() + q0, (size_t)nq * 8, cudaMemcpyDeviceToHost, cc.d2h);
-        }
-        if (e != cudaSuccess) rc = fail(FMX_E_CUDA, "CUDA error %s in the count pipeline (%s)", cudaGetErrorName(e), cudaGetErrorString(e));
-    }
-    ix->last_launches = nchunks * (packed ? 2 : 1); ix->total_launches += nchunks * (packed ? 2 : 1);
-    t.stop();
-    cudaError_t e1 = cudaStreamSynchronize(cc.h2d), e2 = cudaStreamSynchronize(st), e3 = cudaStreamSynchronize(cc.d2h);
-    if (rc == FMX_OK && (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess))
-        rc = fail(FMX_E_CUDA, "CUDA error while draining the count pipeline");
-    t.collect();
-    return rc;
+            if (narrow) return launch_count_fixed(cc.d, cc.cfg, dp.as<uint8_t>() + q0 * len, len, nq, dsp.as<uint32_t>() + q0, dep.as<uint32_t>() + q0, false, nullptr, st);
+            return launch_count_fixed(cc.d, cc.cfg, dp.as<uint8_t>() + q0 * len, len, nq, dsp.as<int64_t>() + q0, dep.as<int64_t>() + q0, true, nullptr, st);
+        },
+        [&](int64_t q0, int64_t nq) {
+            if (only_counts) return cudaMemcpyAsync(counts + q0, dcnt.as<uint32_t>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
+            const size_t row = narrow ? 4 : 8;
+            void *hsp = narrow ? (void *)(sp32 + q0) : (void *)(sp + q0), *hep = narrow ? (void *)(ep32 + q0) : (void *)(ep + q0);
+            const cudaError_t e = cudaMemcpyAsync(hsp, dsp.as<uint8_t>() + q0 * row, nq * row, cudaMemcpyDeviceToHost, cc.d2h);
+            return e != cudaSuccess ? e : cudaMemcpyAsync(hep, dep.as<uint8_t>() + q0 * row, nq * row, cudaMemcpyDeviceToHost, cc.d2h);
+        });
 }
 
 int fmx_count_fixed(fmx_index *ix, const uint8_t *pat, int32_t len, int64_t m, int64_t *sp, int64_t *ep) {
@@ -1015,23 +1022,9 @@ int fmx_count_batch(fmx_index *ix, const uint8_t *pat, const int64_t *off, int64
     for (int64_t i = 0; i < m; ++i) if (off[i + 1] < off[i] || off[i] < 0) return fail(FMX_E_ARG, "offsets must be non-decreasing");
     const int64_t nbytes = off[m];
     if (nbytes && !pat) return fail(FMX_E_ARG, "null pattern buffer");
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dp(st), doff(st), dsp(st), dep(st);
-    CU(dp.alloc(nbytes)); CU(doff.alloc((m + 1) * 8)); CU(dsp.alloc(m * 8)); CU(dep.alloc(m * 8));
-    if (nbytes) CU(cudaMemcpyAsync(dp.p, pat, nbytes, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(doff.p, off, (m + 1) * 8, cudaMemcpyHostToDevice, st));
-    Timed t(ix, cc);
-    CU(launch_count_var(cc.d, cc.cfg, dp.as<uint8_t>(), doff.as<int64_t>(), m, dsp.as<int64_t>(), dep.as<int64_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(sp, dsp.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(ep, dep.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
-    return FMX_OK;
+    return one_launch_call(ix, {{pat, nbytes}, {off, (m + 1) * 8}}, {{sp, m * 8}, {ep, m * 8}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_count_var(cc.d, cc.cfg, d[0].as<uint8_t>(), d[1].as<int64_t>(), m, d[2].as<int64_t>(), d[3].as<int64_t>(), cc.stream);
+    });
 }
 
 int fmx_count_fixed_stats(fmx_index *ix, const uint8_t *pat, int32_t len, int64_t m, int64_t *blocks, int64_t *steps) {
@@ -1060,21 +1053,9 @@ int fmx_get_prev_i_batch(fmx_index *ix, const int64_t *row, int64_t m, int64_t *
     if (m < 0 || (m && (!row || !out))) return fail(FMX_E_ARG, "bad argument");
     if (m == 0) return FMX_OK;
     for (int64_t i = 0; i < m; ++i) if (row[i] < 0 || row[i] >= ix->n) return fail(FMX_E_ARG, "row out of range at %lld", (long long)i);
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dr(st), dout(st);
-    CU(dr.alloc(m * 8)); CU(dout.alloc(m * 8));
-    CU(cudaMemcpyAsync(dr.p, row, m * 8, cudaMemcpyHostToDevice, st));
-    Timed t(ix, cc);
-    CU(launch_lf(cc.d, cc.cfg, dr.as<int64_t>(), m, dout.as<int64_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(out, dout.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
-    return FMX_OK;
+    return one_launch_call(ix, {{row, m * 8}}, {{out, m * 8}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_lf(cc.d, cc.cfg, d[0].as<int64_t>(), m, d[1].as<int64_t>(), cc.stream);
+    });
 }
 
 int fmx_prev_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t len, uint8_t *out, int32_t *out_len) {
@@ -1084,21 +1065,9 @@ int fmx_prev_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t 
     for (int64_t i = 0; i < m; ++i) if (row[i] < 0 || row[i] >= ix->n) return fail(FMX_E_ARG, "row out of range at %lld", (long long)i);
     if (out_len) for (int64_t i = 0; i < m; ++i) out_len[i] = len;      // prevSubstr never stops early (its eof flag is never set)
     if (len == 0) return FMX_OK;
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dr(st), dout(st);
-    CU(dr.alloc(m * 8)); CU(dout.alloc((size_t)m * len));
-    CU(cudaMemcpyAsync(dr.p, row, m * 8, cudaMemcpyHostToDevice, st));
-    Timed t(ix, cc);
-    CU(launch_prev_substr(cc.d, cc.cfg, dr.as<int64_t>(), m, len, dout.as<uint8_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(out, dout.p, (size_t)m * len, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
-    return FMX_OK;
+    return one_launch_call(ix, {{row, m * 8}}, {{out, m * len}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_prev_substr(cc.d, cc.cfg, d[0].as<int64_t>(), m, len, d[1].as<uint8_t>(), cc.stream);
+    });
 }
 
 int fmx_get_next_i_batch(fmx_index *ix, const int64_t *row, int64_t m, int64_t *out) {
@@ -1106,21 +1075,9 @@ int fmx_get_next_i_batch(fmx_index *ix, const int64_t *row, int64_t m, int64_t *
     if (m < 0 || (m && (!row || !out))) return fail(FMX_E_ARG, "bad argument");
     if (m == 0) return FMX_OK;
     for (int64_t i = 0; i < m; ++i) if (row[i] < 0 || row[i] >= ix->n) return fail(FMX_E_ARG, "row out of range at %lld", (long long)i);
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dr(st), dout(st);
-    CU(dr.alloc(m * 8)); CU(dout.alloc(m * 8));
-    CU(cudaMemcpyAsync(dr.p, row, m * 8, cudaMemcpyHostToDevice, st));
-    Timed t(ix, cc);
-    CU(launch_fl(cc.d, cc.cfg, dr.as<int64_t>(), m, dout.as<int64_t>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(out, dout.p, m * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
-    return FMX_OK;
+    return one_launch_call(ix, {{row, m * 8}}, {{out, m * 8}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_fl(cc.d, cc.cfg, d[0].as<int64_t>(), m, d[1].as<int64_t>(), cc.stream);
+    });
 }
 
 int fmx_next_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t len, uint8_t *out, int32_t *out_len) {
@@ -1129,22 +1086,10 @@ int fmx_next_substr_batch(fmx_index *ix, const int64_t *row, int64_t m, int32_t 
     if (m == 0) return FMX_OK;
     for (int64_t i = 0; i < m; ++i) if (row[i] < 0 || row[i] >= ix->n) return fail(FMX_E_ARG, "row out of range at %lld", (long long)i);
     if (len == 0) { for (int64_t i = 0; i < m; ++i) out_len[i] = 0; return FMX_OK; }
-    CallCtx cc(ix);
-    CHECK_CC(cc);
-    DeviceGuard g(ix->device);
-    cudaStream_t st = cc.stream;
-    DBuf dr(st), dout(st), dlen(st);
-    CU(dr.alloc(m * 8)); CU(dout.alloc((size_t)m * len)); CU(dlen.alloc(m * 4));
-    CU(cudaMemcpyAsync(dr.p, row, m * 8, cudaMemcpyHostToDevice, st));
-    CU(cudaMemsetAsync(dout.p, 0, (size_t)m * len, st));
-    Timed t(ix, cc);
-    CU(launch_next_substr(cc.d, cc.cfg, dr.as<int64_t>(), m, len, dout.as<uint8_t>(), dlen.as<int>(), st));
-    ix->last_launches = 1; ix->total_launches += 1;
-    t.stop();
-    CU(cudaMemcpyAsync(out, dout.p, (size_t)m * len, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(out_len, dlen.p, m * 4, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    t.collect();
+    const int rc = one_launch_call(ix, {{row, m * 8}}, {{out, m * len, true}, {out_len, m * 4}}, [&](const std::vector<DBuf> &d, CallCtx &cc) {
+        return launch_next_substr(cc.d, cc.cfg, d[0].as<int64_t>(), m, len, d[1].as<uint8_t>(), d[2].as<int>(), cc.stream);
+    });
+    if (rc) return rc;
     for (int64_t i = 0; i < m; ++i) std::reverse(out + i * len, out + i * len + out_len[i]);     // ret.reverse.toString
     return FMX_OK;
 }
@@ -1177,32 +1122,16 @@ int fmx_text_batch(fmx_index *ix, const int64_t *off, int64_t m, int32_t len, ui
     if (cc.stats) { CU(dreq.alloc(8)); CU(cudaMemsetAsync(dreq.p, 0, 8, st)); }
     // chunks of about 64 MiB of output (at least 2^12 requests), or the caller's fmx_set_chunk
     const int64_t chunk = cc.chunk_queries > 0 ? cc.chunk_queries : std::max<int64_t>(1 << 12, (64ll << 20) / std::max<int32_t>(len, 1));
-    const int64_t nchunks = (m + chunk - 1) / chunk;
-    Events evs_in, evs_k;
-    CU(evs_in.make((size_t)nchunks)); CU(evs_k.make((size_t)nchunks));
-    CU(cudaEventRecord(cc.ev_alloc, st));
-    CU(cudaStreamWaitEvent(cc.h2d, cc.ev_alloc, 0));
-    CU(cudaStreamWaitEvent(cc.d2h, cc.ev_alloc, 0));
-    Timed t(ix, cc);
-    int rc = FMX_OK;
-    for (int64_t k = 0; k < nchunks && rc == FMX_OK; ++k) {
-        const int64_t q0 = k * chunk, nq = std::min(chunk, m - q0);
-        cudaError_t e = cudaMemcpyAsync(doff.as<uint32_t>() + q0, off32.data() + q0, (size_t)nq * 4, cudaMemcpyHostToDevice, cc.h2d);
-        if (e == cudaSuccess) e = cudaEventRecord(evs_in.v[(size_t)k], cc.h2d);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(st, evs_in.v[(size_t)k], 0);
-        if (e == cudaSuccess) e = launch_text(cc.d, cc.cfg, doff.as<uint32_t>() + q0, nq, len, dout.as<uint8_t>() + q0 * len, dlen.as<int>() + q0,
-                                              cc.stats ? dreq.as<unsigned long long>() : nullptr, st);
-        if (e == cudaSuccess) e = cudaEventRecord(evs_k.v[(size_t)k], st);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(cc.d2h, evs_k.v[(size_t)k], 0);
-        if (e == cudaSuccess && len) e = cudaMemcpyAsync(out + q0 * len, dout.as<uint8_t>() + q0 * len, (size_t)nq * len, cudaMemcpyDeviceToHost, cc.d2h);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(out_len + q0, dlen.as<int>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
-        if (e != cudaSuccess) rc = fail(FMX_E_CUDA, "CUDA error %s in the extract pipeline (%s)", cudaGetErrorName(e), cudaGetErrorString(e));
-    }
-    ix->last_launches = nchunks; ix->total_launches += nchunks;
-    t.stop();
-    cudaError_t e1 = cudaStreamSynchronize(cc.h2d), e2 = cudaStreamSynchronize(st), e3 = cudaStreamSynchronize(cc.d2h);
-    if (rc == FMX_OK && (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess)) rc = fail(FMX_E_CUDA, "CUDA error while draining the extract pipeline");
-    t.collect();
+    const int rc = chunk_pipeline(ix, cc, "extract", m, chunk, 1,
+        [&](int64_t q0, int64_t nq) { return cudaMemcpyAsync(doff.as<uint32_t>() + q0, off32.data() + q0, (size_t)nq * 4, cudaMemcpyHostToDevice, cc.h2d); },
+        [&](int64_t q0, int64_t nq) {
+            return launch_text(cc.d, cc.cfg, doff.as<uint32_t>() + q0, nq, len, dout.as<uint8_t>() + q0 * len, dlen.as<int>() + q0,
+                               cc.stats ? dreq.as<unsigned long long>() : nullptr, st);
+        },
+        [&](int64_t q0, int64_t nq) {
+            const cudaError_t e = len ? cudaMemcpyAsync(out + q0 * len, dout.as<uint8_t>() + q0 * len, (size_t)nq * len, cudaMemcpyDeviceToHost, cc.d2h) : cudaSuccess;
+            return e != cudaSuccess ? e : cudaMemcpyAsync(out_len + q0, dlen.as<int>() + q0, (size_t)nq * 4, cudaMemcpyDeviceToHost, cc.d2h);
+        });
     if (rc == FMX_OK && cc.stats) {
         unsigned long long h = 0;
         CU(cudaMemcpy(&h, dreq.p, 8, cudaMemcpyDeviceToHost));

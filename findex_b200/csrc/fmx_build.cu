@@ -562,16 +562,13 @@ cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d
     if (K >= 2) CK(cudaMallocAsync(&d_tmp, size[(size_t)K - 1] * sizeof(uint2), st));
     auto buf = [&](int level) { return ((K - level) % 2 == 0) ? d_table : d_tmp; };      // level K lands in d_table
     kmer_level1_kernel<<<(sigma + 255) / 256, 256, 0, st>>>(ix, d_sym, sigma, buf(1));
-    const int G = (cfg.lanes == 1 || cfg.lanes == 2 || cfg.lanes == 4) ? cfg.lanes : 2;
     for (int j = 2; j <= K; ++j) {
         const unsigned long long cnt = size[(size_t)j];
-        const unsigned long long per = kThreads / G;
+        const unsigned long long per = kThreads / cfg.lanes;
         const unsigned grid = (unsigned)((cnt + per - 1) / per);
-#define CALL(GG, LAY) kmer_extend_kernel<GG, LAY><<<grid, kThreads, 0, st>>>(ix, d_sym, sigma, buf(j - 1), cnt, lex, buf(j))
-        if (ix.layout == FMX_LAYOUT_PLANES) { if (G == 1) CALL(1, FMX_LAYOUT_PLANES); else if (G == 2) CALL(2, FMX_LAYOUT_PLANES); else CALL(4, FMX_LAYOUT_PLANES); }
-        else if (ix.layout == FMX_LAYOUT_WMX) { if (G == 1) CALL(1, FMX_LAYOUT_WMX); else if (G == 2) CALL(2, FMX_LAYOUT_WMX); else CALL(4, FMX_LAYOUT_WMX); }
-        else { if (G == 1) CALL(1, FMX_LAYOUT_WM); else if (G == 2) CALL(2, FMX_LAYOUT_WM); else CALL(4, FMX_LAYOUT_WM); }
-#undef CALL
+        dispatch_layout_lanes(ix.layout, cfg.lanes, [&](auto g, auto lay) {
+            kmer_extend_kernel<g, lay><<<grid, kThreads, 0, st>>>(ix, d_sym, sigma, buf(j - 1), cnt, lex, buf(j));
+        });
         CK(cudaGetLastError());
     }
     if (d_tmp) cudaFreeAsync(d_tmp, st);
@@ -747,9 +744,8 @@ cudaError_t build_dict(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, 
     dict_seed_kernel<<<(unsigned)((table_entries + 255) / 256), 256, 0, st>>>(ix.kmer, table_entries, sigma, K, (uint32_t)bits, min_rows, items, cap, d_cnt);
     unsigned long long lvl_begin = 0, lvl_count = seeds, total = seeds;
     int D = K;
-    const int G = (cfg.lanes == 1 || cfg.lanes == 2 || cfg.lanes == 4) ? cfg.lanes : 2;
     for (int d = K + 1; d <= Dmax + kDictMaxTiers * Jc && lvl_count > 0; ++d) {
-        const unsigned long long groups = lvl_count * sigma, per = kThreads / G;
+        const unsigned long long groups = lvl_count * sigma, per = kThreads / cfg.lanes;
         if ((groups + per - 1) / per > 0x7FFFFFFFull) break;
         const unsigned grid = (unsigned)((groups + per - 1) / per);
         // the deepest level the key can hold is where every pattern of at least that length probes first and nothing is grown from: it may
@@ -758,11 +754,9 @@ cudaError_t build_dict(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, 
         const uint32_t lvl_rows = d > Dmax ? std::max<uint32_t>(min_rows, kCtxMaxRows) : min_rows;
         uint32_t keep = (d == Dmax && min_rows_top < min_rows) ? min_rows_top : lvl_rows;
         for (;;) {
-#define CALL(GG, LAY) dict_extend_kernel<GG, LAY><<<grid, kThreads, 0, st>>>(ix, d_sym, sigma, items + lvl_begin, lvl_count, d, Dmax, Jc, (uint32_t)bits, keep, items, cap, d_cnt)
-            if (ix.layout == FMX_LAYOUT_PLANES) { if (G == 1) CALL(1, FMX_LAYOUT_PLANES); else if (G == 2) CALL(2, FMX_LAYOUT_PLANES); else CALL(4, FMX_LAYOUT_PLANES); }
-            else if (ix.layout == FMX_LAYOUT_WMX) { if (G == 1) CALL(1, FMX_LAYOUT_WMX); else if (G == 2) CALL(2, FMX_LAYOUT_WMX); else CALL(4, FMX_LAYOUT_WMX); }
-            else { if (G == 1) CALL(1, FMX_LAYOUT_WM); else if (G == 2) CALL(2, FMX_LAYOUT_WM); else CALL(4, FMX_LAYOUT_WM); }
-#undef CALL
+            dispatch_layout_lanes(ix.layout, cfg.lanes, [&](auto g, auto lay) {
+                dict_extend_kernel<g, lay><<<grid, kThreads, 0, st>>>(ix, d_sym, sigma, items + lvl_begin, lvl_count, d, Dmax, Jc, (uint32_t)bits, keep, items, cap, d_cnt);
+            });
             CK(cudaGetLastError());
             CK(cudaMemcpyAsync(&h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));

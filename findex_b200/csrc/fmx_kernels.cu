@@ -652,23 +652,6 @@ gather_kernel(const uint4 *__restrict__ base, unsigned long long n_units, long l
 // =====================================================================================================
 // launchers
 // =====================================================================================================
-#define FMX_DISPATCH(cfg, CALL)                                                                      \
-    do {                                                                                             \
-        if ((cfg).layout == FMX_LAYOUT_PLANES) {                                                     \
-            if ((cfg).lanes == 1) { CALL(1, FMX_LAYOUT_PLANES); }                                    \
-            else if ((cfg).lanes == 2) { CALL(2, FMX_LAYOUT_PLANES); }                               \
-            else { CALL(4, FMX_LAYOUT_PLANES); }                                                     \
-        } else if ((cfg).layout == FMX_LAYOUT_WMX) {                                                 \
-            if ((cfg).lanes == 1) { CALL(1, FMX_LAYOUT_WMX); }                                       \
-            else if ((cfg).lanes == 2) { CALL(2, FMX_LAYOUT_WMX); }                                  \
-            else { CALL(4, FMX_LAYOUT_WMX); }                                                        \
-        } else {                                                                                     \
-            if ((cfg).lanes == 1) { CALL(1, FMX_LAYOUT_WM); }                                        \
-            else if ((cfg).lanes == 2) { CALL(2, FMX_LAYOUT_WM); }                                   \
-            else { CALL(4, FMX_LAYOUT_WM); }                                                         \
-        }                                                                                            \
-    } while (0)
-
 static inline unsigned grid_for(int64_t items, int lanes) {
     const int64_t per = kThreads / lanes;
     return (unsigned)((items + per - 1) / per);
@@ -703,46 +686,33 @@ cudaError_t launch_count_fixed(const DevIndex &ix, LaunchCfg cfg, const uint8_t 
             k<<<grid1, kThreads, smem1, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, list, cnt, sinks);
         }
         const unsigned grid2 = grid_for(m, cfg.lanes);
-#define CALL2(G, LAY)                                                                                                  \
-        {                                                                                                              \
-            const size_t smem2 = (size_t)(kThreads / G) * (size_t)((len + 3) & ~3) + 16;                               \
-            if (out64) count_list_kernel<G, LAY, long long><<<grid2, kThreads, smem2, st>>>(ix, d_pat, len, (long long *)d_sp, (long long *)d_ep, list, cnt, sinks); \
-            else count_list_kernel<G, LAY, uint32_t><<<grid2, kThreads, smem2, st>>>(ix, d_pat, len, (uint32_t *)d_sp, (uint32_t *)d_ep, list, cnt, sinks); \
-        }
-        FMX_DISPATCH(cfg, CALL2);
-#undef CALL2
+        dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+            const size_t smem2 = (size_t)(kThreads / g) * (size_t)((len + 3) & ~3) + 16;
+            if (out64) count_list_kernel<g, lay, long long><<<grid2, kThreads, smem2, st>>>(ix, d_pat, len, (long long *)d_sp, (long long *)d_ep, list, cnt, sinks);
+            else count_list_kernel<g, lay, uint32_t><<<grid2, kThreads, smem2, st>>>(ix, d_pat, len, (uint32_t *)d_sp, (uint32_t *)d_ep, list, cnt, sinks);
+        });
         cudaFreeAsync(cnt, st);
         return cudaGetLastError();
     }
-#define CALL(G, LAY)                                                                                                  \
-    {                                                                                                                 \
-        if (too_long && !d_stats) {                                                                                   \
-            if (out64) count_fixed_gmem_kernel<G, LAY, long long><<<grid_for(m, G), kThreads, 0, st>>>(ix, d_pat, len, m, (long long *)d_sp, (long long *)d_ep, sinks); \
-            else count_fixed_gmem_kernel<G, LAY, uint32_t><<<grid_for(m, G), kThreads, 0, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, sinks); \
-        } else if (too_long) {                                                                                        \
-            return cudaErrorInvalidValue;                                                                             \
-        } else if (d_stats) {                                                                                                \
-            auto k = count_fixed_kernel<G, LAY, true, uint32_t>;                                                      \
-            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                          \
-            k<<<grid_for(m, G), kThreads, smem, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, d_stats, sinks); \
-        } else if (out64) {                                                                                           \
-            auto k = count_fixed_kernel<G, LAY, false, long long>;                                                    \
-            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                          \
-            k<<<grid_for(m, G), kThreads, smem, st>>>(ix, d_pat, len, m, (long long *)d_sp, (long long *)d_ep, nullptr, sinks); \
-        } else if (cfg.min_blocks >= 4 && cfg.min_blocks <= 8) {            /* occupancy experiment (FMX_MINB) */          \
-            auto k = cfg.min_blocks == 4 ? count_fixed_kernel<G, LAY, false, uint32_t, 4> : cfg.min_blocks == 5 ? count_fixed_kernel<G, LAY, false, uint32_t, 5> : \
-                     cfg.min_blocks == 6 ? count_fixed_kernel<G, LAY, false, uint32_t, 6> : cfg.min_blocks == 7 ? count_fixed_kernel<G, LAY, false, uint32_t, 7> : \
-                     count_fixed_kernel<G, LAY, false, uint32_t, 8>;                                                  \
-            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                          \
-            k<<<grid_for(m, G), kThreads, smem, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, nullptr, sinks); \
-        } else {                                                                                                      \
-            auto k = count_fixed_kernel<G, LAY, false, uint32_t>;                                                     \
-            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                          \
-            k<<<grid_for(m, G), kThreads, smem, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, nullptr, sinks); \
-        }                                                                                                             \
-    }
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    if (too_long && d_stats) return cudaErrorInvalidValue;
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        if (too_long) {
+            if (out64) count_fixed_gmem_kernel<g, lay, long long><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_pat, len, m, (long long *)d_sp, (long long *)d_ep, sinks);
+            else count_fixed_gmem_kernel<g, lay, uint32_t><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, sinks);
+        } else if (d_stats) {
+            auto k = count_fixed_kernel<g, lay, true, uint32_t>;
+            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            k<<<grid_for(m, g), kThreads, smem, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, d_stats, sinks);
+        } else if (out64) {
+            auto k = count_fixed_kernel<g, lay, false, long long>;
+            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            k<<<grid_for(m, g), kThreads, smem, st>>>(ix, d_pat, len, m, (long long *)d_sp, (long long *)d_ep, nullptr, sinks);
+        } else {
+            auto k = count_fixed_kernel<g, lay, false, uint32_t>;
+            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            k<<<grid_for(m, g), kThreads, smem, st>>>(ix, d_pat, len, m, (uint32_t *)d_sp, (uint32_t *)d_ep, nullptr, sinks);
+        }
+    });
     return cudaGetLastError();
 }
 
@@ -750,27 +720,27 @@ cudaError_t launch_count_var(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d
                              int64_t *d_sp, int64_t *d_ep, cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
     if (cfg.count_lanes) cfg.lanes = cfg.count_lanes;
-#define CALL(G, LAY) count_var_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, d_pat, (const long long *)d_off, m, (long long *)d_sp, (long long *)d_ep)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        count_var_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_pat, (const long long *)d_off, m, (long long *)d_sp, (long long *)d_ep);
+    });
     return cudaGetLastError();
 }
 
 cudaError_t launch_occ(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_c, const int64_t *d_key, int64_t m, int64_t *d_out,
                        cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
-#define CALL(G, LAY) occ_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, d_c, (const long long *)d_key, m, (long long *)d_out)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        occ_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_c, (const long long *)d_key, m, (long long *)d_out);
+    });
     return cudaGetLastError();
 }
 
 cudaError_t launch_prev_range(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_sp, const int64_t *d_ep, const uint8_t *d_c,
                               int64_t m, int64_t *d_sp1, int64_t *d_ep1, cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
-#define CALL(G, LAY) prev_range_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (const long long *)d_sp, (const long long *)d_ep, d_c, m, (long long *)d_sp1, (long long *)d_ep1)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        prev_range_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, (const long long *)d_sp, (const long long *)d_ep, d_c, m, (long long *)d_sp1, (long long *)d_ep1);
+    });
     return cudaGetLastError();
 }
 
@@ -778,26 +748,26 @@ cudaError_t launch_interval_prev_range(const DevIndex &ix, LaunchCfg cfg, int64_
                                        int64_t *d_sp1, int64_t *d_ep1, cudaStream_t st) {
     const int64_t m = cend - cstart + 1;
     if (m <= 0) return cudaSuccess;
-#define CALL(G, LAY) interval_prev_range_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (uint32_t)sp, (uint32_t)ep, cstart, cend, (long long *)d_sp1, (long long *)d_ep1)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        interval_prev_range_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, (uint32_t)sp, (uint32_t)ep, cstart, cend, (long long *)d_sp1, (long long *)d_ep1);
+    });
     return cudaGetLastError();
 }
 
 cudaError_t launch_lf(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_row, int64_t m, int64_t *d_out, cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
-#define CALL(G, LAY) lf_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (const long long *)d_row, m, (long long *)d_out)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        lf_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, (const long long *)d_row, m, (long long *)d_out);
+    });
     return cudaGetLastError();
 }
 
 cudaError_t launch_prev_substr(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_row, int64_t m, int len, uint8_t *d_out,
                                cudaStream_t st) {
     if (m <= 0 || len <= 0) return cudaSuccess;
-#define CALL(G, LAY) prev_substr_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (const long long *)d_row, m, len, d_out)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        prev_substr_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, (const long long *)d_row, m, len, d_out);
+    });
     return cudaGetLastError();
 }
 
@@ -811,54 +781,47 @@ cudaError_t launch_text(const DevIndex &ix, LaunchCfg cfg, const uint32_t *d_off
     const int path = text_path(ix);
     if (path < 0) return cudaErrorInvalidValue;
     const int nseg = len > 0 ? (len + kTextSegment - 1) / kTextSegment : 1;
-    // the hop paths are one lane per segment (one request per entry); the LF walk shares each rank block among cfg.lanes lanes
-#define TEXT1(LAY, P) TEXTG(1, LAY, P)
-#define TEXTG(G, LAY, P)                                                                                                                  \
-    do {                                                                                                                                  \
-        if (d_requests) text_kernel<G, LAY, P, true><<<grid_for(mj * nseg, G), kThreads, 0, st>>>(ix, d_off + j0, mj, len, nseg, d_out + j0 * len, d_out_len + j0, d_requests); \
-        else text_kernel<G, LAY, P, false><<<grid_for(mj * nseg, G), kThreads, 0, st>>>(ix, d_off + j0, mj, len, nseg, d_out + j0 * len, d_out_len + j0, nullptr);          \
-    } while (0)
-#define CALL(G, LAY) TEXTG(G, LAY, kTextLf)
     const int64_t slice = (1ll << 30) / nseg;                     // requests per launch: the kernel's work-item indices stay 32-bit
     for (int64_t j0 = 0; j0 < m; j0 += slice) {
         const int64_t mj = std::min(slice, m - j0);
-        if (path == kTextIsat) TEXT1(FMX_LAYOUT_PLANES, kTextIsat);
-        else if (path == kTextCtx) TEXT1(FMX_LAYOUT_PLANES, kTextCtx);
-        else if (path == kTextCtx8) {
-            if (cfg.layout == FMX_LAYOUT_PLANES) TEXT1(FMX_LAYOUT_PLANES, kTextCtx8);
-            else if (cfg.layout == FMX_LAYOUT_WMX) TEXT1(FMX_LAYOUT_WMX, kTextCtx8);
-            else TEXT1(FMX_LAYOUT_WM, kTextCtx8);
-        } else FMX_DISPATCH(cfg, CALL);
+        auto text = [&](auto g, auto lay, auto p) {
+            if (d_requests) text_kernel<g, lay, p, true><<<grid_for(mj * nseg, g), kThreads, 0, st>>>(ix, d_off + j0, mj, len, nseg, d_out + j0 * len, d_out_len + j0, d_requests);
+            else text_kernel<g, lay, p, false><<<grid_for(mj * nseg, g), kThreads, 0, st>>>(ix, d_off + j0, mj, len, nseg, d_out + j0 * len, d_out_len + j0, nullptr);
+        };
+        // the hop paths are one lane per segment (one request per entry); the LF walk shares each rank block among cfg.lanes lanes
+        using One = std::integral_constant<int, 1>;
+        using Planes = std::integral_constant<int, FMX_LAYOUT_PLANES>;
+        if (path == kTextIsat) text(One{}, Planes{}, std::integral_constant<int, kTextIsat>{});
+        else if (path == kTextCtx) text(One{}, Planes{}, std::integral_constant<int, kTextCtx>{});
+        else if (path == kTextCtx8) dispatch_layout(cfg.layout, [&](auto lay) { text(One{}, lay, std::integral_constant<int, kTextCtx8>{}); });
+        else dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) { text(g, lay, std::integral_constant<int, kTextLf>{}); });
     }
-#undef CALL
-#undef TEXTG
-#undef TEXT1
     return cudaGetLastError();
 }
 
 cudaError_t launch_fl(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_row, int64_t m, int64_t *d_out, cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
-#define CALL(G, LAY) fl_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (const long long *)d_row, m, (long long *)d_out)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        fl_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, (const long long *)d_row, m, (long long *)d_out);
+    });
     return cudaGetLastError();
 }
 
 cudaError_t launch_next_substr(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_row, int64_t m, int len, uint8_t *d_out,
                                int *d_out_len, cudaStream_t st) {
     if (m <= 0) return cudaSuccess;
-#define CALL(G, LAY) next_substr_kernel<G, LAY><<<grid_for(m, G), kThreads, 0, st>>>(ix, (const long long *)d_row, m, len, d_out, d_out_len)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        next_substr_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, (const long long *)d_row, m, len, d_out, d_out_len);
+    });
     return cudaGetLastError();
 }
 
 cudaError_t launch_locate(const DevIndex &ix, LaunchCfg cfg, const uint32_t *d_sp, const int64_t *d_off, int64_t q0, int64_t q1,
                           int64_t t0, int64_t count, uint32_t *d_pos, uint64_t *d_key, unsigned long long *d_steps, cudaStream_t st) {
     if (count <= 0) return cudaSuccess;
-#define CALL(G, LAY) locate_kernel<G, LAY><<<grid_for(count, G), kThreads, 0, st>>>(ix, d_sp, (const long long *)d_off, q0, q1, t0, count, d_pos, (unsigned long long *)d_key, d_steps)
-    FMX_DISPATCH(cfg, CALL);
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        locate_kernel<g, lay><<<grid_for(count, g), kThreads, 0, st>>>(ix, d_sp, (const long long *)d_off, q0, q1, t0, count, d_pos, (unsigned long long *)d_key, d_steps);
+    });
     return cudaGetLastError();
 }
 

@@ -1,5 +1,7 @@
 // fmx_kernels.cuh — host-callable launchers of the search kernels (definitions in fmx_kernels.cu).
 #pragma once
+#include <type_traits>
+
 #include "fmx_device.cuh"
 
 namespace fmx {
@@ -11,8 +13,23 @@ struct LaunchCfg {
     int lanes;           // 1, 2 or 4 lanes per query
     int count_lanes = 0;       // > 0: lanes per query of the count kernels only (one lane once row contexts answer most queries in a
                                // single 32-byte request each: twice the queries in flight, half the instructions per query)
-    int min_blocks = 0;        // 4 or 6: the device-pointer count kernel compiled for that many resident CTAs per SM (0 = default: 8, 6 at one lane)
 };
+
+// The run-time layout (and lanes per query) as the kernels' template arguments: f(lay) / f(g, lay) with std::integral_constant<int, ...>
+// arguments, which convert to int constants (kernel<g, lay><<<...>>>).  Layouts other than PLANES and WMX are WM; lanes other than 1 and
+// 2 are 4 (upload_index and fmx_set_lanes accept only 1, 2 and 4).
+template <typename F> void dispatch_layout(int layout, F &&f) {
+    if (layout == FMX_LAYOUT_PLANES) f(std::integral_constant<int, FMX_LAYOUT_PLANES>{});
+    else if (layout == FMX_LAYOUT_WMX) f(std::integral_constant<int, FMX_LAYOUT_WMX>{});
+    else f(std::integral_constant<int, FMX_LAYOUT_WM>{});
+}
+template <typename F> void dispatch_layout_lanes(int layout, int lanes, F &&f) {
+    dispatch_layout(layout, [&](auto lay) {
+        if (lanes == 1) f(std::integral_constant<int, 1>{}, lay);
+        else if (lanes == 2) f(std::integral_constant<int, 2>{}, lay);
+        else f(std::integral_constant<int, 4>{}, lay);
+    });
+}
 
 // fused exchange: up to 8 gathered buffers (one per rank, peer-mapped) that receive this shard's hit counts
 struct PeerSinks {

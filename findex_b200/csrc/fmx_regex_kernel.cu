@@ -328,24 +328,15 @@ cudaError_t launch_regex_search(const DevIndex &ix, LaunchCfg cfg, const RegexTa
     // children a warp keeps on its own stack; what exceeds it goes to the global ring where idle warps find it (a '.' expansion is 253
     // children: all-local leaves the other warps idle, all-global pays an atomic round trip per child)
     const uint32_t local_keep = (uint32_t)std::min(std::max(g_regex_local_keep.load(), 0), kLocalSlots);
-#define CALL(G, LAY)                                                                                                  \
-    {                                                                                                                 \
-        auto k = regex_queue_kernel<G, LAY>;                                                                          \
-        int per_sm = 0;                                                                                               \
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kThreads, 0);                                   \
-        if (e == cudaSuccess) {                                                                                       \
-            if (per_sm <= 0) e = cudaErrorLaunchOutOfResources;                                                       \
-            else k<<<(unsigned)(sms * per_sm), kThreads, 0, st>>>(ix, rt, d_ring, d_seq, (unsigned long long)(ring_cap - 1), d_res, cap_res, d_ctrl, max_len, local_keep); \
-        }                                                                                                             \
-    }
-    if (cfg.layout == FMX_LAYOUT_PLANES) {
-        if (cfg.lanes == 1) { CALL(1, FMX_LAYOUT_PLANES); } else if (cfg.lanes == 2) { CALL(2, FMX_LAYOUT_PLANES); } else { CALL(4, FMX_LAYOUT_PLANES); }
-    } else if (cfg.layout == FMX_LAYOUT_WMX) {
-        if (cfg.lanes == 1) { CALL(1, FMX_LAYOUT_WMX); } else if (cfg.lanes == 2) { CALL(2, FMX_LAYOUT_WMX); } else { CALL(4, FMX_LAYOUT_WMX); }
-    } else {
-        if (cfg.lanes == 1) { CALL(1, FMX_LAYOUT_WM); } else if (cfg.lanes == 2) { CALL(2, FMX_LAYOUT_WM); } else { CALL(4, FMX_LAYOUT_WM); }
-    }
-#undef CALL
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        auto k = regex_queue_kernel<g, lay>;
+        int per_sm = 0;
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kThreads, 0);
+        if (e == cudaSuccess) {
+            if (per_sm <= 0) e = cudaErrorLaunchOutOfResources;
+            else k<<<(unsigned)(sms * per_sm), kThreads, 0, st>>>(ix, rt, d_ring, d_seq, (unsigned long long)(ring_cap - 1), d_res, cap_res, d_ctrl, max_len, local_keep);
+        }
+    });
     return e != cudaSuccess ? e : cudaGetLastError();
 }
 
