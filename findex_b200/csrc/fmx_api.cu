@@ -37,12 +37,13 @@ struct fmx_index {
     int64_t C[257] = {0};
     int64_t counts0[256] = {0};        // raw counts (bucketStarts0 / pos2char)
     int sigma = 0, levels = 0, sample_rate = 0, text_rate = 0;
-    int64_t nblk = 0, index_bytes = 0, n_samples = 0, rank_units64 = 0, dict_entries = 0;
+    int64_t nblk = 0, index_bytes = 0, n_samples = 0, rank_units64 = 0, dict_entries = 0, lcp_bytes = 0;
     int api_layout = FMX_LAYOUT_WM;    // what fmx_info reports
     std::vector<void *> owned;         // device allocations freed at close
     std::atomic<double> last_ms{0.0}, locate_walk_ms{0.0}, locate_sort_ms{0.0};      // diagnostics of the most recent call
     bool stats = false;                // fmx_set_stats: the next locate / regex calls also count their LF steps / items
     std::atomic<int64_t> last_steps{0}, last_launches{0}, total_launches{0}, last_levels{0};
+    std::atomic<int64_t> match_req[3] = {{0}, {0}, {0}};   // the last counting match call: rank blocks, LCP requests, minima lines
     std::mutex mu;                     // guards cfg / d / chunk_queries / stats and the pool below; never held across GPU work
     // Batch calls run concurrently: each takes one of kCallSets private stream sets for its duration (copies and kernels of different
     // host threads overlap; the index itself is read-only).  `stream`/`h2d`/`d2h` above belong to fmx_open and the rare whole-index calls.
@@ -243,6 +244,7 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
     if (n < 1 || eof < 0 || eof >= n) return fail(FMX_E_ARG, "bad n/eof");
     if (n >= (1ll << 32) - 1) return fail(FMX_E_UNSUPPORTED, "n = %lld needs 64-bit rows; this build indexes n < 2^32-1", (long long)n);
     if (o.text_sample_rate < 0 || o.text_sample_rate > 65536) return fail(FMX_E_ARG, "text_sample_rate = %d: 0 (none) or 1 .. 65536", o.text_sample_rate);
+    if (o.lcp != 0 && o.lcp != 1) return fail(FMX_E_ARG, "lcp = %d: 0 (none) or 1", o.lcp);
     ix->n = n; ix->eof = eof;
     // C table: bucketStarts with counts[0] := 1   (bwtmerger.scala:346-350, util.scala:109-119)
     int64_t tot = 0;
@@ -278,7 +280,7 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
         size_t fr = 0, to = 0;
         cudaMemGetInfo(&fr, &to);
         const int64_t sampled = (o.sa_sample_rate > 0 ? nblk * 64 + (n / o.sa_sample_rate + 1) * 4 + (n / kRowsPerWalkBlock + 1) * 64 : 0) +
-                                (o.text_sample_rate > 0 ? ((n - 1) / o.text_sample_rate + 1) * 4 : 0);
+                                (o.text_sample_rate > 0 ? ((n - 1) / o.text_sample_rate + 1) * 4 : 0) + (o.lcp ? lcp_layout(n).fixed_bytes : 0);
         layout = (planes_bytes <= budget && planes_bytes + n + sampled <= total_cap && planes_bytes + (6ll << 30) + 2 * n < (int64_t)fr) ? FMX_LAYOUT_PLANES
                  : (wmx_bytes + n + sampled <= total_cap ? FMX_LAYOUT_WMX : FMX_LAYOUT_WM);
     }
@@ -368,6 +370,8 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
     d.dict = nullptr; d.dict_buckets = 0; d.dict_D = 0; d.dict_bits = 0; d.dict_Dx = 0; d.dict_Jc = 1;
     for (int t = 0; t < 8; ++t) d.ctx_S[t] = 0;
     d.tsamp = nullptr; d.tsamp_rate = 0; d.sym = d_sym;
+    d.lcp8 = nullptr; d.lcp_rec = nullptr; d.lcpx = nullptr; d.lcp_tree = nullptr; d.lcp_top = 0;
+    for (int t = 0; t < 6; ++t) d.lcp_lvl[t] = 0;
     d.mark = nullptr; d.samples = nullptr; d.n = (uint32_t)n; d.eof = (uint32_t)eof; d.layout = layout; d.levels = levels;
     for (int l = 0; l < 8; ++l) d.z[l] = z[l];
     d.wmx_b = wmx ? xb : 0; d.wmx_levels = wmx ? xlevels : 0; d.wmx_stride = (uint64_t)nblkx;
@@ -391,6 +395,39 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
         }
         d.tsamp = tsamp; d.tsamp_rate = (uint32_t)o.text_sample_rate;
     }
+    // LCP structure (matching statistics): its fixed part is counted here, before the accelerators are sized; the escaped values (4 bytes
+    // per row with LCP >= 255) are known once it is built below
+    const LcpLayout lcp_lay = lcp_layout(n);
+    if (o.lcp) {
+        if (ix->index_bytes + lcp_lay.fixed_bytes > total_cap)
+            return fail(FMX_E_ARG, "max_total_bytes = %lld leaves no room for the %lld bytes of the LCP structure", (long long)total_cap, (long long)lcp_lay.fixed_bytes);
+        ix->index_bytes += lcp_lay.fixed_bytes;
+    }
+    // from the suffix array, its inverse and T' (scratch of the row-context construction when that runs): LCP array -> compact structure
+    auto make_lcp = [&](const uint32_t *sa, const uint32_t *isa, const uint8_t *text) -> int {
+        DBuf lcp(ix->stream);
+        CU(lcp.alloc((size_t)n * 4));
+        if (n <= 2) CU(cudaMemsetAsync(lcp.p, 0, (size_t)n * 4, ix->stream));      // no two suffixes share a symbol
+        else CU(build_lcp(sa, isa, text, n, lcp.as<int32_t>(), ix->stream));
+        void *p = nullptr;
+        int64_t bytes = 0;
+        const cudaError_t be = build_lcp_struct(lcp.as<int32_t>(), n, lcp_lay, &p, &bytes, ix->stream);
+        if (p) ix->owned.push_back(p);
+        CU(be);
+        if (ix->index_bytes - lcp_lay.fixed_bytes + bytes > total_cap)
+            return fail(FMX_E_ARG, "max_total_bytes = %lld leaves no room for the %lld bytes of the LCP structure", (long long)total_cap, (long long)bytes);
+        ix->index_bytes += bytes - lcp_lay.fixed_bytes;
+        ix->lcp_bytes = bytes;
+        const uint8_t *b = reinterpret_cast<const uint8_t *>(p);
+        d.lcp8 = reinterpret_cast<const uint4 *>(b);
+        d.lcp_rec = reinterpret_cast<const uint2 *>(b + lcp_lay.rec_off);
+        d.lcp_tree = reinterpret_cast<const uint32_t *>(b + lcp_lay.tree_off);
+        d.lcpx = reinterpret_cast<const uint32_t *>(b + lcp_lay.x_off);
+        d.lcp_top = lcp_lay.top;
+        for (int t = 0; t < 6; ++t) d.lcp_lvl[t] = (uint64_t)lcp_lay.lvl[t];
+        CU(cudaStreamSynchronize(ix->stream));
+        return FMX_OK;
+    };
     if (o.sa_sample_rate > 0) {
         const int64_t ns = (n + o.sa_sample_rate - 1) / o.sa_sample_rate;
         void *mark = nullptr, *samples = nullptr;
@@ -489,6 +526,7 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
                 ix->index_bytes += 8 * n;
             }
         }
+        if (o.lcp) { const int rc = make_lcp(sa.as<uint32_t>(), isa.as<uint32_t>(), text.as<uint8_t>()); if (rc) return rc; }
         // the full suffix array stays resident (locate = one load per occurrence) when the singleton shortcut needs it, or when no sampled
         // SA was asked for and neither the cap nor FMX_ACCEL_NO_SA forbids it; otherwise it was scratch
         const bool keep_sa = want_isat || (o.sa_sample_rate == 0 && !(accel & FMX_ACCEL_NO_SA) && 4 * n <= room() - (want_kmer ? room() / 4 : 0));
@@ -499,6 +537,17 @@ int upload_index(fmx_index *ix, const uint8_t *bwt, int64_t n, int64_t eof, cons
             sa.p = nullptr;
             ix->index_bytes += 4 * n;
         }
+    }
+    if (o.lcp && !build_sa) {
+        DBuf sa(ix->stream), isa(ix->stream), text(ix->stream);
+        if (n > 2) {
+            CU(sa.alloc((size_t)n * 4)); CU(isa.alloc((size_t)n * 4)); CU(text.alloc((size_t)n + 16));
+            std::string err;
+            e = build_full_sa(d, layout, sa.as<uint32_t>(), isa.as<uint32_t>(), text.as<uint8_t>(), ix->stream, err);
+            if (e != cudaSuccess) return fail(err.empty() ? FMX_E_CUDA : FMX_E_FORMAT, "suffix array construction failed: %s", err.empty() ? cudaGetErrorString(e) : err.c_str());
+        }
+        const int rc = make_lcp(sa.as<uint32_t>(), isa.as<uint32_t>(), text.as<uint8_t>());
+        if (rc) return rc;
     }
     trim_pool(ix->device);
     if (want_kmer && sigma >= 1) {
@@ -1159,6 +1208,177 @@ int fmx_text_dev(fmx_index *ix, const void *d_off, int64_t m, int32_t len, void 
         CU(cudaStreamSynchronize(st));
         ix->last_steps = (int64_t)h;
     }
+    return FMX_OK;
+}
+
+// ---- matching statistics and SMEMs (include/fmgpu.h) -------------------------------------------------------------
+int64_t fmx_lcp_bytes(const fmx_index *ix) { return ix ? ix->lcp_bytes : 0; }
+int fmx_last_match_requests(const fmx_index *ix, int64_t req[3]) {
+    CHECK_IX(ix);
+    if (!req) return fail(FMX_E_ARG, "null argument");
+    for (int k = 0; k < 3; ++k) req[k] = ix->match_req[k].load();
+    return FMX_OK;
+}
+
+}  // extern "C"
+
+namespace {
+int check_queries(const fmx_index *ix, const uint8_t *pat, const int64_t *off, int64_t m) {
+    if (m < 0 || !off) return fail(FMX_E_ARG, "bad argument");
+    if (off[0] < 0) return fail(FMX_E_ARG, "offsets must be non-negative");
+    for (int64_t i = 0; i < m; ++i) if (off[i + 1] < off[i]) return fail(FMX_E_ARG, "offsets must be non-decreasing (at %lld)", (long long)i);
+    if (off[m] && !pat) return fail(FMX_E_ARG, "null pattern buffer");
+    if (off[m] >= (1ll << 32) - 1) return fail(FMX_E_ARG, "a batch holds fewer than 2^32 - 1 query symbols");
+    if (ix->d_full.lcp8 == nullptr) return fail(FMX_E_UNSUPPORTED, "matching statistics need the LCP structure: open the index with fmx_opts.lcp = 1");
+    return FMX_OK;
+}
+
+// the counters of a counting run (fmx_set_stats) -> fmx_last_steps / fmx_last_match_requests
+int collect_match_stats(fmx_index *ix, const DBuf &dstats, cudaStream_t st) {
+    unsigned long long h[3] = {0, 0, 0};
+    CU(cudaMemcpyAsync(h, dstats.p, 24, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    for (int k = 0; k < 3; ++k) ix->match_req[k] = (int64_t)h[k];
+    ix->last_steps = (int64_t)(h[0] + h[1] + h[2]);
+    return FMX_OK;
+}
+
+// The matching statistics of a host batch through the call's three streams (pattern bytes and offsets of chunk k+1 in, the kernel on chunk
+// k, its results out), by text position into d_len / d_sp / d_ep (device, off[m] entries) and, with `flags`, the SMEM flags of min_len.
+// d2h(q0, nq) copies what the caller wants back of the chunk.
+template <typename D2H>
+int match_pipeline(fmx_index *ix, CallCtx &cc, const uint8_t *pat, const int64_t *off, int64_t m, DBuf &dpat, DBuf &doff, DBuf &dlen, bool iv,
+                   DBuf &dsp, DBuf &dep, DBuf *dflag, int min_len, DBuf &dstats, D2H &&d2h) {
+    cudaStream_t st = cc.stream;
+    const int64_t T = off[m];
+    CU(dpat.alloc((size_t)T + 16)); CU(doff.alloc((size_t)(m + 1) * 8)); CU(dlen.alloc((size_t)T * 4));
+    if (iv) { CU(dsp.alloc((size_t)T * 4)); CU(dep.alloc((size_t)T * 4)); }
+    if (dflag) { CU(dflag->alloc((size_t)(T + 1) * 4)); CU(cudaMemsetAsync(dflag->p, 0, (size_t)(T + 1) * 4, st)); }
+    if (cc.stats) { CU(dstats.alloc(24)); CU(cudaMemsetAsync(dstats.p, 0, 24, st)); }
+    const int64_t chunk = cc.chunk_queries > 0 ? cc.chunk_queries : (1 << 20);
+    const int rc = chunk_pipeline(ix, cc, "match", m, chunk, 1,
+        [&](int64_t q0, int64_t nq) {
+            const int64_t a = off[q0], b = off[q0 + nq];
+            cudaError_t e = b > a ? cudaMemcpyAsync(dpat.as<uint8_t>() + a, pat + a, (size_t)(b - a), cudaMemcpyHostToDevice, cc.h2d) : cudaSuccess;
+            return e != cudaSuccess ? e : cudaMemcpyAsync(doff.as<int64_t>() + q0, off + q0, (size_t)(nq + 1) * 8, cudaMemcpyHostToDevice, cc.h2d);
+        },
+        [&](int64_t q0, int64_t nq) {
+            return launch_match(cc.d, cc.cfg, dpat.as<uint8_t>(), doff.as<int64_t>() + q0, nq, dlen.as<int32_t>(), dsp.as<uint32_t>(), dep.as<uint32_t>(),
+                                dflag ? dflag->as<uint32_t>() : nullptr, min_len, cc.stats ? dstats.as<unsigned long long>() : nullptr, st);
+        },
+        d2h);
+    if (rc == FMX_OK && cc.stats) return collect_match_stats(ix, dstats, st);
+    return rc;
+}
+}  // namespace
+
+extern "C" {
+
+int fmx_match_stats_batch(fmx_index *ix, const uint8_t *pat, const int64_t *off, int64_t m, int32_t *ms_len, int64_t *ms_sp, int64_t *ms_ep) {
+    CHECK_IX(ix);
+    int rc = check_queries(ix, pat, off, m);
+    if (rc) return rc;
+    if (m == 0 || off[m] == off[0]) return FMX_OK;
+    if (!ms_len) return fail(FMX_E_ARG, "null output");
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = cc.stream;
+    const bool iv = ms_sp || ms_ep;
+    DBuf dpat(st), doff(st), dlen(st), dsp(st), dep(st), dstats(st), dwide(st);
+    if (iv) CU(dwide.alloc((size_t)off[m] * 16));
+    int64_t *wsp = dwide.as<int64_t>(), *wep = wsp + off[m];
+    return match_pipeline(ix, cc, pat, off, m, dpat, doff, dlen, iv, dsp, dep, nullptr, 0, dstats, [&](int64_t q0, int64_t nq) {
+        const int64_t a = off[q0], b = off[q0 + nq];
+        if (b == a) return cudaSuccess;
+        cudaError_t e = cudaMemcpyAsync(ms_len + a, dlen.as<int32_t>() + a, (size_t)(b - a) * 4, cudaMemcpyDeviceToHost, cc.d2h);
+        if (iv) {                                                  // rows are uint32 on the device, int64 at the ABI
+            if (e == cudaSuccess) e = widen_u32_i64(dsp.as<uint32_t>() + a, wsp + a, b - a, cc.d2h);
+            if (e == cudaSuccess) e = widen_u32_i64(dep.as<uint32_t>() + a, wep + a, b - a, cc.d2h);
+            if (e == cudaSuccess && ms_sp) e = cudaMemcpyAsync(ms_sp + a, wsp + a, (size_t)(b - a) * 8, cudaMemcpyDeviceToHost, cc.d2h);
+            if (e == cudaSuccess && ms_ep) e = cudaMemcpyAsync(ms_ep + a, wep + a, (size_t)(b - a) * 8, cudaMemcpyDeviceToHost, cc.d2h);
+        }
+        return e;
+    });
+}
+
+int fmx_smem_batch(fmx_index *ix, const uint8_t *pat, const int64_t *off, int64_t m, int32_t min_len, int64_t cap_total, int64_t *out_off,
+                   int32_t *start, int32_t *len, int64_t *sp, int64_t *ep) {
+    CHECK_IX(ix);
+    int rc = check_queries(ix, pat, off, m);
+    if (rc) return rc;
+    if (min_len < 1) return fail(FMX_E_ARG, "min_len = %d: at least 1", min_len);
+    if (!out_off || cap_total < 0 || (cap_total > 0 && (!start || !len || !sp || !ep))) return fail(FMX_E_ARG, "bad argument");
+    for (int64_t q = 0; q <= m; ++q) out_off[q] = 0;
+    if (m == 0 || off[m] == off[0]) return FMX_OK;
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = cc.stream;
+    const int64_t T = off[m];
+    DBuf dpat(st), doff(st), dlen(st), dsp(st), dep(st), dflag(st), dstats(st), dscan(st);
+    rc = match_pipeline(ix, cc, pat, off, m, dpat, doff, dlen, true, dsp, dep, &dflag, min_len, dstats, [](int64_t, int64_t) { return cudaSuccess; });
+    if (rc) return rc;
+    DBuf doo(st);
+    CU(dscan.alloc((size_t)(T + 1) * 4)); CU(doo.alloc((size_t)(m + 1) * 8));
+    CU(exclusive_sum_u32(dflag.as<uint32_t>(), dscan.as<uint32_t>(), T + 1, st));
+    CU(launch_smem_offsets(dscan.as<uint32_t>(), doff.as<int64_t>(), m, doo.as<int64_t>(), st));
+    CU(cudaMemcpyAsync(out_off, doo.p, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const int64_t total = out_off[m];
+    if (total > cap_total) return fail(FMX_E_CAPACITY, "the SMEMs need %lld output slots, capacity %lld", (long long)total, (long long)cap_total);
+    if (total == 0) return FMX_OK;
+    DBuf dst(st), dln(st), dsp32(st), dep32(st), dw(st);
+    CU(dst.alloc((size_t)total * 4)); CU(dln.alloc((size_t)total * 4)); CU(dsp32.alloc((size_t)total * 4)); CU(dep32.alloc((size_t)total * 4));
+    CU(dw.alloc((size_t)total * 16));
+    CU(launch_smem_compact(dflag.as<uint32_t>(), dscan.as<uint32_t>(), dlen.as<int32_t>(), dsp.as<uint32_t>(), dep.as<uint32_t>(), doff.as<int64_t>(), m, T,
+                           dst.as<int32_t>(), dln.as<int32_t>(), dsp32.as<uint32_t>(), dep32.as<uint32_t>(), st));
+    CU(widen_u32_i64(dsp32.as<uint32_t>(), dw.as<int64_t>(), total, st));
+    CU(widen_u32_i64(dep32.as<uint32_t>(), dw.as<int64_t>() + total, total, st));
+    CU(cudaMemcpyAsync(start, dst.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(len, dln.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(sp, dw.p, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(ep, dw.as<int64_t>() + total, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return FMX_OK;
+}
+
+// Device-resident SMEMs: reads off[m] (the number of query symbols, to size the scratch) and the total back, everything else stays on
+// `stream`.  The offsets are not checked on the host.
+int fmx_smem_dev(fmx_index *ix, const void *d_pat, const void *d_off, int64_t m, int32_t min_len, void *d_out_off, void *d_start, void *d_len,
+                 void *d_sp, void *d_ep, int64_t cap, int64_t *total_out, void *stream) {
+    CHECK_IX(ix);
+    if (m < 0 || !d_off || !d_out_off || !total_out || cap < 0 || (cap > 0 && (!d_start || !d_len || !d_sp || !d_ep))) return fail(FMX_E_ARG, "bad argument");
+    if (min_len < 1) return fail(FMX_E_ARG, "min_len = %d: at least 1", min_len);
+    if (ix->d_full.lcp8 == nullptr) return fail(FMX_E_UNSUPPORTED, "matching statistics need the LCP structure: open the index with fmx_opts.lcp = 1");
+    *total_out = 0;
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    int64_t T = 0;
+    CU(cudaMemcpyAsync(&T, (const int64_t *)d_off + m, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (T < 0 || T >= (1ll << 32) - 1) return fail(FMX_E_ARG, "off[m] = %lld: a batch holds 0 .. 2^32 - 2 query symbols", (long long)T);
+    if (T > 0 && !d_pat) return fail(FMX_E_ARG, "null pattern buffer");
+    DBuf dlen(st), dsp(st), dep(st), dflag(st), dscan(st), dstats(st);
+    CU(dlen.alloc((size_t)T * 4)); CU(dsp.alloc((size_t)T * 4)); CU(dep.alloc((size_t)T * 4));
+    CU(dflag.alloc((size_t)(T + 1) * 4)); CU(dscan.alloc((size_t)(T + 1) * 4));
+    CU(cudaMemsetAsync(dflag.p, 0, (size_t)(T + 1) * 4, st));
+    if (cc.stats) { CU(dstats.alloc(24)); CU(cudaMemsetAsync(dstats.p, 0, 24, st)); }
+    CU(launch_match(cc.d, cc.cfg, (const uint8_t *)d_pat, (const int64_t *)d_off, m, dlen.as<int32_t>(), dsp.as<uint32_t>(), dep.as<uint32_t>(),
+                    dflag.as<uint32_t>(), min_len, cc.stats ? dstats.as<unsigned long long>() : nullptr, st));
+    CU(exclusive_sum_u32(dflag.as<uint32_t>(), dscan.as<uint32_t>(), T + 1, st));
+    CU(launch_smem_offsets(dscan.as<uint32_t>(), (const int64_t *)d_off, m, (int64_t *)d_out_off, st));
+    ix->last_launches = 1; ix->total_launches += 1;
+    int64_t total = 0;
+    CU(cudaMemcpyAsync(&total, (const int64_t *)d_out_off + m, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    *total_out = total;
+    if (cc.stats) { const int src = collect_match_stats(ix, dstats, st); if (src) return src; }
+    if (total > cap) return fail(FMX_E_CAPACITY, "the SMEMs need %lld output slots, capacity %lld", (long long)total, (long long)cap);
+    CU(launch_smem_compact(dflag.as<uint32_t>(), dscan.as<uint32_t>(), dlen.as<int32_t>(), dsp.as<uint32_t>(), dep.as<uint32_t>(), (const int64_t *)d_off, m, T,
+                           (int32_t *)d_start, (int32_t *)d_len, (uint32_t *)d_sp, (uint32_t *)d_ep, st));
     return FMX_OK;
 }
 

@@ -525,6 +525,105 @@ cudaError_t build_lcp(const uint32_t *d_sa, const uint32_t *d_isa, const uint8_t
     return cudaGetLastError();
 }
 
+// ---- resident LCP structure (DevIndex::lcp8 / lcp_rec / lcpx / lcp_tree) -------------------------------------------------------------
+LcpLayout lcp_layout(int64_t n) {
+    LcpLayout L{};
+    L.nb = (n + kLcpRows - 1) / kLcpRows;
+    auto up = [](int64_t b) { return (b + 127) / 128 * 128; };
+    int64_t at = up(L.nb * kLcpRows);
+    L.rec_off = at;
+    at += up((L.nb + kLcpRecLine - 1) / kLcpRecLine * 128);
+    L.tree_off = at;
+    int64_t count = L.nb, words = 0;
+    int t = 0;
+    for (uint32_t F = kLcpRecLine; count > F; F = kLcpFan) {          // level t+1: one minimum per line of level t
+        count = (count + F - 1) / F;
+        L.lvl[t] = words;
+        L.lvl_count[t] = count;
+        words += (count + kLcpFan - 1) / kLcpFan * kLcpFan;
+        ++t;
+    }
+    L.top = t;
+    at += words * 4;
+    L.x_off = at;
+    L.fixed_bytes = at;
+    return L;
+}
+
+__global__ void lcp8_kernel(const int32_t *__restrict__ lcp, int64_t n, int64_t rows, uint8_t *__restrict__ lcp8) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= rows) return;
+    const int32_t v = r < n ? lcp[r] : 0;
+    lcp8[r] = (uint8_t)(v < (int32_t)kLcpEsc ? v : (int32_t)kLcpEsc);
+}
+// escaped rows (LCP >= 255) per block
+__global__ void lcp_count_kernel(const int32_t *__restrict__ lcp, int64_t n, int64_t nb, uint32_t *__restrict__ cnt) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nb) return;
+    uint32_t c = 0;
+    for (int64_t r = b * kLcpRows; r < (b + 1) * kLcpRows && r < n; ++r) c += (uint32_t)lcp[r] >= kLcpEsc;
+    cnt[b] = c;
+}
+// record { minimum, first escape } of every block (records past the last block: 0xFFFFFFFF, the padding of the line) and its escapes
+__global__ void lcp_rec_kernel(const int32_t *__restrict__ lcp, int64_t n, int64_t nb, int64_t nrec, const uint32_t *__restrict__ base,
+                               uint2 *__restrict__ rec, uint32_t *__restrict__ lcpx) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nrec) return;
+    if (b >= nb) { rec[b] = make_uint2(0xFFFFFFFFu, 0u); return; }
+    uint32_t mn = 0xFFFFFFFFu, k = base[b];
+    rec[b] = make_uint2(0u, k);
+    for (int64_t r = b * kLcpRows; r < (b + 1) * kLcpRows; ++r) {
+        const uint32_t v = r < n ? (uint32_t)lcp[r] : 0u;             // rows past n-1 pad the last block with 0 (LCP[n-1] is 0 anyway)
+        mn = v < mn ? v : mn;
+        if (v >= kLcpEsc) lcpx[k++] = v;
+    }
+    rec[b].x = mn;
+}
+// level entry j = minimum of line j of the level below (`stride` words per slot: 2 for the records); padding entries 0xFFFFFFFF
+__global__ void lcp_tree_kernel(const uint32_t *__restrict__ src, int stride, int fan, int64_t count, int64_t padded, uint32_t *__restrict__ dst) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= padded) return;
+    uint32_t mn = 0xFFFFFFFFu;
+    if (j < count)
+        for (int k = 0; k < fan; ++k) { const uint32_t v = src[(j * fan + k) * stride]; mn = v < mn ? v : mn; }
+    dst[j] = mn;
+}
+
+cudaError_t build_lcp_struct(const int32_t *d_lcp, int64_t n, const LcpLayout &L, void **d_out, int64_t *bytes_out, cudaStream_t st) {
+    *d_out = nullptr;
+    const int64_t rows = L.nb * kLcpRows, nrec = (L.nb + kLcpRecLine - 1) / kLcpRecLine * kLcpRecLine;
+    uint32_t *cnt = nullptr;
+    CK(cudaMallocAsync(&cnt, (size_t)(L.nb + 1) * 8, st));
+    uint32_t *base = cnt + L.nb + 1;
+    CK(cudaMemsetAsync(cnt, 0, (size_t)(L.nb + 1) * 4, st));
+    lcp_count_kernel<<<(unsigned)((L.nb + 255) / 256), 256, 0, st>>>(d_lcp, n, L.nb, cnt);
+    cudaError_t e = exclusive_sum_u32(cnt, base, L.nb + 1, st);
+    uint32_t total = 0;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&total, base + L.nb, 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    const int64_t bytes = L.fixed_bytes + (int64_t)total * 4;
+    if (e == cudaSuccess) e = cudaMalloc(d_out, (size_t)bytes);
+    if (e == cudaSuccess) {
+        uint8_t *out = reinterpret_cast<uint8_t *>(*d_out);
+        uint2 *rec = reinterpret_cast<uint2 *>(out + L.rec_off);
+        uint32_t *tree = reinterpret_cast<uint32_t *>(out + L.tree_off);
+        lcp8_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(d_lcp, n, rows, out);
+        lcp_rec_kernel<<<(unsigned)((nrec + 255) / 256), 256, 0, st>>>(d_lcp, n, L.nb, nrec, base, rec, reinterpret_cast<uint32_t *>(out + L.x_off));
+        const uint32_t *src = reinterpret_cast<const uint32_t *>(rec);
+        int stride = 2, fan = (int)kLcpRecLine;
+        for (int t = 0; t < L.top; ++t) {
+            const int64_t count = L.lvl_count[t], padded = (count + kLcpFan - 1) / kLcpFan * kLcpFan;
+            lcp_tree_kernel<<<(unsigned)((padded + 255) / 256), 256, 0, st>>>(src, stride, fan, count, padded, tree + L.lvl[t]);
+            src = tree + L.lvl[t];
+            stride = 1; fan = (int)kLcpFan;
+        }
+        e = cudaGetLastError();
+    } else *d_out = nullptr;
+    cudaFreeAsync(cnt, st);
+    *bytes_out = bytes;
+    return e;
+}
+
 // k-mer table: entry idx <-> the K-byte pattern P with P[K-1-j] = sym[digit_j(idx)] (digit 0 most significant = the byte search()
 // consumes first, i.e. the LAST pattern byte); entry = (sp,ep) after those K backward steps, (0,0) when the interval is empty.
 // Built level by level: level 1 is (C[c], C[c+1]); an entry of level j+1 is one backward step from its parent idx/sigma of level j

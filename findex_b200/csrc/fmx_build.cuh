@@ -36,6 +36,16 @@ cudaError_t build_ctx8(const uint32_t *d_sa, const uint32_t *d_isa, const uint8_
                        uint2 *d_ctx8, cudaStream_t st);
 // d_lcp[r] = lcp(suffix of row r, suffix of row r+1), d_lcp[n-1] = 0   (bwtFm2LCP, util.scala:153-212)
 cudaError_t build_lcp(const uint32_t *d_sa, const uint32_t *d_isa, const uint8_t *d_text, int64_t n, int32_t *d_lcp, cudaStream_t st);
+// the resident LCP structure (DevIndex::lcp8 ...; fmx_device.cuh lcp_widen) in one allocation: lcp8 | records | minima levels | lcpx, each
+// part 128-byte aligned; fixed_bytes = everything but the 4 bytes per escaped row (LCP >= 255)
+struct LcpLayout {
+    int64_t nb, rec_off, tree_off, x_off, fixed_bytes;
+    int64_t lvl[6], lvl_count[6];      // level t+1: u32 offset from tree_off / 4, entries before padding
+    int top;                           // levels above the records
+};
+LcpLayout lcp_layout(int64_t n);
+// from the int32 LCP array: *d_out = cudaMalloc'ed structure of *bytes_out bytes
+cudaError_t build_lcp_struct(const int32_t *d_lcp, int64_t n, const LcpLayout &L, void **d_out, int64_t *bytes_out, cudaStream_t st);
 // (sp,ep) after the first K backward steps for every K-mer over the sigma occurring symbols; lex = false: the first consumed (last) pattern
 // byte is the most significant digit of the entry index, lex = true: lexicographic order of the K-mer (its first byte most significant)
 cudaError_t build_kmer_table(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_sym, uint32_t sigma, int K, uint2 *d_table, cudaStream_t st,

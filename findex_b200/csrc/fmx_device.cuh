@@ -85,6 +85,17 @@ struct DevIndex {
     const uint32_t *tsamp;
     uint32_t        tsamp_rate;     // 0 = no samples
     const uint8_t  *sym;
+    // LCP structure (fmx_opts.lcp), what the matching-statistics kernel widens an interval to its parent with (lcp_widen below):
+    // lcp8[r] = min(LCP[r], 255) in 64-row blocks; lcp_rec[b] = { exact minimum of block b, index in lcpx of its first escaped value },
+    // 16 records per 128-byte line; lcpx = the exact LCP of the rows whose lcp8 is 255, in row order; above the records a tree of exact
+    // minima, level t >= 1 at lcp_tree + lcp_lvl[t-1], entry j = minimum of line j of level t-1 (32 u32 = one 128-byte line per node).
+    // Every level is padded to whole lines with 0xFFFFFFFF; level lcp_top fits one line.  lcp8 == nullptr: not built.
+    const uint4    *lcp8;
+    const uint2    *lcp_rec;
+    const uint32_t *lcpx;
+    const uint32_t *lcp_tree;
+    uint64_t        lcp_lvl[6];
+    int32_t         lcp_top;
 };
 
 // Pattern accessors handed to search_pattern: operator()(i) = byte i; word(w) = bytes 4w..4w+3 packed little-endian (bytes at or
@@ -424,6 +435,180 @@ __device__ __forceinline__ void backward_step(const DevIndex &ix, const SharedTa
         sp = t.base[c] + p;
         ep = t.base[c] + q;
     }
+}
+
+// ---- LCP parent widening (matching statistics; DESIGN.md §3) ---------------------------------------------------------------------------
+// An interval [sp, ep) of the l-symbol prefix X of its rows' suffixes that cannot be extended is widened to the interval of the longest
+// proper prefix of X that has more rows: d = max(LCP[sp-1], LCP[ep-1]) (LCP[-1] = 0), then the run of rows around [sp, ep) whose LCPs with
+// their neighbours stay >= d.  The lanes of a group split each 64-byte lcp8 block (as a rank block) and each 128-byte minima line.
+constexpr uint32_t kLcpRows = 64, kLcpRecLine = 16, kLcpFan = 32, kLcpEsc = 255;
+
+__device__ __forceinline__ uint32_t byte_flags4(uint32_t x) {          // 0xFF / 0x00 per byte -> one bit per byte
+    return (x & 1u) | ((x >> 7) & 2u) | ((x >> 14) & 4u) | ((x >> 21) & 8u);
+}
+
+// rows of the block (bit o = row o) whose lcp8 is below dd (`lt`) and whose lcp8 is 255 (`esc`), in every lane of the group
+template <int G>
+__device__ __forceinline__ void lcp_masks(const LaneBlock<G> &b, uint32_t dd, unsigned long long &lt, unsigned long long &esc) {
+    const int lane = (G == 1) ? 0 : (threadIdx.x & (G - 1));
+    const uint32_t dup = dd * 0x01010101u;
+    lt = 0; esc = 0;
+#pragma unroll
+    for (int i = 0; i < 4 / G; ++i) {
+        const uint32_t w[4] = {b.v[i].x, b.v[i].y, b.v[i].z, b.v[i].w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int first = (lane * (4 / G) + i) * 16 + 4 * k;
+            lt |= (unsigned long long)byte_flags4(__vcmpltu4(w[k], dup)) << first;
+            esc |= (unsigned long long)byte_flags4(__vcmpeq4(w[k], 0xFFFFFFFFu)) << first;
+        }
+    }
+    if (G > 1) {
+        const uint32_t mask = group_mask<G>();
+        lt |= __shfl_xor_sync(mask, lt, 1); esc |= __shfl_xor_sync(mask, esc, 1);
+        if (G > 2) { lt |= __shfl_xor_sync(mask, lt, 2); esc |= __shfl_xor_sync(mask, esc, 2); }
+    }
+}
+
+// exact LCP of row o of block blk: lcp8, or for an escaped row lcpx[record's first escape + the 255s before it] (two more requests)
+template <int G, bool STATS>
+__device__ __forceinline__ uint32_t lcp_value(const DevIndex &ix, const LaneBlock<G> &b, uint32_t blk, uint32_t o, uint32_t &req) {
+    const int lane = (G == 1) ? 0 : (threadIdx.x & (G - 1));
+    uint32_t v = 0, below = 0;
+#pragma unroll
+    for (int i = 0; i < 4 / G; ++i) {
+        const uint32_t first = (uint32_t)(lane * (4 / G) + i) * 16u;
+        const uint32_t w[4] = {b.v[i].x, b.v[i].y, b.v[i].z, b.v[i].w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const uint32_t f = first + 4u * k, e = byte_flags4(__vcmpeq4(w[k], 0xFFFFFFFFu));
+            if (o >= f && o < f + 4u) v = (w[k] >> (8u * (o - f))) & 0xFFu;
+            below += __popc(e & (o > f ? (o - f >= 4u ? 0xFu : (1u << (o - f)) - 1u) : 0u));
+        }
+    }
+    if (G > 1) { const uint32_t mask = group_mask<G>(); v = group_sum<G>(v, mask); below = group_sum<G>(below, mask); }
+    if (v != kLcpEsc) return v;
+    if (STATS) req += 2;
+    return ldg32(ix.lcpx + ldg64(ix.lcp_rec + blk).y + below);
+}
+
+// last row <= o (left) / first row >= o (right) of block blk whose LCP is below d, -1 / 64 when none.  Rows with lcp8 < min(d, 255) qualify
+// outright; for d > 255 the escaped rows between the nearest of those and o are read from lcpx, where they are consecutive.
+template <bool LEFT, bool STATS>
+__device__ __forceinline__ int lcp_scan(const DevIndex &ix, uint32_t blk, unsigned long long lt, unsigned long long esc, int o, uint32_t d,
+                                        uint32_t &req) {
+    const unsigned long long c = LEFT ? (lt & ((2ull << o) - 1ull)) : (lt & (~0ull << o));
+    const int k1 = LEFT ? (c ? 63 - __clzll((long long)c) : -1) : (c ? __ffsll((long long)c) - 1 : 64);
+    if (d <= kLcpEsc || k1 == o) return k1;
+    uint32_t x = ldg64(ix.lcp_rec + blk).y + (uint32_t)__popcll(esc & ((1ull << o) - 1ull));   // lcpx index of row o (an escaped row)
+    if (STATS) ++req;
+    for (int k = o; LEFT ? k > k1 : k < k1; k += LEFT ? -1 : 1) {
+        if (STATS) ++req;
+        if (ldg32(ix.lcpx + x) < d) return k;
+        x = LEFT ? x - 1u : x + 1u;
+    }
+    return k1;
+}
+
+// slots of line `line` of level t (0: the 16 records, t >= 1: 32 minima) whose minimum is below d, in every lane of the group
+template <int G>
+__device__ __forceinline__ uint32_t lcp_line_mask(const DevIndex &ix, int t, uint32_t line, uint32_t d) {
+    const int lane = (G == 1) ? 0 : (threadIdx.x & (G - 1));
+    const uint4 *base = t == 0 ? reinterpret_cast<const uint4 *>(ix.lcp_rec) : reinterpret_cast<const uint4 *>(ix.lcp_tree + ix.lcp_lvl[t - 1]);
+    const LaneBlockX<G> L = load_block_x<G>(base, line, lane);
+    uint32_t mask = 0;
+#pragma unroll
+    for (int i = 0; i < 8 / G; ++i) {
+        const uint32_t w[4] = {L.v[i].x, L.v[i].y, L.v[i].z, L.v[i].w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int wi = (lane * (8 / G) + i) * 4 + k;                  // word of the line
+            if (t == 0) { if (!(wi & 1) && w[k] < d) mask |= 1u << (wi >> 1); }
+            else if (w[k] < d) mask |= 1u << wi;
+        }
+    }
+    if (G > 1) {
+        const uint32_t gm = group_mask<G>();
+        mask |= __shfl_xor_sync(gm, mask, 1);
+        if (G > 2) mask |= __shfl_xor_sync(gm, mask, 2);
+    }
+    return mask;
+}
+
+// the nearest block before (LEFT) / after block b whose minimum is below d, or -1: up the tree one line per level until a line holds such
+// a slot on the searched side, then down one line per level to the nearest such block
+template <int G, bool LEFT, bool STATS>
+__device__ __forceinline__ int64_t lcp_climb(const DevIndex &ix, uint32_t b, uint32_t d, uint32_t &req) {
+    uint32_t p = b, q = 0;
+    int t = 0;
+    for (;; ++t) {
+        if (t > ix.lcp_top) return -1;
+        const uint32_t F = t == 0 ? kLcpRecLine : kLcpFan, line = p / F, slot = p % F;
+        uint32_t mask = lcp_line_mask<G>(ix, t, line, d);
+        if (STATS) ++req;
+        mask &= LEFT ? ((1u << slot) - 1u) : (~1u << slot);
+        if (mask) { q = line * F + (LEFT ? 31 - __clz(mask) : __ffs(mask) - 1); break; }
+        p = line;
+    }
+    while (t > 0) {
+        --t;
+        const uint32_t mask = lcp_line_mask<G>(ix, t, q, d);
+        if (STATS) ++req;
+        q = q * (t == 0 ? kLcpRecLine : kLcpFan) + (LEFT ? 31 - __clz(mask) : __ffs(mask) - 1);
+    }
+    return (int64_t)q;
+}
+
+// [sp, ep) (not empty, l > 0) -> the parent interval and its depth l = d; d = 0 gives (0, n).  All G lanes of the group call this together.
+// lreq += 64-byte lcp8 blocks + record and lcpx reads, mreq += 128-byte record / minima lines.
+template <int G, bool STATS>
+__device__ __forceinline__ void lcp_widen(const DevIndex &ix, uint32_t &sp, uint32_t &ep, uint32_t &l, uint32_t &lreq, uint32_t &mreq) {
+    const int lane = (G == 1) ? 0 : (threadIdx.x & (G - 1));
+    const bool has_a = sp > 0;
+    const uint32_t ra = has_a ? sp - 1u : 0u, rb = ep - 1u, ba = ra / kLcpRows, bb = rb / kLcpRows;
+    const int oa = (int)(ra % kLcpRows), ob = (int)(rb % kLcpRows);
+    const LaneBlock<G> B = load_block<G>(ix.lcp8, bb, lane);
+    LaneBlock<G> A = B;
+    if (has_a && ba != bb) A = load_block<G>(ix.lcp8, ba, lane);
+    if (STATS) lreq += (has_a && ba != bb) ? 2u : 1u;
+    const uint32_t vb = lcp_value<G, STATS>(ix, B, bb, (uint32_t)ob, lreq);
+    const uint32_t va = has_a ? lcp_value<G, STATS>(ix, A, ba, (uint32_t)oa, lreq) : 0u;
+    const uint32_t d = va > vb ? va : vb;
+    if (d == 0) { sp = 0; ep = ix.n; l = 0; return; }
+    const uint32_t dd = d < kLcpEsc ? d : kLcpEsc;
+    unsigned long long lt, esc;
+    uint32_t nsp = 0, nep;
+    if (has_a && va < d) nsp = sp;                                 // row sp-1 already differs within the first d symbols
+    else if (has_a) {
+        lcp_masks<G>(A, dd, lt, esc);
+        int k = lcp_scan<true, STATS>(ix, ba, lt, esc, oa, d, lreq);
+        if (k >= 0) nsp = ba * kLcpRows + (uint32_t)k + 1u;
+        else {
+            const int64_t b2 = lcp_climb<G, true, STATS>(ix, ba, d, mreq);
+            if (b2 >= 0) {
+                const LaneBlock<G> Cb = load_block<G>(ix.lcp8, (uint32_t)b2, lane);
+                if (STATS) ++lreq;
+                lcp_masks<G>(Cb, dd, lt, esc);
+                k = lcp_scan<true, STATS>(ix, (uint32_t)b2, lt, esc, 63, d, lreq);
+                nsp = (uint32_t)b2 * kLcpRows + (uint32_t)k + 1u;
+            }
+        }
+    }
+    if (vb < d) nep = ep;
+    else {
+        lcp_masks<G>(B, dd, lt, esc);
+        int k = lcp_scan<false, STATS>(ix, bb, lt, esc, ob, d, lreq);
+        if (k < 64) nep = bb * kLcpRows + (uint32_t)k + 1u;
+        else {                                                     // LCP[n-1] = 0: there always is a block on the right
+            const uint32_t b2 = (uint32_t)lcp_climb<G, false, STATS>(ix, bb, d, mreq);
+            const LaneBlock<G> Cb = load_block<G>(ix.lcp8, b2, lane);
+            if (STATS) ++lreq;
+            lcp_masks<G>(Cb, dd, lt, esc);
+            k = lcp_scan<false, STATS>(ix, b2, lt, esc, 0, d, lreq);
+            nep = b2 * kLcpRows + (uint32_t)k + 1u;
+        }
+    }
+    sp = nsp; ep = nep; l = d;
 }
 
 // ---- wide-interval dictionary probe ----------------------------------------------------------------------------------------------

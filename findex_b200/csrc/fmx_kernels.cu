@@ -260,6 +260,77 @@ count_var_kernel(const __grid_constant__ DevIndex ix, const uint8_t *__restrict_
     }
 }
 
+// ---- matching statistics (fmx_match_stats_batch / fmx_smem_*; include/fmgpu.h) -----------------------------------------------------
+// One query per group, left to right (file order), state (l, sp, ep) = the longest suffix S of the query so far that occurs and the
+// interval of reverse(S).  A symbol extends S by one backward step; when the step comes back empty, the interval is widened to its LCP
+// parent (lcp_widen) and the step retried, until it succeeds or l = 0 (from (0, n) the step is (C[c], C[c+1]), no request).  Each retry
+// lowers l, so a query of length L takes at most 2L steps and L widenings.  Outputs by text position off[q] + j: ms_len, and the interval
+// when ms_sp != nullptr; flag != nullptr: flag = 1 where an SMEM of at least min_len symbols ends (ms_len[j] >= min_len and j is the last
+// position or ms_len[j+1] <= ms_len[j]).  STATS: stats[0..2] += rank blocks, lcp8 blocks + record / lcpx reads, minima lines.
+template <int G, int LAYOUT, bool STATS>
+__global__ void __launch_bounds__(kThreads)
+match_kernel(const __grid_constant__ DevIndex ix, const uint8_t *__restrict__ pat, const long long *__restrict__ off, long long m,
+             int *__restrict__ ms_len, uint32_t *__restrict__ ms_sp, uint32_t *__restrict__ ms_ep, uint32_t *__restrict__ flag, int min_len,
+             unsigned long long *__restrict__ stats) {
+    __shared__ SharedTables tb;
+    load_tables(tb, ix);
+    __syncthreads();
+    const long long q = (long long)blockIdx.x * (kThreads / G) + threadIdx.x / G;
+    if (q >= m) return;                                                   // group-uniform; only group shuffles follow
+    const bool lead = (threadIdx.x % G) == 0;
+    const long long lo = off[q], hi = off[q + 1];
+    uint32_t l = 0, sp = 0, ep = ix.n, prev = 0, rank_req = 0, lcp_req = 0, min_req = 0;
+    for (long long i = lo; i < hi; ++i) {
+        const uint32_t c = __ldg(pat + i);
+        for (;;) {
+            if (l == 0) {
+                sp = tb.C[c]; ep = tb.C[c + 1];
+                if (sp < ep) l = 1; else { sp = 0; ep = ix.n; }
+                break;
+            }
+            uint32_t s = sp, e = ep;
+            backward_step<G, LAYOUT, STATS>(ix, tb, c, s, e, rank_req);
+            if (s < e) { sp = s; ep = e; ++l; break; }
+            lcp_widen<G, STATS>(ix, sp, ep, l, lcp_req, min_req);
+        }
+        if (lead) {
+            ms_len[i] = (int)l;
+            if (ms_sp) { ms_sp[i] = sp; ms_ep[i] = ep; }
+            if (flag && i > lo) flag[i - 1] = (prev >= (uint32_t)min_len && l <= prev) ? 1u : 0u;
+        }
+        prev = l;
+    }
+    if (lead && flag && hi > lo) flag[hi - 1] = prev >= (uint32_t)min_len ? 1u : 0u;
+    if (STATS && lead) {
+        atomicAdd(&stats[0], (unsigned long long)rank_req);
+        atomicAdd(&stats[1], (unsigned long long)lcp_req);
+        atomicAdd(&stats[2], (unsigned long long)min_req);
+    }
+}
+
+// SMEM offsets per query: out_off[q] = the exclusive scan of the flags at the query's first position (q = m: the total)
+__global__ void smem_offsets_kernel(const uint32_t *__restrict__ scan, const long long *__restrict__ off, long long m, long long *__restrict__ out_off) {
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q <= m) out_off[q] = (long long)scan[off[q]];
+}
+
+// every flagged position i -> its SMEM (start inside the query, length, interval) at slot scan[i]
+__global__ void smem_compact_kernel(const uint32_t *__restrict__ flag, const uint32_t *__restrict__ scan, const int *__restrict__ ms_len,
+                                    const uint32_t *__restrict__ ms_sp, const uint32_t *__restrict__ ms_ep, const long long *__restrict__ off,
+                                    long long m, long long T, int *__restrict__ start, int *__restrict__ len, uint32_t *__restrict__ sp,
+                                    uint32_t *__restrict__ ep) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= T || !flag[i]) return;
+    long long a = 0, b = m;                                               // the query: last q < m with off[q] <= i
+    while (b - a > 1) { const long long mid = (a + b) >> 1; if (off[mid] <= i) a = mid; else b = mid; }
+    const uint32_t k = scan[i];
+    const int l = ms_len[i];
+    start[k] = (int)(i - off[a]) - l + 1;
+    len[k] = l;
+    sp[k] = ms_sp[i];
+    ep[k] = ms_ep[i];
+}
+
 // =====================================================================================================
 // element-wise operator calls
 // =====================================================================================================
@@ -723,6 +794,31 @@ cudaError_t launch_count_var(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d
     dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
         count_var_kernel<g, lay><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_pat, (const long long *)d_off, m, (long long *)d_sp, (long long *)d_ep);
     });
+    return cudaGetLastError();
+}
+
+cudaError_t launch_match(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_pat, const int64_t *d_off, int64_t m, int32_t *d_len,
+                         uint32_t *d_sp, uint32_t *d_ep, uint32_t *d_flag, int min_len, unsigned long long *d_stats, cudaStream_t st) {
+    if (m <= 0) return cudaSuccess;
+    if (ix.lcp8 == nullptr) return cudaErrorInvalidValue;
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) {
+        if (d_stats) match_kernel<g, lay, true><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_pat, (const long long *)d_off, m, d_len, d_sp, d_ep, d_flag, min_len, d_stats);
+        else match_kernel<g, lay, false><<<grid_for(m, g), kThreads, 0, st>>>(ix, d_pat, (const long long *)d_off, m, d_len, d_sp, d_ep, d_flag, min_len, nullptr);
+    });
+    return cudaGetLastError();
+}
+
+cudaError_t launch_smem_offsets(const uint32_t *d_scan, const int64_t *d_off, int64_t m, int64_t *d_out_off, cudaStream_t st) {
+    smem_offsets_kernel<<<(unsigned)((m + 1 + 255) / 256), 256, 0, st>>>(d_scan, (const long long *)d_off, m, (long long *)d_out_off);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_smem_compact(const uint32_t *d_flag, const uint32_t *d_scan, const int32_t *d_ms_len, const uint32_t *d_ms_sp,
+                                const uint32_t *d_ms_ep, const int64_t *d_off, int64_t m, int64_t T, int32_t *d_start, int32_t *d_len,
+                                uint32_t *d_sp, uint32_t *d_ep, cudaStream_t st) {
+    if (T <= 0 || m <= 0) return cudaSuccess;
+    smem_compact_kernel<<<(unsigned)((T + 255) / 256), 256, 0, st>>>(d_flag, d_scan, d_ms_len, d_ms_sp, d_ms_ep, (const long long *)d_off, m, T,
+                                                                     d_start, d_len, d_sp, d_ep);
     return cudaGetLastError();
 }
 

@@ -45,6 +45,17 @@ cudaError_t launch_count_fixed(const DevIndex &ix, LaunchCfg cfg, const uint8_t 
 // count: variable-length patterns with int64 offsets.
 cudaError_t launch_count_var(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_pat, const int64_t *d_off, int64_t m,
                              int64_t *d_sp, int64_t *d_ep, cudaStream_t st);
+// matching statistics of m queries (d_off[m+1]: query q = d_pat[off[q] .. off[q+1])), outputs by text position: d_len, and (sp, ep) when
+// d_sp != nullptr; d_flag != nullptr: 1 where an SMEM of at least min_len symbols ends, else 0 (positions outside every query are not
+// written).  d_stats != nullptr: += { rank blocks, lcp8 blocks + record / lcpx reads, minima lines } (the counting instance).  Needs ix.lcp8.
+cudaError_t launch_match(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_pat, const int64_t *d_off, int64_t m, int32_t *d_len,
+                         uint32_t *d_sp, uint32_t *d_ep, uint32_t *d_flag, int min_len, unsigned long long *d_stats, cudaStream_t st);
+// SMEMs from the flags: d_scan = exclusive scan of d_flag over the T positions (+ the total at T); d_out_off[q] = d_scan[d_off[q]], q <= m;
+// every flagged position's SMEM goes to slot d_scan[i] (start inside its query, length, interval)
+cudaError_t launch_smem_offsets(const uint32_t *d_scan, const int64_t *d_off, int64_t m, int64_t *d_out_off, cudaStream_t st);
+cudaError_t launch_smem_compact(const uint32_t *d_flag, const uint32_t *d_scan, const int32_t *d_ms_len, const uint32_t *d_ms_sp,
+                                const uint32_t *d_ms_ep, const int64_t *d_off, int64_t m, int64_t T, int32_t *d_start, int32_t *d_len,
+                                uint32_t *d_sp, uint32_t *d_ep, cudaStream_t st);
 cudaError_t launch_occ(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_c, const int64_t *d_key, int64_t m,
                        int64_t *d_out, cudaStream_t st);
 cudaError_t launch_prev_range(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_sp, const int64_t *d_ep,

@@ -40,7 +40,7 @@ class fmx_opts(C.Structure):
     _fields_ = [("device", C.c_int32), ("layout", C.c_int32), ("sa_sample_rate", C.c_int32), ("require_fm", C.c_int32),
                 ("max_index_bytes", C.c_int64), ("lanes_per_query", C.c_int32), ("accel", C.c_int32), ("kmer_table_bytes", C.c_int64),
                 ("max_total_bytes", C.c_int64), ("dict_bytes", C.c_int64), ("dict_min_rows", C.c_int32), ("dict_top_min_rows", C.c_int32),
-                ("text_sample_rate", C.c_int32)]
+                ("text_sample_rate", C.c_int32), ("lcp", C.c_int32)]
 
 
 _lib = None
@@ -109,6 +109,12 @@ def lib():
     L.fmx_text_batch.argtypes = [p, p, i64, i32, p, p]
     L.fmx_text_dev.argtypes = [p, p, i64, i32, p, p, p]
     L.fmx_next_substr_batch.argtypes = [p, p, i64, i32, p, p]
+    L.fmx_lcp_bytes.restype = i64
+    L.fmx_lcp_bytes.argtypes = [p]
+    L.fmx_match_stats_batch.argtypes = [p, p, p, i64, p, p, p]
+    L.fmx_smem_batch.argtypes = [p, p, p, i64, i32, i64, p, p, p, p, p]
+    L.fmx_smem_dev.argtypes = [p, p, p, i64, i32, p, p, p, p, p, i64, C.POINTER(i64), p]
+    L.fmx_last_match_requests.argtypes = [p, p]
     L.fmx_regex_compile.argtypes = [p, i64, C.c_int, pp]
     L.fmx_regex_compile_engine.argtypes = [p, i64, C.c_int, C.c_int, pp]
     L.fmx_regex_free.argtypes = [p]
@@ -165,7 +171,7 @@ def _u8(a):
 
 
 def make_opts(device=-1, layout=LAYOUT_AUTO, sa_sample_rate=0, require_fm=False, max_index_bytes=0, lanes_per_query=0, accel=ACCEL_AUTO,
-              kmer_table_bytes=0, max_total_bytes=0, dict_bytes=0, dict_min_rows=0, dict_top_min_rows=0, text_sample_rate=0):
+              kmer_table_bytes=0, max_total_bytes=0, dict_bytes=0, dict_min_rows=0, dict_top_min_rows=0, text_sample_rate=0, lcp=0):
     o = fmx_opts()
     lib().fmx_opts_default(C.byref(o))
     o.device, o.layout, o.sa_sample_rate = device, layout, sa_sample_rate
@@ -174,6 +180,7 @@ def make_opts(device=-1, layout=LAYOUT_AUTO, sa_sample_rate=0, require_fm=False,
     o.max_total_bytes = max_total_bytes
     o.dict_bytes, o.dict_min_rows, o.dict_top_min_rows = dict_bytes, dict_min_rows, dict_top_min_rows
     o.text_sample_rate = text_sample_rate
+    o.lcp = int(lcp)
     return o
 
 
@@ -313,7 +320,8 @@ class GpuFMSearcher:
                 "dict_depth": dd.value, "dict_chain_depth": dx.value, "dict_entries": de.value, "dict_bytes": db.value,
                 "index_bytes": nb.value, "sa_sample_rate": rate.value, "kmer_k": k.value, "kmer_rows": lib().fmx_kmer_rows(self.h), "text_shortcut": bool(t.value),
                 "ctx_depth": lib().fmx_ctx_depth(self.h), "ctx_entry_bytes": lib().fmx_ctx_entry_bytes(self.h),
-                "lanes_per_query": lib().fmx_get_lanes(self.h), "text_sample_rate": lib().fmx_text_sample_rate(self.h)}
+                "lanes_per_query": lib().fmx_get_lanes(self.h), "text_sample_rate": lib().fmx_text_sample_rate(self.h),
+                "lcp_bytes": lib().fmx_lcp_bytes(self.h)}
 
     # ---- scalar trait members (each is a batch of one) -------------------------------------------------
     def cf(self, c):
@@ -488,6 +496,58 @@ class GpuFMSearcher:
         """fmx_text_dev (raw device pointers as ints): uint32 file offsets [m] in, uint8 [m, length] rows and int32 lengths out;
         asynchronous on `stream`"""
         _check(lib().fmx_text_dev(self.h, C.c_void_p(d_off), m, length, C.c_void_p(d_out), C.c_void_p(d_out_len), C.c_void_p(stream)))
+
+    # ---- longest matches (index opened with lcp=1; include/fmgpu.h) --------------------------------------------------------------------
+    @staticmethod
+    def _queries(queries):
+        off = np.zeros(len(queries) + 1, np.int64)
+        np.cumsum([len(x) for x in queries], out=off[1:])
+        pat = _u8(b"".join(bytes(x) for x in queries)) if off[-1] else np.zeros(1, np.uint8)
+        return pat, off
+
+    def match_stats(self, queries, intervals=True):
+        """fmx_match_stats_batch over queries in file order (list of bytes): (off[m+1], ms_len int32, ms_sp, ms_ep int64), entry off[q] + j
+        for position j of query q; ms_len[i] = the longest l such that the l bytes ending there occur, (ms_sp, ms_ep) = count of their
+        reverse ((0, n) when l = 0).  intervals=False skips the intervals (None)."""
+        pat, off = self._queries(queries)
+        T = int(off[-1])
+        ln = np.zeros(max(T, 1), np.int32)
+        sp = np.zeros(max(T, 1), np.int64) if intervals else None
+        ep = np.zeros(max(T, 1), np.int64) if intervals else None
+        _check(lib().fmx_match_stats_batch(self.h, _ptr(pat), _ptr(off), len(queries), _ptr(ln), None if sp is None else _ptr(sp),
+                                           None if ep is None else _ptr(ep)))
+        return off, ln[:T], (sp[:T] if intervals else None), (ep[:T] if intervals else None)
+
+    def smems(self, queries, min_len=1, cap_total=1 << 20):
+        """fmx_smem_batch: (out_off[m+1], start, len, sp, ep) — the SMEMs of at least min_len bytes of query q are entries
+        out_off[q] .. out_off[q+1], in increasing start order; start is inside the query (file order)"""
+        pat, off = self._queries(queries)
+        m = len(queries)
+        out_off = np.zeros(m + 1, np.int64)
+        while True:
+            k = max(cap_total, 1)
+            st, ln, sp, ep = np.zeros(k, np.int32), np.zeros(k, np.int32), np.zeros(k, np.int64), np.zeros(k, np.int64)
+            rc = lib().fmx_smem_batch(self.h, _ptr(pat), _ptr(off), m, min_len, cap_total, _ptr(out_off), _ptr(st), _ptr(ln), _ptr(sp), _ptr(ep))
+            if rc == FMX_E_CAPACITY:
+                cap_total = int(out_off[m])
+                continue
+            _check(rc)
+            t = int(out_off[m])
+            return out_off, st[:t], ln[:t], sp[:t], ep[:t]
+
+    def smems_dev(self, d_pat, d_off, m, min_len, d_out_off, d_start, d_len, d_sp, d_ep, cap, stream=0):
+        """fmx_smem_dev (raw device pointers as ints): uint8 queries and int64 offsets [m+1] in; int64 out_off [m+1], int32 start / len and
+        uint32 sp / ep [cap] out.  Returns the number of SMEMs; raises FmxError(FMX_E_CAPACITY) when cap is too small."""
+        total = C.c_int64()
+        _check(lib().fmx_smem_dev(self.h, C.c_void_p(d_pat), C.c_void_p(d_off), m, min_len, C.c_void_p(d_out_off), C.c_void_p(d_start),
+                                  C.c_void_p(d_len), C.c_void_p(d_sp), C.c_void_p(d_ep), cap, C.byref(total), C.c_void_p(stream)))
+        return total.value
+
+    def last_match_requests(self):
+        """(rank blocks, LCP block / record / escape reads, minima lines) of the last match call with set_stats(True)"""
+        r = np.zeros(3, np.int64)
+        _check(lib().fmx_last_match_requests(self.h, _ptr(r)))
+        return tuple(int(x) for x in r)
 
     def regex_search_batch(self, trees, cap_total=1 << 20):
         """trees: list of ReTree.  Returns per regex the sorted list of (len, sp, ep)."""

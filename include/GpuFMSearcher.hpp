@@ -101,6 +101,28 @@ public:
         for (size_t i = 0; i < off.size(); ++i) r.emplace_back(reinterpret_cast<const char *>(out.data()) + i * (size_t)len, (size_t)ol[i]);
         return r;
     }
+    // longest matches (index opened with fmx_opts.lcp = 1) of a query in file order: for every position j the length of the longest
+    // match ending there and the interval of its reverse ((0, n) for length 0); the SMEMs of at least min_len bytes in increasing start order
+    struct MatchStats { std::vector<int32_t> len; std::vector<int64_t> sp, ep; };
+    MatchStats matchStats(const std::string &q) const {
+        MatchStats r;
+        r.len.resize(q.size()); r.sp.resize(q.size()); r.ep.resize(q.size());
+        const int64_t off[2] = {0, (int64_t)q.size()};
+        check(fmx_match_stats_batch(h_, reinterpret_cast<const uint8_t *>(q.data()), off, 1, r.len.data(), r.sp.data(), r.ep.data()));
+        return r;
+    }
+    struct Smem { int32_t start, len; int64_t sp, ep; };
+    std::vector<Smem> smems(const std::string &q, int32_t min_len = 1) const {
+        const int64_t off[2] = {0, (int64_t)q.size()};
+        int64_t oo[2] = {0, 0};
+        const int64_t cap = (int64_t)q.size() + 1;                 // at most one SMEM ends at each position
+        std::vector<int32_t> st((size_t)cap), ln((size_t)cap);
+        std::vector<int64_t> sp((size_t)cap), ep((size_t)cap);
+        check(fmx_smem_batch(h_, reinterpret_cast<const uint8_t *>(q.data()), off, 1, min_len, cap, oo, st.data(), ln.data(), sp.data(), ep.data()));
+        std::vector<Smem> r;
+        for (int64_t k = 0; k < oo[1]; ++k) r.push_back({st[(size_t)k], ln[(size_t)k], sp[(size_t)k], ep[(size_t)k]});
+        return r;
+    }
     std::string nextSubstr(int64_t sp, int len) const {
         std::string out((size_t)(len > 0 ? len : 1), '\0'); int32_t ol = 0;
         check(fmx_next_substr_batch(h_, &sp, 1, len, reinterpret_cast<uint8_t *>(&out[0]), &ol));

@@ -86,6 +86,8 @@ typedef struct fmx_opts {
                                    everything that occurs twice, when it fits the budget, else dict_min_rows                                   */
     int32_t  text_sample_rate;  /* 0 = none; s in 1..65536: the row of every s-th text position is kept (4 * ((n-1)/s + 1) bytes), which
                                    fmx_text_batch / fmx_text_dev start their walks from                                                   */
+    int32_t  lcp;               /* 0 = none; 1 = build the LCP structure of the matching-statistics / SMEM calls at open (about 1.13 n bytes + 4 bytes
+                                   per row whose LCP is >= 255; counted in index_bytes and checked against max_total_bytes)                   */
 } fmx_opts;
 
 void        fmx_opts_default(fmx_opts *o);
@@ -225,6 +227,36 @@ int fmx_text_batch(fmx_index *ix, const int64_t *off, int64_t m, int32_t len, ui
 /* device-resident, asynchronous on `stream`: d_off uint32[m] file offsets, d_out uint8[m*len], d_out_len int32[m]; an offset above
  * n-1 is not checked on the host and yields out_len = -1                                                                               */
 int fmx_text_dev(fmx_index *ix, const void *d_off_u32, int64_t m, int32_t len, void *d_out, void *d_out_len, void *stream);
+
+/* ---- longest matches: matching statistics and super-maximal exact matches (SMEMs) ------------------------------------------------
+ * A query Q is a byte string in file order (the order the regex engines feed getPrevRange).  A substring S of Q occurs when
+ * search(reverse(S)) is Some, i.e. when S is a substring of F + "\0" + F (F = the file with its 0x00 bytes dropped; queries of at most
+ * |F| + 1 bytes): the backward search is cyclic at '$', so a 0x00 in a query stands for the boundary between the file's last byte and
+ * its first, exactly as in the count calls.
+ *   matching statistics: for every position j of Q, ms_len[j] = the largest l such that Q[j-l+1 .. j] occurs, and (ms_sp[j], ms_ep[j]) =
+ *     the interval fmx_count_batch gives its reverse ((0, n) when l = 0).  Outputs are indexed like the query bytes: entry off[q] + j.
+ *   SMEMs of at least min_len symbols: for every j with l = ms_len[j] >= min_len and (j = |Q| - 1 or ms_len[j+1] <= l) the match
+ *     (start = j - l + 1, len = l, sp, ep) — exactly the substrings of Q that occur and lie in no longer substring of Q that occurs;
+ *     per query in increasing start (and end) order, out_off[m+1] = the exclusive offsets.
+ * Each position is one backward step from the previous state; a step that comes back empty widens the interval to its LCP parent
+ * (fmx_opts.lcp) and is retried: at most 2|Q| steps and |Q| widenings per query.  FMX_E_UNSUPPORTED when the index was opened without
+ * lcp; FMX_E_ARG for null pointers, decreasing offsets or min_len < 1; with fmx_set_stats(ix, 1), fmx_last_steps = the index requests of
+ * the last call and fmx_last_match_requests their split.                                                                             */
+int64_t fmx_lcp_bytes(const fmx_index *ix);                 /* bytes of the LCP structure, 0 = not built */
+/* ms arrays hold off[m] entries; ms_sp / ms_ep may be NULL */
+int fmx_match_stats_batch(fmx_index *ix, const uint8_t *pat, const int64_t *off, int64_t m, int32_t *ms_len, int64_t *ms_sp, int64_t *ms_ep);
+/* out_off[m+1]; FMX_E_CAPACITY with the required total in out_off[m] when cap_total is too small (nothing is written to the SMEM arrays) */
+int fmx_smem_batch(fmx_index *ix, const uint8_t *pat, const int64_t *off, int64_t m, int32_t min_len, int64_t cap_total,
+                   int64_t *out_off, int32_t *start, int32_t *len, int64_t *sp, int64_t *ep);
+/* device-resident, on `stream`: d_off int64[m+1] (not checked on the host; off[m] is read back to size the scratch), d_out_off int64[m+1],
+ * SMEMs into d_start / d_len (int32[cap]) and d_sp / d_ep (uint32[cap], exactly as fmx_locate_dev takes them: seed -> locate without the
+ * host).  Synchronises `stream` once to learn the total (*total_out); FMX_E_CAPACITY when it exceeds cap, and nothing is written past cap. */
+int fmx_smem_dev(fmx_index *ix, const void *d_pat, const void *d_off_i64, int64_t m, int32_t min_len,
+                 void *d_out_off_i64, void *d_start_i32, void *d_len_i32, void *d_sp_u32, void *d_ep_u32,
+                 int64_t cap, int64_t *total_out, void *stream);
+/* the last counting (fmx_set_stats) match call's index requests: req[0] = rank blocks of the backward steps, req[1] = 64-byte LCP
+ * blocks and the record / escaped-value reads, req[2] = 128-byte minima lines of the widenings that leave their block                */
+int fmx_last_match_requests(const fmx_index *ix, int64_t req[3]);
 
 /* ---- regex: REParser.re2post M/re2/re2.scala:50-185 + ReTree.apply M/re2/retree.scala:156-370 -------
  * Compiles on the host to the reference's Glushkov position automaton, quirks included (SURVEY Q1-Q5);
