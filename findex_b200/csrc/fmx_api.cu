@@ -1382,6 +1382,158 @@ int fmx_smem_dev(fmx_index *ix, const void *d_pat, const void *d_off, int64_t m,
     return FMX_OK;
 }
 
+// ---- k-mer census (include/fmgpu.h) -----------------------------------------------------------------------------------------------
+}  // extern "C"
+
+namespace {
+int census_unsupported() {
+    return fail(FMX_E_UNSUPPORTED, "the k-mer census needs the LCP structure: open the index with fmx_opts.lcp = 1");
+}
+
+int check_list_args(int32_t k, int64_t min_count, int64_t max_count) {
+    if (k < 1) return fail(FMX_E_ARG, "k = %d: at least 1", k);
+    if (min_count < 1 || max_count < 0 || (max_count > 0 && max_count < min_count))
+        return fail(FMX_E_ARG, "min_count = %lld, max_count = %lld: 1 <= min_count, and max_count = 0 (no bound) or >= min_count", (long long)min_count,
+                    (long long)max_count);
+    return FMX_OK;
+}
+
+// every tile's open run: d_incl[t] = the row after the last run end in tiles 0 .. t (tile t + 1 starts its first run there)
+int census_open_runs(CallCtx &cc, uint32_t k, DBuf &dincl, cudaStream_t st) {
+    const int64_t ntiles = census_tiles(cc.ix->n);
+    DBuf dlast(st);
+    CU(dlast.alloc((size_t)ntiles * 4)); CU(dincl.alloc((size_t)ntiles * 4));
+    CU(launch_census_last(cc.d, k, dlast.as<uint32_t>(), st));
+    CU(inclusive_max_u32(dlast.as<uint32_t>(), dincl.as<uint32_t>(), ntiles, st));
+    return FMX_OK;
+}
+
+// The counting half of a listing (1 <= k <= |F| = n - 1): open runs, the sorted short-suffix rows when min_count = 1 (k - 1 LF
+// steps from row 0), the qualifying runs per tile and their exclusive scan (d_off[ntiles] = the total, read back: one synchronisation).
+struct CensusList {
+    DBuf incl, ex, cnt, off;
+    uint32_t nex = 0, mn = 0, mx = 0;
+    int64_t total = 0;
+    explicit CensusList(cudaStream_t st) : incl(st), ex(st), cnt(st), off(st) {}
+};
+int census_count(CallCtx &cc, uint32_t k, int64_t min_count, int64_t max_count, CensusList &L, cudaStream_t st) {
+    const int64_t ntiles = census_tiles(cc.ix->n);
+    // counts are < 2^32 - 1: a lower bound beyond that lists nothing, an upper bound beyond it bounds nothing
+    L.mn = (uint32_t)std::min<int64_t>(min_count, 0xFFFFFFFFll);
+    L.mx = max_count >= 0xFFFFFFFFll ? 0u : (uint32_t)max_count;
+    int rc = census_open_runs(cc, k, L.incl, st);
+    if (rc) return rc;
+    if (L.mn == 1) {
+        DBuf walk(st);
+        L.nex = k;
+        CU(walk.alloc((size_t)k * 4)); CU(L.ex.alloc((size_t)k * 4));
+        CU(launch_census_walk(cc.d, cc.cfg, k - 1, walk.as<uint32_t>(), st));
+        CU(radix_sort_u32(walk.as<uint32_t>(), L.ex.as<uint32_t>(), k, st));
+    }
+    CU(L.cnt.alloc((size_t)(ntiles + 1) * 4)); CU(L.off.alloc((size_t)(ntiles + 1) * 4));
+    CU(cudaMemsetAsync(L.cnt.as<uint32_t>() + ntiles, 0, 4, st));
+    CU(launch_census_list(cc.d, k, L.incl.as<uint32_t>(), L.mn, L.mx, L.ex.as<uint32_t>(), L.nex, L.cnt.as<uint32_t>(), nullptr, nullptr, nullptr, st));
+    CU(exclusive_sum_u32(L.cnt.as<uint32_t>(), L.off.as<uint32_t>(), ntiles + 1, st));
+    uint32_t total = 0;
+    CU(cudaMemcpyAsync(&total, L.off.as<uint32_t>() + ntiles, 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    L.total = total;
+    cc.ix->last_launches = 4 + (L.mn == 1 ? 2 : 0); cc.ix->total_launches += cc.ix->last_launches;
+    return FMX_OK;
+}
+
+int census_emit(CallCtx &cc, uint32_t k, CensusList &L, uint32_t *d_sp, uint32_t *d_ep, cudaStream_t st) {
+    if (L.total == 0) return FMX_OK;
+    CU(launch_census_list(cc.d, k, L.incl.as<uint32_t>(), L.mn, L.mx, L.ex.as<uint32_t>(), L.nex, nullptr, L.off.as<uint32_t>(), d_sp, d_ep, st));
+    cc.ix->last_launches += 1; cc.ix->total_launches += 1;
+    return FMX_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int fmx_kmer_spectrum(fmx_index *ix, int32_t k, int32_t buckets, int64_t *hist, int64_t *distinct, int64_t *max_occ) {
+    CHECK_IX(ix);
+    if (k < 1 || buckets < 1) return fail(FMX_E_ARG, "k = %d, buckets = %d: both at least 1", k, buckets);
+    if (!hist || !distinct || !max_occ) return fail(FMX_E_ARG, "null argument");
+    if (ix->d_full.lcp8 == nullptr) return census_unsupported();
+    std::fill(hist, hist + buckets, 0);
+    *distinct = 0; *max_occ = 0;
+    if (k > ix->n - 1) return FMX_OK;                                 // no window of k symbols in F
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = cc.stream;
+    DBuf dincl(st), dh(st);
+    CU(dh.alloc((size_t)(buckets + 1) * 8));
+    CU(cudaMemsetAsync(dh.p, 0, (size_t)(buckets + 1) * 8, st));
+    const int rc = census_open_runs(cc, (uint32_t)k, dincl, st);
+    if (rc) return rc;
+    unsigned long long *h = dh.as<unsigned long long>();
+    CU(launch_census_spectrum(cc.d, (uint32_t)k, dincl.as<uint32_t>(), (uint32_t)buckets, h, h + buckets, st));
+    ix->last_launches = 3; ix->total_launches += 3;
+    CU(cudaMemcpyAsync(hist, h, (size_t)buckets * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(max_occ, h + buckets, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    hist[0] -= k;                                                     // the k short-suffix rows: runs of one row that are no k-mer
+    int64_t d = 0;
+    for (int32_t b = 0; b < buckets; ++b) d += hist[b];
+    *distinct = d;
+    return FMX_OK;
+}
+
+int fmx_kmer_list_batch(fmx_index *ix, int32_t k, int64_t min_count, int64_t max_count, int64_t cap, int64_t *total, int64_t *sp, int64_t *ep) {
+    CHECK_IX(ix);
+    int rc = check_list_args(k, min_count, max_count);
+    if (rc) return rc;
+    if (!total || cap < 0 || (cap > 0 && (!sp || !ep))) return fail(FMX_E_ARG, "bad argument");
+    if (ix->d_full.lcp8 == nullptr) return census_unsupported();
+    *total = 0;
+    if (k > ix->n - 1) return FMX_OK;
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = cc.stream;
+    CensusList L(st);
+    rc = census_count(cc, (uint32_t)k, min_count, max_count, L, st);
+    if (rc) return rc;
+    *total = L.total;
+    if (L.total > cap) return fail(FMX_E_CAPACITY, "the listing holds %lld k-mers, capacity %lld", (long long)L.total, (long long)cap);
+    if (L.total == 0) return FMX_OK;
+    DBuf d32(st), d64(st);
+    CU(d32.alloc((size_t)L.total * 8)); CU(d64.alloc((size_t)L.total * 16));
+    uint32_t *dsp = d32.as<uint32_t>(), *dep = dsp + L.total;
+    rc = census_emit(cc, (uint32_t)k, L, dsp, dep, st);
+    if (rc) return rc;
+    CU(widen_u32_i64(dsp, d64.as<int64_t>(), L.total, st));
+    CU(widen_u32_i64(dep, d64.as<int64_t>() + L.total, L.total, st));
+    CU(cudaMemcpyAsync(sp, d64.p, (size_t)L.total * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(ep, d64.as<int64_t>() + L.total, (size_t)L.total * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return FMX_OK;
+}
+
+int fmx_kmer_list_dev(fmx_index *ix, int32_t k, int64_t min_count, int64_t max_count, void *d_sp, void *d_ep, int64_t cap, int64_t *total_out,
+                      void *stream) {
+    CHECK_IX(ix);
+    int rc = check_list_args(k, min_count, max_count);
+    if (rc) return rc;
+    if (!total_out || cap < 0 || (cap > 0 && (!d_sp || !d_ep))) return fail(FMX_E_ARG, "bad argument");
+    if (ix->d_full.lcp8 == nullptr) return census_unsupported();
+    *total_out = 0;
+    if (k > ix->n - 1) return FMX_OK;
+    CallCtx cc(ix);
+    CHECK_CC(cc);
+    DeviceGuard g(ix->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    CensusList L(st);
+    rc = census_count(cc, (uint32_t)k, min_count, max_count, L, st);
+    if (rc) return rc;
+    *total_out = L.total;
+    if (L.total > cap) return fail(FMX_E_CAPACITY, "the listing holds %lld k-mers, capacity %lld", (long long)L.total, (long long)cap);
+    return census_emit(cc, (uint32_t)k, L, (uint32_t *)d_sp, (uint32_t *)d_ep, st);
+}
+
 // ---- locate ---------------------------------------------------------------------------------------------------
 namespace {
 bool debug_sync() { static const bool on = std::getenv("FMX_DEBUG_SYNC") != nullptr; return on; }     // synchronise + check after each stage

@@ -331,6 +331,206 @@ __global__ void smem_compact_kernel(const uint32_t *__restrict__ flag, const uin
     ep[k] = ms_ep[i];
 }
 
+// ---- k-mer census (fmx_kmer_spectrum / fmx_kmer_list_*; include/fmgpu.h) --------------------------------------------------------------
+// Row r < n-1 ends a run of rows that share their first k symbols when LCP[r] < k; row n-1 always does (its LCP is 0).  The run from the
+// row after the previous end to an end row e is the interval [start, e+1) of one k-mer, or one of the k single rows whose suffix is
+// shorter than k + 1 ('$' within its first k symbols).  One streaming pass over lcp8: a warp owns a tile of kCensusTile consecutive
+// 64-row blocks and walks it 32 blocks (one per lane, two 32-byte loads) at a time; each lane turns its block into the 64-bit mask of its
+// end rows.  The run open at a lane's first row comes from the lanes before it (a warp max scan of "row after the last end", 0 = none),
+// at a tile's first row from the tiles before it (census_last_kernel, then inclusive_max_u32 over the tiles), so a run may span any
+// number of lanes and tiles.
+constexpr uint32_t kCensusTile = 256, kCensusBuckets = 1024;
+
+__device__ __forceinline__ void ldg256_stream(const uint4 *p, uint4 &a, uint4 &b) {
+    asm volatile("ld.global.nc.L1::no_allocate.L2::256B.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w) : "l"(p));
+}
+
+// end rows of block blk (bit o = row 64 blk + o), 0 past the last block.  For k > 255 the rows with lcp8 = 255 compare their exact LCP,
+// read from lcpx, where a block's escaped values are consecutive from its record's first escape.
+__device__ __forceinline__ unsigned long long census_mask(const DevIndex &ix, uint32_t blk, uint32_t nb, uint32_t k) {
+    if (blk >= nb) return 0ull;
+    uint4 v[4];
+    ldg256_stream(ix.lcp8 + (uint64_t)blk * 4, v[0], v[1]);
+    ldg256_stream(ix.lcp8 + (uint64_t)blk * 4 + 2, v[2], v[3]);
+    const uint32_t dup = (k < kLcpEsc ? k : kLcpEsc) * 0x01010101u;
+    unsigned long long m = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const uint32_t w[4] = {v[i].x, v[i].y, v[i].z, v[i].w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) m |= (unsigned long long)byte_flags4(__vcmpltu4(w[j], dup)) << (16 * i + 4 * j);
+    }
+    const uint32_t rows = ix.n - blk * kLcpRows;
+    const unsigned long long valid = rows < kLcpRows ? (1ull << rows) - 1ull : ~0ull;      // rows >= n pad the last block
+    m &= valid;
+    if (k > kLcpEsc) {
+        unsigned long long esc = ~m & valid;
+        if (esc) {
+            uint32_t x = ldg64(ix.lcp_rec + blk).y;
+            for (; esc; esc &= esc - 1ull, ++x)
+                if (ldg32(ix.lcpx + x) < k) m |= esc & (0ull - esc);
+        }
+    }
+    return m;
+}
+
+// the row after the last end row before this lane's block (lanes before it, else `carry`); carry becomes the warp's last end + 1
+__device__ __forceinline__ uint32_t census_open(unsigned long long m, uint32_t r0, uint32_t &carry) {
+    const int lane = threadIdx.x & 31;
+    uint32_t incl = m ? r0 + 64u - (uint32_t)__clzll((long long)m) : 0u;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t o = __shfl_up_sync(0xFFFFFFFFu, incl, d);
+        if (lane >= d) incl = max(incl, o);
+    }
+    uint32_t excl = __shfl_up_sync(0xFFFFFFFFu, incl, 1);
+    excl = lane == 0 ? 0u : excl;
+    const uint32_t open = max(carry, excl);
+    carry = max(carry, __shfl_sync(0xFFFFFFFFu, incl, 31));
+    return open;
+}
+
+// the start row of the run that ends at bit e of a lane's mask m (block rows from r0; `open` = the start of the lane's first run)
+__device__ __forceinline__ uint32_t census_start(unsigned long long m, int e, uint32_t r0, uint32_t open) {
+    const unsigned long long below = m & ((1ull << e) - 1ull);
+    return below ? r0 + 64u - (uint32_t)__clzll((long long)below) : open;
+}
+
+// tile_last[t] = the row after the last end row of tile t, 0 when it has none; the warp reads its tile backwards and stops at the first
+// 32 blocks that hold an end row (for most k the tile's last ones)
+__global__ void __launch_bounds__(kThreads)
+census_last_kernel(const __grid_constant__ DevIndex ix, uint32_t nb, uint32_t ntiles, uint32_t k, uint32_t *__restrict__ tile_last) {
+    const int lane = threadIdx.x & 31;
+    for (uint32_t t = blockIdx.x * (kThreads / 32) + threadIdx.x / 32; t < ntiles; t += gridDim.x * (kThreads / 32)) {
+        uint32_t after = 0;
+        for (int c = (int)(kCensusTile / 32) - 1; c >= 0; --c) {
+            const uint32_t blk = t * kCensusTile + (uint32_t)c * 32u + (uint32_t)lane;
+            const unsigned long long m = census_mask(ix, blk, nb, k);
+            const uint32_t bal = __ballot_sync(0xFFFFFFFFu, m != 0ull);
+            if (bal) {
+                const int hl = 31 - __clz(bal);
+                after = __shfl_sync(0xFFFFFFFFu, m ? blk * kLcpRows + 64u - (uint32_t)__clzll((long long)m) : 0u, hl);
+                break;
+            }
+        }
+        if (lane == 0) tile_last[t] = after;
+    }
+}
+
+// MODE kCensusSpectrum: hist[min(count, buckets) - 1] += 1 and max_occ = max count over every run (the short-suffix rows included; the
+// host takes them out).  Runs of one row (an end row after an end row) are counted by popcount; the others go to a shared histogram of
+// the first kCensusBuckets buckets (one global atomic per non-empty bucket and CTA) or straight to the global one.
+// MODE kCensusCount: tile_cnt[t] = the runs of tile t with min_count <= count <= max_count (0 = no bound) — single rows only when
+// min_count = 1, and then not those in ex[0 .. nex) (sorted: the short-suffix rows).  MODE kCensusEmit: the same runs, (start, end + 1)
+// to sp / ep from slot tile_off[t] on, in row order.
+enum { kCensusSpectrum = 0, kCensusCount = 1, kCensusEmit = 2 };
+template <int MODE>
+__global__ void __launch_bounds__(kThreads)
+census_kernel(const __grid_constant__ DevIndex ix, uint32_t nb, uint32_t ntiles, uint32_t k, const uint32_t *__restrict__ tile_incl,
+              uint32_t buckets, unsigned long long *__restrict__ hist, unsigned long long *__restrict__ max_occ, uint32_t min_count,
+              uint32_t max_count, const uint32_t *__restrict__ ex, uint32_t nex, uint32_t *__restrict__ tile_cnt,
+              const uint32_t *__restrict__ tile_off, uint32_t *__restrict__ sp, uint32_t *__restrict__ ep) {
+    __shared__ uint32_t sh[MODE == kCensusSpectrum ? kCensusBuckets : 1];
+    __shared__ uint32_t sh_max;
+    const int lane = threadIdx.x & 31;
+    const uint32_t nsh = buckets < kCensusBuckets ? buckets : kCensusBuckets;
+    if (MODE == kCensusSpectrum) {
+        for (uint32_t i = threadIdx.x; i < nsh; i += blockDim.x) sh[i] = 0;
+        if (threadIdx.x == 0) sh_max = 0;
+        __syncthreads();
+    }
+    uint32_t ones = 0, mx = 0;
+    for (uint32_t t = blockIdx.x * (kThreads / 32) + threadIdx.x / 32; t < ntiles; t += gridDim.x * (kThreads / 32)) {
+        uint32_t carry = t ? tile_incl[t - 1] : 0u;
+        uint32_t lo = 0, hi = 0, slot = 0;
+        if (MODE != kCensusSpectrum && min_count == 1 && nex) {                // short-suffix rows of this tile: ex[lo .. hi)
+            const uint64_t a = (uint64_t)t * kCensusTile * kLcpRows, b = a + kCensusTile * kLcpRows;
+            uint32_t l = 0, h = nex;
+            while (l < h) { const uint32_t md = (l + h) >> 1; if ((uint64_t)ex[md] < a) l = md + 1; else h = md; }
+            lo = l; h = nex;
+            while (l < h) { const uint32_t md = (l + h) >> 1; if ((uint64_t)ex[md] < b) l = md + 1; else h = md; }
+            hi = l;
+        }
+        if (MODE == kCensusEmit) slot = tile_off[t];
+        uint32_t tcount = 0;
+        for (uint32_t c = 0; c < kCensusTile / 32; ++c) {
+            const uint32_t blk = t * kCensusTile + c * 32u + (uint32_t)lane, r0 = blk * kLcpRows;
+            const unsigned long long m = census_mask(ix, blk, nb, k);
+            if (__all_sync(0xFFFFFFFFu, m == 0ull)) { if (t * kCensusTile + c * 32u >= nb) break; continue; }
+            const uint32_t open = census_open(m, r0, carry);
+            const unsigned long long prev = (m << 1) | (open == r0 ? 1ull : 0ull);   // rows whose previous row ends a run
+            if (MODE == kCensusSpectrum) {
+                ones += (uint32_t)__popcll(m & prev);
+                for (unsigned long long R = m & ~prev; R; R &= R - 1ull) {
+                    const int e = __ffsll((long long)R) - 1;
+                    const uint32_t cnt = r0 + (uint32_t)e + 1u - census_start(m, e, r0, open);
+                    const uint32_t bk = (cnt < buckets ? cnt : buckets) - 1u;
+                    if (bk < kCensusBuckets) atomicAdd(&sh[bk], 1u); else atomicAdd(&hist[bk], 1ull);
+                    mx = max(mx, cnt);
+                }
+                if (m & prev) mx = max(mx, 1u);
+            } else {
+                unsigned long long X = 0;                                    // short-suffix rows of this block
+                if (hi > lo) {
+                    uint32_t l = lo, h = hi;
+                    while (l < h) { const uint32_t md = (l + h) >> 1; if (ex[md] < r0) l = md + 1; else h = md; }
+                    for (; l < hi && ex[l] - r0 < 64u && ex[l] >= r0; ++l) X |= 1ull << (ex[l] - r0);
+                }
+                auto keep = [&](uint32_t cnt) { return cnt >= min_count && (max_count == 0 || cnt <= max_count); };
+                uint32_t cl = min_count == 1 ? (uint32_t)__popcll(m & prev & ~X) : 0u;
+                if (max_count != 1)
+                    for (unsigned long long R = m & ~prev; R; R &= R - 1ull) {
+                        const int e = __ffsll((long long)R) - 1;
+                        cl += keep(r0 + (uint32_t)e + 1u - census_start(m, e, r0, open)) ? 1u : 0u;
+                    }
+                if (MODE == kCensusCount) tcount += cl;
+                else {
+                    uint32_t pre = cl;                                           // exclusive warp scan of the lanes' counts
+#pragma unroll
+                    for (int d = 1; d < 32; d <<= 1) { const uint32_t o = __shfl_up_sync(0xFFFFFFFFu, pre, d); if (lane >= d) pre += o; }
+                    const uint32_t total = __shfl_sync(0xFFFFFFFFu, pre, 31);
+                    uint32_t s = slot + pre - cl;
+                    for (unsigned long long R = cl ? (min_count == 1 ? m & ~X : m & ~prev) : 0ull; R; R &= R - 1ull) {
+                        const int e = __ffsll((long long)R) - 1;
+                        const uint32_t st = census_start(m, e, r0, open), end = r0 + (uint32_t)e + 1u;
+                        if (keep(end - st)) { sp[s] = st; ep[s] = end; ++s; }
+                    }
+                    slot += total;
+                }
+            }
+        }
+        if (MODE == kCensusCount) {
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) tcount += __shfl_xor_sync(0xFFFFFFFFu, tcount, d);
+            if (lane == 0) tile_cnt[t] = tcount;
+        }
+    }
+    if (MODE == kCensusSpectrum) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) { ones += __shfl_xor_sync(0xFFFFFFFFu, ones, d); mx = max(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, d)); }
+        if (lane == 0) { if (ones) atomicAdd(&sh[0], ones); atomicMax(&sh_max, mx); }
+        __syncthreads();
+        for (uint32_t i = threadIdx.x; i < nsh; i += blockDim.x)
+            if (sh[i]) atomicAdd(&hist[i], (unsigned long long)sh[i]);
+        if (threadIdx.x == 0 && sh_max) atomicMax(max_occ, (unsigned long long)sh_max);
+    }
+}
+
+// rows[0 .. steps] = row 0 and the rows of the LF walk from it: the rows of T' positions n-1, n-2, .. n-1-steps (one group)
+template <int G, int LAYOUT>
+__global__ void census_walk_kernel(const __grid_constant__ DevIndex ix, uint32_t steps, uint32_t *__restrict__ rows) {
+    __shared__ SharedTables tb;
+    load_tables(tb, ix);
+    __syncthreads();
+    uint32_t r = 0;
+    if (threadIdx.x == 0) rows[0] = 0;
+    for (uint32_t i = 1; i <= steps; ++i) {
+        r = lf_value<G, LAYOUT>(ix, tb, ix.bwt[r], r);
+        if (threadIdx.x == 0) rows[i] = r;
+    }
+}
+
 // =====================================================================================================
 // element-wise operator calls
 // =====================================================================================================
@@ -819,6 +1019,53 @@ cudaError_t launch_smem_compact(const uint32_t *d_flag, const uint32_t *d_scan, 
     if (T <= 0 || m <= 0) return cudaSuccess;
     smem_compact_kernel<<<(unsigned)((T + 255) / 256), 256, 0, st>>>(d_flag, d_scan, d_ms_len, d_ms_sp, d_ms_ep, (const long long *)d_off, m, T,
                                                                      d_start, d_len, d_sp, d_ep);
+    return cudaGetLastError();
+}
+
+int64_t census_tiles(int64_t n) { return ((n + kLcpRows - 1) / kLcpRows + kCensusTile - 1) / kCensusTile; }
+
+// a grid-stride grid of at most what is resident at once, so that the spectrum's shared histogram is flushed once per resident CTA
+template <typename K> static unsigned census_grid(K kernel, int64_t ntiles) {
+    int dev = 0, sms = 148, per_sm = 1;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0);
+    const int64_t want = (ntiles + kThreads / 32 - 1) / (kThreads / 32);
+    return (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sms * std::max(per_sm, 1)));
+}
+
+cudaError_t launch_census_last(const DevIndex &ix, uint32_t k, uint32_t *d_tile_last, cudaStream_t st) {
+    if (ix.lcp8 == nullptr) return cudaErrorInvalidValue;
+    const int64_t ntiles = census_tiles(ix.n);
+    census_last_kernel<<<census_grid(census_last_kernel, ntiles), kThreads, 0, st>>>(ix, (uint32_t)((ix.n + kLcpRows - 1) / kLcpRows),
+                                                                                  (uint32_t)ntiles, k, d_tile_last);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_census_spectrum(const DevIndex &ix, uint32_t k, const uint32_t *d_tile_incl, uint32_t buckets, unsigned long long *d_hist,
+                                   unsigned long long *d_max, cudaStream_t st) {
+    if (ix.lcp8 == nullptr) return cudaErrorInvalidValue;
+    const int64_t ntiles = census_tiles(ix.n);
+    auto kern = census_kernel<kCensusSpectrum>;
+    kern<<<census_grid(kern, ntiles), kThreads, 0, st>>>(ix, (uint32_t)((ix.n + kLcpRows - 1) / kLcpRows), (uint32_t)ntiles, k, d_tile_incl,
+                                                         buckets, d_hist, d_max, 0, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_census_list(const DevIndex &ix, uint32_t k, const uint32_t *d_tile_incl, uint32_t min_count, uint32_t max_count,
+                               const uint32_t *d_ex, uint32_t nex, uint32_t *d_tile_cnt, const uint32_t *d_tile_off, uint32_t *d_sp,
+                               uint32_t *d_ep, cudaStream_t st) {
+    if (ix.lcp8 == nullptr) return cudaErrorInvalidValue;
+    const int64_t ntiles = census_tiles(ix.n);
+    const uint32_t nb = (uint32_t)((ix.n + kLcpRows - 1) / kLcpRows);
+    auto kern = d_tile_off ? census_kernel<kCensusEmit> : census_kernel<kCensusCount>;
+    kern<<<census_grid(kern, ntiles), kThreads, 0, st>>>(ix, nb, (uint32_t)ntiles, k, d_tile_incl, 1, nullptr, nullptr, min_count, max_count,
+                                                         d_ex, nex, d_tile_cnt, d_tile_off, d_sp, d_ep);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_census_walk(const DevIndex &ix, LaunchCfg cfg, uint32_t steps, uint32_t *d_rows, cudaStream_t st) {
+    dispatch_layout_lanes(cfg.layout, cfg.lanes, [&](auto g, auto lay) { census_walk_kernel<g, lay><<<1, (unsigned)g, 0, st>>>(ix, steps, d_rows); });
     return cudaGetLastError();
 }
 

@@ -56,6 +56,21 @@ cudaError_t launch_smem_offsets(const uint32_t *d_scan, const int64_t *d_off, in
 cudaError_t launch_smem_compact(const uint32_t *d_flag, const uint32_t *d_scan, const int32_t *d_ms_len, const uint32_t *d_ms_sp,
                                 const uint32_t *d_ms_ep, const int64_t *d_off, int64_t m, int64_t T, int32_t *d_start, int32_t *d_len,
                                 uint32_t *d_sp, uint32_t *d_ep, cudaStream_t st);
+// k-mer census over the LCP structure (needs ix.lcp8; 1 <= k): runs of rows that share their first k symbols, in tiles of 256 lcp8
+// blocks.  launch_census_last: d_tile_last[t] = the row after the last run end of tile t (0: none), t < census_tiles(n); its inclusive max
+// scan d_tile_incl gives every tile the start of the run open at its first row.  launch_census_spectrum: d_hist[min(count, buckets) - 1]
+// += 1 for every run, *d_max = max(*d_max, count) (both zeroed by the caller).  launch_census_list: the runs with min_count <= count <=
+// max_count (0 = no bound), without the rows d_ex[0 .. nex) (sorted) when min_count = 1 — d_tile_off == nullptr: their number per tile
+// to d_tile_cnt; else (sp, end) of each to d_sp / d_ep from slot d_tile_off[t] on, in row order.
+int64_t census_tiles(int64_t n);
+cudaError_t launch_census_last(const DevIndex &ix, uint32_t k, uint32_t *d_tile_last, cudaStream_t st);
+cudaError_t launch_census_spectrum(const DevIndex &ix, uint32_t k, const uint32_t *d_tile_incl, uint32_t buckets, unsigned long long *d_hist,
+                                   unsigned long long *d_max, cudaStream_t st);
+cudaError_t launch_census_list(const DevIndex &ix, uint32_t k, const uint32_t *d_tile_incl, uint32_t min_count, uint32_t max_count,
+                               const uint32_t *d_ex, uint32_t nex, uint32_t *d_tile_cnt, const uint32_t *d_tile_off, uint32_t *d_sp,
+                               uint32_t *d_ep, cudaStream_t st);
+// d_rows[0 .. steps] = row 0 and the rows `steps` LF steps from it (steps dependent rank requests in one lane group)
+cudaError_t launch_census_walk(const DevIndex &ix, LaunchCfg cfg, uint32_t steps, uint32_t *d_rows, cudaStream_t st);
 cudaError_t launch_occ(const DevIndex &ix, LaunchCfg cfg, const uint8_t *d_c, const int64_t *d_key, int64_t m,
                        int64_t *d_out, cudaStream_t st);
 cudaError_t launch_prev_range(const DevIndex &ix, LaunchCfg cfg, const int64_t *d_sp, const int64_t *d_ep,

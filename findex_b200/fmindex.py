@@ -115,6 +115,9 @@ def lib():
     L.fmx_smem_batch.argtypes = [p, p, p, i64, i32, i64, p, p, p, p, p]
     L.fmx_smem_dev.argtypes = [p, p, p, i64, i32, p, p, p, p, p, i64, C.POINTER(i64), p]
     L.fmx_last_match_requests.argtypes = [p, p]
+    L.fmx_kmer_spectrum.argtypes = [p, i32, i32, p, C.POINTER(i64), C.POINTER(i64)]
+    L.fmx_kmer_list_batch.argtypes = [p, i32, i64, i64, i64, C.POINTER(i64), p, p]
+    L.fmx_kmer_list_dev.argtypes = [p, i32, i64, i64, p, p, i64, C.POINTER(i64), p]
     L.fmx_regex_compile.argtypes = [p, i64, C.c_int, pp]
     L.fmx_regex_compile_engine.argtypes = [p, i64, C.c_int, C.c_int, pp]
     L.fmx_regex_free.argtypes = [p]
@@ -548,6 +551,58 @@ class GpuFMSearcher:
         r = np.zeros(3, np.int64)
         _check(lib().fmx_last_match_requests(self.h, _ptr(r)))
         return tuple(int(x) for x in r)
+
+    # ---- k-mer census (index opened with lcp=1; include/fmgpu.h) -----------------------------------------------------------------------
+    def kmer_spectrum(self, k, buckets):
+        """fmx_kmer_spectrum: (hist int64[buckets], distinct, max_occ); hist[b] = distinct k-mers of F occurring exactly b+1 times, the last
+        bucket those occurring >= buckets times"""
+        hist = np.zeros(max(buckets, 1), np.int64)
+        d, mx = C.c_int64(), C.c_int64()
+        _check(lib().fmx_kmer_spectrum(self.h, k, buckets, _ptr(hist), C.byref(d), C.byref(mx)))
+        return hist[:buckets], d.value, mx.value
+
+    def kmers(self, k, min_count=1, max_count=0, text=False):
+        """fmx_kmer_list_batch: (sp, ep) int64 of every distinct k-mer with min_count <= count <= max_count (0 = no bound), in row order
+        (count = ep - sp).  text=True also returns the k-mers' bytes in file order: nextSubstr(sp, k) of each interval."""
+        cap = min(self.n, 1 << 22)
+        total = C.c_int64()
+        while True:
+            sp, ep = np.zeros(max(cap, 1), np.int64), np.zeros(max(cap, 1), np.int64)
+            rc = lib().fmx_kmer_list_batch(self.h, k, min_count, max_count, cap, C.byref(total), _ptr(sp), _ptr(ep))
+            if rc == FMX_E_CAPACITY:
+                cap = total.value
+                continue
+            _check(rc)
+            t = total.value
+            sp, ep = sp[:t], ep[:t]
+            if not text:
+                return sp, ep
+            return sp, ep, self.next_substr_batch(sp, k) if t else []
+
+    def kmers_dev(self, k, d_sp, d_ep, cap, min_count=1, max_count=0, stream=0):
+        """fmx_kmer_list_dev (raw device pointers as ints): uint32 sp / ep [cap] out, as locate_dev takes them.  Returns the number of
+        k-mers listed; raises FmxError(FMX_E_CAPACITY) when cap is too small."""
+        total = C.c_int64()
+        _check(lib().fmx_kmer_list_dev(self.h, k, min_count, max_count, C.c_void_p(d_sp), C.c_void_p(d_ep), cap, C.byref(total), C.c_void_p(stream)))
+        return total.value
+
+    def top_kmers(self, k, t):
+        """the t most frequent k-mers (fewer when there are fewer), by count descending, then sp ascending: (sp, ep) int64.  The threshold
+        comes from the spectrum; the k-mers at or above it are listed and sorted here."""
+        _, distinct, max_occ = self.kmer_spectrum(k, 1)
+        if t <= 0 or distinct == 0:
+            return np.zeros(0, np.int64), np.zeros(0, np.int64)
+        buckets = min(max_occ, 1 << 16) + 1
+        hist, _, _ = self.kmer_spectrum(k, buckets)
+        above, threshold = 0, 1
+        for b in range(buckets - 1, -1, -1):                     # the largest count c with at least t k-mers occurring >= c times
+            above += int(hist[b])
+            if above >= t:
+                threshold = b + 1
+                break
+        sp, ep = self.kmers(k, min_count=threshold)
+        order = np.lexsort((sp, -(ep - sp)))[:t]
+        return sp[order], ep[order]
 
     def regex_search_batch(self, trees, cap_total=1 << 20):
         """trees: list of ReTree.  Returns per regex the sorted list of (len, sp, ep)."""

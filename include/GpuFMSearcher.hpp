@@ -123,6 +123,26 @@ public:
         for (int64_t k = 0; k < oo[1]; ++k) r.push_back({st[(size_t)k], ln[(size_t)k], sp[(size_t)k], ep[(size_t)k]});
         return r;
     }
+    // k-mer census (index opened with fmx_opts.lcp = 1): hist[b] = distinct k-mers occurring b+1 times (the last bucket: >= buckets
+    // times); the intervals of the k-mers with min_count <= count <= max_count (0 = no bound) in row order, count = ep - sp
+    struct KmerSpectrum { std::vector<int64_t> hist; int64_t distinct = 0, maxOcc = 0; };
+    KmerSpectrum kmerSpectrum(int32_t k, int32_t buckets) const {
+        KmerSpectrum r;
+        r.hist.resize((size_t)(buckets > 0 ? buckets : 1));
+        check(fmx_kmer_spectrum(h_, k, buckets, r.hist.data(), &r.distinct, &r.maxOcc));
+        r.hist.resize((size_t)buckets);
+        return r;
+    }
+    struct Kmers { std::vector<int64_t> sp, ep; };
+    Kmers kmers(int32_t k, int64_t minCount = 1, int64_t maxCount = 0) const {
+        Kmers r;
+        int64_t total = 0;
+        const int rc = fmx_kmer_list_batch(h_, k, minCount, maxCount, 0, &total, nullptr, nullptr);
+        if (rc != FMX_E_CAPACITY) { check(rc); return r; }        // FMX_OK here: nothing to list
+        r.sp.resize((size_t)total); r.ep.resize((size_t)total);
+        check(fmx_kmer_list_batch(h_, k, minCount, maxCount, total, &total, r.sp.data(), r.ep.data()));
+        return r;
+    }
     std::string nextSubstr(int64_t sp, int len) const {
         std::string out((size_t)(len > 0 ? len : 1), '\0'); int32_t ol = 0;
         check(fmx_next_substr_batch(h_, &sp, 1, len, reinterpret_cast<uint8_t *>(&out[0]), &ol));

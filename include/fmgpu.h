@@ -258,6 +258,32 @@ int fmx_smem_dev(fmx_index *ix, const void *d_pat, const void *d_off_i64, int64_
  * blocks and the record / escaped-value reads, req[2] = 128-byte minima lines of the widenings that leave their block                */
 int fmx_last_match_requests(const fmx_index *ix, int64_t req[3]);
 
+/* ---- k-mer census: which substrings of length k occur in the file, and how often -------------------------------------------------
+ * F is the file with its 0x00 bytes dropped (|F| = n - 1), T' = reverse(F) + '$'.  A k-mer is a string K of k >= 1 bytes that occurs in F;
+ * its count is the number of its occurrences in F, overlapping ones included; its interval is what fmx_count_batch returns for reverse(K)
+ * (the rows whose suffix starts with reverse(K)), so count = ep - sp.  Distinct k-mers have disjoint intervals; every listing is in row
+ * order, i.e. sorted by reverse(K), bytewise unsigned.  k-mers do not cross the end of the file (a window holding '$' is none), so the
+ * counts of all k-mers add up to |F| - k + 1; for k > |F| there are none and the calls return an empty result with FMX_OK.
+ * Row r < n - 1 ends a run of rows that share their first k symbols exactly when LCP[r] < k (row n - 1 always does), so the census is one
+ * streaming pass over the LCP structure of fmx_opts.lcp, about one byte per row (plus the escaped values of the rows with LCP >= 255
+ * when k > 255).  The k rows of T' positions n - k .. n - 1 ('$' within their first k symbols) are runs of one row that are no k-mer:
+ * the spectrum takes them out of its first bucket and of `distinct`, and a listing with min_count = 1 finds them by walking k - 1 LF
+ * steps from row 0 — k - 1 dependent rank requests, so such a listing costs time in proportion to k as well.
+ * These calls need the LCP structure and use no other accelerator; in particular they neither need nor use FMX_ACCEL_KMER or
+ * fmx_kmer_rows (the count path's table of k-mer intervals).  FMX_E_UNSUPPORTED when the index was opened without lcp; FMX_E_ARG for
+ * k < 1, buckets < 1, min_count < 1, max_count < 0, 0 < max_count < min_count, or null pointers (cap > 0 with null outputs).           */
+/* hist[b] = distinct k-mers occurring exactly b+1 times (b < buckets-1); hist[buckets-1] = those occurring >= buckets times;
+ * *distinct = the number of distinct k-mers, *max_occ = the largest count (0 when there are none) */
+int fmx_kmer_spectrum(fmx_index *ix, int32_t k, int32_t buckets, int64_t *hist, int64_t *distinct, int64_t *max_occ);
+/* every distinct k-mer with min_count <= count <= max_count (max_count 0 = no bound), in row order: its interval (sp[i], ep[i]).
+ * *total = their number; FMX_E_CAPACITY (with *total) when it exceeds cap, and nothing is written to sp / ep */
+int fmx_kmer_list_batch(fmx_index *ix, int32_t k, int64_t min_count, int64_t max_count, int64_t cap, int64_t *total,
+                        int64_t *sp, int64_t *ep);
+/* device-resident on `stream`: uint32 sp / ep[cap], exactly as fmx_locate_dev takes them (k-mers -> their positions without the host).
+ * Synchronises `stream` once to learn *total_out; FMX_E_CAPACITY when it exceeds cap, and nothing is written past cap */
+int fmx_kmer_list_dev(fmx_index *ix, int32_t k, int64_t min_count, int64_t max_count, void *d_sp_u32, void *d_ep_u32,
+                      int64_t cap, int64_t *total_out, void *stream);
+
 /* ---- regex: REParser.re2post M/re2/re2.scala:50-185 + ReTree.apply M/re2/retree.scala:156-370 -------
  * Compiles on the host to the reference's Glushkov position automaton, quirks included (SURVEY Q1-Q5);
  * FMX_E_SYNTAX / FMX_E_UNSUPPORTED exactly where the reference throws.                                  */
